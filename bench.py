@@ -7,6 +7,7 @@ Weak scaling: every rank processes `--samples-per-gpu` samples; `value` is the w
 
     python bench.py [--gpus N --steps K --warmup W]          (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference ...                     (the CPU oracle port on the host cores)
+    python bench.py --dump-outputs DIR ...                   (+ the results of the last timed step as DIR/<name>.npy)
 """
 from __future__ import annotations
 
@@ -55,7 +56,14 @@ def parse_args():
                     help="how the small result tables of the shards reach every GPU: fused = written into peer memory by the kernels that produce "
                          "them (no gather step), peer = copy-engine pushes after the step, nccl = one all_gather_into_tensor after the step")
     ap.add_argument("--cpu-samples", type=int, default=0, help="samples in the bounded CPU sample (0 = 4 x cores)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm (--impl b200) only: after the timed steps, write what the last step computed as DIR/<name>.npy (finite "
+                         "float32 / float64, at most 64 MB; rank 0's shard when N > 1), so that two builds can be compared output for output "
+                         "on the same seeded inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl b200)")
+    return args
 
 
 def workload_kwargs(name):
@@ -140,6 +148,49 @@ def cpu_oracle_throughput(hb, params, n_samples: int, threads: int):
     return n_samples / dt, dt
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLES = 16  # samples whose BEV grids (and relation tables) are written: ~1 MB each, the whole batch's grids would be far larger
+
+
+def dump_outputs(path, out, rel=None):
+    """Write one step's results as path/<name>.npy: the per-box and per-sample tables of the whole batch, the BEV grids of a fixed
+    seeded sample of it (bev_sample_index) and, with `rel` = (relation batch, its device tables), the footprints and pairwise
+    relation tables of the same samples.  Tables that would not fit the size limit next to the grids are cut to the sampled samples
+    as well (table_sample_index).  Integers are written as float64 (exact for uint32), floats as they are, and every value is finite:
+    box_nearest of a box without member points, +inf in the result, is written as -1."""
+    import torch
+    got = out.to_host()
+    keep = np.sort(np.random.default_rng(0).choice(out.n_samples, min(out.n_samples, DUMP_SAMPLES), replace=False))
+
+    def rows_of(off, samples):
+        return np.concatenate([np.arange(off[i], off[i + 1]) for i in samples] + [np.zeros(0, np.int64)])
+
+    arrays = {"bev_sample_index": keep}
+    arrays.update({k: got[k][keep] for k in ("bev_count", "bev_isum_q", "bev_intensity_sum", "bev_height")})
+    if rel is not None:
+        rel_db, tabs = rel
+        box_off = rel_db.host.sample_box_off.astype(np.int64)
+        pair_off = np.concatenate([[0], np.cumsum(np.diff(box_off) ** 2)])  # the n x n tables of the samples, back to back
+        rows, pairs = rows_of(box_off, keep), rows_of(pair_off, keep)
+        for k, idx in (("rect", rows), ("dist", pairs), ("bearing", pairs), ("category", pairs), ("overlap", pairs)):
+            arrays["relation_" + k] = tabs[k][torch.from_numpy(idx).to(tabs[k].device)].cpu().numpy()
+    tables = {k: got[k] for k in ("box_count", "box_nearest", "box_centroid", "proj_visible", "proj_extent", "stats")}
+    # +inf marks a box without member points (include/msc_geom.h); a distance is never negative, so -1 stands for it without loss
+    tables["box_nearest"] = np.where(np.isposinf(tables["box_nearest"]), np.float32(-1), tables["box_nearest"])
+    if 8 * sum(a.size for a in list(arrays.values()) + list(tables.values())) > DUMP_LIMIT_BYTES:
+        rows = rows_of(got["sample_box_off"].astype(np.int64), keep)
+        tables = {k: v[keep] if k == "stats" else v[rows] for k, v in tables.items()}
+        arrays["table_sample_index"] = keep
+    arrays.update(tables)
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for k, a in arrays.items()}
+    bad = [k for k, a in arrays.items() if not np.isfinite(a).all()]
+    if bad:  # the path writes no other NaN / inf: one here is a defect, and a dump must not hide it
+        raise ValueError("--dump-outputs: non-finite values in " + ", ".join(bad))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -212,9 +263,10 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def run_device_resident(workload: str, steps: int, warmup: int, samples_per_gpu: int, total_override: int = 0, sampler=None):
+    def run_device_resident(workload: str, steps: int, warmup: int, samples_per_gpu: int, total_override: int = 0, sampler=None, dump=None):
         """`steps` timed passes of the hot path over one HBM-resident batch of `workload`, sharded over the ranks; tables gathered with
-        one overlapped collective per step.  Returns the measurement and the pieces the caller reuses (distinct-sample batch, engine state)."""
+        one overlapped collective per step; `dump`: directory for the results of the last step (rank 0).  Returns the measurement and
+        the pieces the caller reuses (distinct-sample batch, engine state)."""
         wkw_, wname_ = workload_kwargs(workload)
         strong = {"mini404": 404, "trainval": 34149}.get(workload, 0)
         if strong:
@@ -318,11 +370,14 @@ def main():
         if rel_events:
             m["relation_table_ms"] = sum(a.elapsed_time(b) for a, b in rel_events) / len(rel_events)
             m["relation_table_bytes"] = int(hb.n_samples * (40 * 200 + 10 * 200 * 200))
+        if dump and rank == 0:
+            dump_outputs(dump, outs[(steps - 1) % len(outs)], (rel_db, rel) if rel_db is not None else None)
         return m, hb_u, reps
 
     # ---------------------------------------------------------------- the metric: BASELINE config 3, weak scaling, inputs resident in HBM
     sampler = ClockSampler(local_rank)
-    main, hb_u, reps = run_device_resident(args.workload, args.steps, args.warmup, args.samples_per_gpu, args.total_samples, sampler)
+    main, hb_u, reps = run_device_resident(args.workload, args.steps, args.warmup, args.samples_per_gpu, args.total_samples, sampler,
+                                           args.dump_outputs)
     strong_total = main["total_samples"] if main["scaling"] == "strong" else 0
 
     # ---------------------------------------------------------------- end to end: pinned host buffers in, host tables + BEV out

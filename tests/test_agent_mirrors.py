@@ -1,5 +1,5 @@
 """Agent-boundary mirrors against outputs of the reference itself (tests/golden/agent_golden.json, made by make_agent_golden.py),
-and integration.patch_reference applied to the REAL reference classes where /root/reference exists (build container only)."""
+and integration.patch_reference applied to the REAL reference classes when MSC_REFERENCE_SRC names the original project's src/ directory."""
 import inspect
 import json
 import os
@@ -8,8 +8,37 @@ import sys
 import numpy as np
 import pytest
 
-GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "agent_golden.json")))
-REF_SRC = "/root/reference/src"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLD = json.load(open(os.path.join(GOLDEN, "agent_golden.json")))
+REF_SRC = os.environ.get("MSC_REFERENCE_SRC", "")  # src/ of a checkout of the original project, which this repository does not carry
+
+
+# the methods whose parameter lists the mirrors share with the reference's classes (SURVEY.md section 8(b))
+SHARED_METHODS = {"LiDARAgent": ("_preprocess_point_cloud", "_segment_ground", "_generate_multi_layer_bev", "_generate_cluster_visualization",
+                                 "_detect_objects_3d", "_extract_semantic_features", "_generate_structured_report", "process",
+                                 "_classify_batch_with_llm"),
+                  "SceneGraphAgent": ("_parse_annotations", "_categorize_objects", "_build_spatial_zones", "process", "_generate_scene_graph",
+                                      "_generate_summary"),
+                  "CameraAgent": ("process",)}
+
+
+def mirror_signatures():
+    """Parameter names of the shared methods on the mirror classes (tests/golden/interface_golden.json records them)."""
+    from msc_geom.camera_agent import CameraAgent
+    from msc_geom.lidar_agent import LiDARAgent
+    from msc_geom.scenegraph_agent import SceneGraphAgent
+    classes = {"LiDARAgent": LiDARAgent, "SceneGraphAgent": SceneGraphAgent, "CameraAgent": CameraAgent}
+    return {c: {n: list(inspect.signature(getattr(classes[c], n)).parameters) for n in names} for c, names in SHARED_METHODS.items()}
+
+
+def test_mirror_signatures_equal_the_recorded_interface():
+    """The parameter lists test_patch_reference_on_the_real_reference_classes compares with the reference's own classes, against the
+    record of them: a change to the interface the reference's callers use fails here without the reference at hand."""
+    rec = json.load(open(os.path.join(GOLDEN, "interface_golden.json")))["signatures"]
+    assert mirror_signatures() == rec
+    from msc_geom import integration                                                   # the patch leaves the LLM half and process alone
+    assert not set(integration._LIDAR_METHODS) & {"_classify_batch_with_llm", "_extract_semantic_features", "_generate_structured_report", "process"}
+    assert set(integration._SCENE_METHODS) <= set(rec["SceneGraphAgent"]) - {"process", "_categorize_objects"}
 
 
 def test_fallback_scene_graph_and_summary_equal_reference():
@@ -47,7 +76,7 @@ def test_camera_agent_mirror_equals_reference():
             assert content[3]["image_url"]["url"] == GOLD["camera_first_image_url"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="needs the original project's src/ directory in MSC_REFERENCE_SRC")
 def test_patch_reference_on_the_real_reference_classes():
     """Names, signatures and attributes: everything the patch replaces exists on the reference's own classes with the same parameters,
     what it must leave alone is left alone, and the patched methods reach the engine they were given (a recorder; no GPU here)."""

@@ -1,7 +1,9 @@
 """Rows a1 / a2 / (f3) of SURVEY.md section 8 on an on-disk dataset: msc_geom.io.write_nuscenes_tree writes a v1.0-mini-shaped tree
 (JSON tables + .pcd.bin + .jpg), tests/devkit_shim stands in for the un-vendored devkit's table access, and the REAL NuScenesLoader code
-paths run against it -- this repo's, and (in the build container) the reference's own, unmodified, for a key-by-key comparison."""
+paths run against it -- this repo's, and (with MSC_REFERENCE_SRC set) the reference's own, unmodified, for a key-by-key comparison."""
+import hashlib
 import importlib
+import json
 import os
 import sys
 
@@ -10,7 +12,8 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SHIM = os.path.join(HERE, "devkit_shim")
-REF_SRC = "/root/reference/src"
+INTERFACE = os.path.join(HERE, "golden", "interface_golden.json")
+REF_SRC = os.environ.get("MSC_REFERENCE_SRC", "")  # src/ of a checkout of the original project, which this repository does not carry
 
 
 @pytest.fixture()
@@ -44,6 +47,47 @@ def _scenes():
             sc.append(s)
         scenes.append(sc)
     return scenes
+
+
+def _digest(a):
+    return [str(a.dtype), list(a.shape), list(a.strides), hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()]
+
+
+def loader_record(loader):
+    """What test_reference_loader_and_mirror_agree_on_the_same_tree compares between the reference's loader and the mirror, on the tree
+    of _scenes(), as JSON: scene list, camera channels, and per sample the key order, the scalar fields, the annotation dicts and
+    dtype / shape / strides / SHA-256 of the point cloud and of every camera frame (tests/golden/interface_golden.json records it)."""
+    samples = []
+    for sc in loader.get_scene_list():
+        for s in loader.load_scene_samples(sc["token"]):
+            rec = {"keys": list(s), "point_cloud": _digest(s["point_cloud"]), "images": [_digest(im) for im in s["images"]]}
+            rec.update({k: s[k] for k in ("sample_token", "timestamp", "scene_description", "scene_name", "camera_names", "metadata")})
+            rec["annotations"] = [{k: (np.asarray(v).tolist() if k == "velocity" else v) for k, v in a.items()} for a in s["annotations"]]
+            samples.append(rec)
+    return {"scene_list": loader.get_scene_list(), "camera_channels": list(loader.camera_channels), "samples": samples,
+            "sample_1_1": loader.get_sample_by_scene_index(1, 1)["sample_token"]}
+
+
+def test_loader_output_on_a_written_tree_equals_the_recorded_interface(tmp_path, devkit_shim):
+    """The mirror's output on the tree of _scenes(), against the record of it: the values the reference comparison below checks, here
+    on every run (NaN velocities compare equal)."""
+    from msc_geom import io as mio
+    mio.write_nuscenes_tree(str(tmp_path), _scenes())
+    got = json.loads(json.dumps(loader_record(devkit_shim.create_loader(str(tmp_path), "v1.0-mini"))))   # the JSON form of the record
+    want = json.load(open(INTERFACE))["loader"]
+    assert set(got) == set(want) and len(got["samples"]) == len(want["samples"]) == 4
+    for k in ("scene_list", "camera_channels", "sample_1_1"):
+        assert got[k] == want[k], k
+    for g, w in zip(got["samples"], want["samples"]):
+        assert list(g) == list(w)
+        for k in g:
+            if k != "annotations":
+                assert g[k] == w[k], (w["sample_token"], k)
+        assert len(g["annotations"]) == len(w["annotations"])
+        for a, b in zip(g["annotations"], w["annotations"]):
+            assert list(a) == list(b)
+            for k in a:
+                assert np.array_equal(np.asarray(a[k], dtype=float), np.asarray(b[k], dtype=float), equal_nan=True) if k == "velocity" else a[k] == b[k], k
 
 
 def test_real_loader_code_path_on_a_written_tree(tmp_path, devkit_shim):
@@ -90,7 +134,7 @@ def test_real_loader_code_path_on_a_written_tree(tmp_path, devkit_shim):
         assert np.array_equal(getattr(hb_files, k), getattr(hb_mem, k), equal_nan=True), k
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="needs the original project's src/ directory in MSC_REFERENCE_SRC")
 def test_reference_loader_and_mirror_agree_on_the_same_tree(tmp_path, devkit_shim):
     """The reference's own NuScenesLoader (src/nuscenes_loader.py:15-207), unmodified, on the written tree: every key of its sample dict
     equals the mirror's (which only ADDS keys)."""
