@@ -118,7 +118,9 @@ int msc_device_info(int32_t* sm_count, int32_t* smem_optin_bytes, int32_t* cc_ma
  * Layout rules the library cannot check (the arrays are on the device; msc_geom.engine.DeviceBatch.check_layout does, on the host copy):
  * sweep_start[] multiples of 4, the points buffer 16 bytes longer than the last sweep row.
  * stats[13] bit 0 (a cell count reached 65536) covers the cells of the shared-memory window (the centre of the grid, where counts are
- * high); cells outside it are accumulated with 64-bit global reductions and are not scanned.
+ * high), whatever the partition: a sample split over CTAs sets it exactly when the same sample on one CTA would; cells outside the
+ * window are accumulated with 64-bit global reductions and are not scanned.  Bit 31: the sample holds more boxes than the kernel has
+ * room for (max_boxes_per_sample under-declared); words 14 and 15 are 0.
  *
  * Context: options, the timing ring and the facts about the last call live in an msc_fused_ctx, created on the current
  * device.  Calls that share a context are serialised by it; contexts are independent, so host threads / streams / devices that each

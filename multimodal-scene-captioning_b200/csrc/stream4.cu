@@ -796,15 +796,17 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                 const uint32_t c0 = c2.x & kS4CountMask, c1 = c2.y & kS4CountMask;
                 const int cx = wx + win_lo, cy = wy + win_lo;
                 const size_t cell = (size_t)cy * (size_t)res + (size_t)cx;
+                uint32_t t0 = c0, t1 = c1;  // the cells' counts once this part's points are in
                 if (n_parts == 1) {
                     *reinterpret_cast<uint4*>(g_ci + cell * 2) = make_uint4(c0, s2.x, c1, s2.y);
-                } else {  // a part of a straddling sample merges with reductions (stream4_straddle_kernel zero-filled the layers)
-                    if (c0) atomicAdd(ci64 + cell, (unsigned long long)c0 | ((unsigned long long)s2.x << 32));
-                    if (c1) atomicAdd(ci64 + cell + 1, (unsigned long long)c1 | ((unsigned long long)s2.y << 32));
+                } else {  // a part of a straddling sample merges with atomics (stream4_straddle_kernel zero-filled the layers); the part whose
+                    // add takes a cell to 65536 sees it in the returned count, so the flag does not depend on how the sample is split
+                    if (c0) t0 += (uint32_t)atomicAdd(ci64 + cell, (unsigned long long)c0 | ((unsigned long long)s2.x << 32));
+                    if (c1) t1 += (uint32_t)atomicAdd(ci64 + cell + 1, (unsigned long long)c1 | ((unsigned long long)s2.y << 32));
                 }
                 if ((c0 | c1) == 0u) continue;
                 kept += c0 + c1;
-                flags |= (c0 >= 65536u || c1 >= 65536u) ? 1u : 0u;
+                flags |= (t0 >= 65536u || t1 >= 65536u) ? 1u : 0u;
                 if (FOV) {
                     const uint32_t d0 = s4_decided_in(class_of(cx, cy)), d1 = s4_decided_in(class_of(cx + 1, cy));
 #pragma unroll
