@@ -11,7 +11,9 @@
 // The device version: counting sort of the points into a grid of cells slightly larger than eps, neighbour counts over the
 // 27 surrounding cells, atomic-min union-find over core-core edges (the root of a component is its smallest index), rank of
 // the roots by an exclusive scan, and a final labelling pass.  Everything is float64 with -fmad=false, so the neighbour
-// relation -- and therefore every label -- is identical to scikit-learn's.
+// relation -- and therefore every label -- is identical to scikit-learn's whenever scikit-learn uses a tree (n >= 12 points).
+// For n <= 11 scikit-learn brute-forces the neighbour search with a BLAS expansion |a|^2 - 2ab + |b|^2 that can drop a pair at
+// exactly eps; this file keeps the rule above there too, so labels can differ from scikit-learn's only through such pairs.
 #include "msc_common.cuh"
 
 namespace msc {

@@ -107,7 +107,9 @@ __device__ __forceinline__ int bev_index(float c, float r, float two_r, float re
 }
 
 // 4-way bearing bins of scenegraph_agent.py:194-201 as exact predicates (0 front, 1 left, 2 back, 3 right)
+// At the origin the reference's atan2 follows the sign of dx: (-0, +-0) is +-180 degrees (left), (+0, +-0) is 0 (right).
 __device__ __forceinline__ uint8_t bearing4(double dx, double dy) {
+    if (dx == 0.0 && dy == 0.0) return signbit(dx) ? 1 : 3;
     if (dy > 0.0 && dx <= dy && -dx < dy) return 0;
     if (dx < 0.0 && dy <= -dx && dy > dx) return 1;
     if (dy < 0.0 && dx >= dy && dx < -dy) return 2;

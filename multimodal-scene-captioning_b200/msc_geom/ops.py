@@ -237,7 +237,12 @@ def cluster_views(eng: GeometryEngine, points: np.ndarray, clusters) -> np.ndarr
 
 def dbscan(eng: GeometryEngine, xyz: np.ndarray, eps: float = 0.5, min_samples: int = 10) -> np.ndarray:
     """sklearn.cluster.DBSCAN(eps, min_samples).fit(xyz).labels_ (lidar_agent.py:148-153), computed on the device with
-    scikit-learn's own labelling rule (see csrc/dbscan.cu).  Returns int64 labels like scikit-learn."""
+    scikit-learn's labelling rule (see csrc/dbscan.cu).  Returns int64 labels like scikit-learn.
+
+    Neighbours are the pairs with (dx^2 + dy^2) + dz^2 <= eps^2 in float64, scikit-learn's KD-tree rule.  The labels equal
+    scikit-learn's for 12 or more points.  For 11 or fewer scikit-learn searches by brute force, whose BLAS distance can drop a
+    pair at exactly eps; there the labels equal scikit-learn's when no pair is within 1e-6 of eps, and follow the rule above
+    otherwise."""
     rows, pitch = _raw_rows(xyz)
     n = int(rows.shape[0])
     if n == 0:

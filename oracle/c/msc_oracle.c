@@ -372,10 +372,12 @@ void orc_project_boxes(int n_boxes, const double* boxes, int n_cams, const doubl
 }
 
 /* 4-way bearing category with the bins of scenegraph_agent.py:190-201, written as exact predicates on
- * (dx, dy): 0=front [45,135)  1=left [135,225)  2=back [225,315)  3=right otherwise (incl. NaN, (0,0)).
+ * (dx, dy): 0=front [45,135)  1=left [135,225)  2=back [225,315)  3=right otherwise (incl. NaN, (+0,+-0));
+ * (-0,+-0) is left, because atan2(+-0, -0) = +-pi.
  * Equivalent to the reference's atan2 formula wherever that formula is exact (verified on the diagonals
  * and axes by tests/test_oracle_golden.py against the reference itself). */
 static inline uint8_t bearing4(double dx, double dy) {
+    if (dx == 0.0 && dy == 0.0) return signbit(dx) ? 1 : 3; /* atan2(+-0, -0) = +-pi: left; atan2(+-0, +0) = +-0: right */
     if (dy > 0.0 && dx <= dy && -dx < dy) return 0;
     if (dx < 0.0 && dy <= -dx && dy > dx) return 1;
     if (dy < 0.0 && dx >= dy && dx < -dy) return 2;
