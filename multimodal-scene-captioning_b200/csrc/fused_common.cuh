@@ -32,31 +32,14 @@ struct FusedArgs {
     // host-precomputed scalars (exact): 2r, res, RN(1/2r), 2^centroid_shift, 2^intensity_shift
     float two_r, resf, rcp_two_r, cscale, iscale;
     int32_t centroid_bias;  // 2^(centroid_shift + 6): makes the quantised coordinate non-negative
-    int32_t split;          // (unused since stream3.cu was retired: always 1)
+    int32_t pad_;           // (unused; it keeps the parameter offsets of the members below, and ptxas schedules the PPT = 4 main loops of
+                            // stream4.cu differently when they move)
     // Replicas of the small result tables (per-box tables, projection tables, stats): the kernels that produce a value also store it
     // through these pointers -- peer-mapped (symmetric) memory of the other GPUs of the box -- so the "gather" of a sharded batch is
     // part of the producing kernels (P2P stores over NVLink / NVSwitch), not a collective after them.  bev_* members are ignored.
     int32_t n_replicas;
     msc_batch_out replica[MSC_MAX_REPLICAS];
 };
-
-// BEV cell index, lidar_agent.py:547-552.  FASTDIV replaces the IEEE division by the 3-instruction Markstein
-// sequence, which tools/markstein_check.c proves equal to RN(a/b) for every float a outside the subnormal
-// quotient range for the whitelisted divisors (a = fl(c + r) is 0 or >= 2^-24 r here).
-template <bool FASTDIV>
-__device__ __forceinline__ int bev_cell(float c, float r, float two_r, float rcp_two_r, float resf, int res_m1) {
-    const float a = __fadd_rn(c, r);
-    float q;
-    if (FASTDIV) {
-        const float q0 = __fmul_rn(a, rcp_two_r);
-        const float rem = __fmaf_rn(-two_r, q0, a);
-        q = __fmaf_rn(rem, rcp_two_r, q0);
-    } else {
-        q = __fdiv_rn(a, two_r);
-    }
-    const int i = __float2int_rz(__fmul_rn(q, resf));
-    return min(max(i, 0), res_m1);
-}
 
 // Packed pairs of f32 (Blackwell FADD2 / FMUL2 / FFMA2: two IEEE round-to-nearest operations per lane and issue slot; each half is
 // bit-identical to the scalar instruction, so the arithmetic contract of msc_common.cuh is unchanged).
@@ -81,26 +64,108 @@ __device__ __forceinline__ unsigned long long f2_fma(unsigned long long a, unsig
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
     return r;
 }
-// bev_cell() of x and y in one packed pass (same operations, same order, per half)
-template <bool FASTDIV>
-__device__ __forceinline__ void bev_cell_xy(float x, float y, float r, float two_r, float rcp_two_r, float resf, int res_m1, int& ix, int& iy) {
-    const unsigned long long a = f2_add(f2_pack(x, y), f2_pack(r, r));
-    unsigned long long q;
-    if (FASTDIV) {
-        const unsigned long long rc = f2_pack(rcp_two_r, rcp_two_r);
-        const unsigned long long q0 = f2_mul(a, rc);
-        const unsigned long long rem = f2_fma(f2_pack(-two_r, -two_r), q0, a);
-        q = f2_fma(rem, rc, q0);
-    } else {
-        float ax, ay;
-        f2_unpack(a, ax, ay);
-        q = f2_pack(__fdiv_rn(ax, two_r), __fdiv_rn(ay, two_r));
-    }
-    float tx, ty;
-    f2_unpack(f2_mul(q, f2_pack(resf, resf)), tx, ty);
-    ix = min(max(__float2int_rz(tx), 0), res_m1);
-    iy = min(max(__float2int_rz(ty), 0), res_m1);
+// ---------------------------------------------------------------- shared-memory, mbarrier and bulk-copy (TMA) PTX
+// Every address is a 32-bit shared-state-space address: both streaming kernels derive theirs from one opaque base register, so their
+// loops carry no generic-address arithmetic.
+__device__ __forceinline__ uint32_t lds8(uint32_t saddr) {
+    uint32_t v;
+    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(saddr));
+    return v;
 }
+__device__ __forceinline__ uint32_t lds32(uint32_t saddr) {
+    uint32_t v;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(saddr));
+    return v;
+}
+__device__ __forceinline__ uint2 lds64(uint32_t saddr) {
+    uint2 v;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
+    return v;
+}
+__device__ __forceinline__ float4 lds128(uint32_t saddr) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr));
+    return v;
+}
+__device__ __forceinline__ void lds_f64x2(uint32_t saddr, double& a, double& b) {
+    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"(saddr));
+}
+__device__ __forceinline__ void red_shared_add(uint32_t saddr, uint32_t v) {
+    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(saddr), "r"(v) : "memory");
+}
+__device__ __forceinline__ uint32_t atom_shared_add(uint32_t saddr, uint32_t v) {
+    uint32_t old;
+    asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(old) : "r"(saddr), "r"(v) : "memory");
+    return old;
+}
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "MSC_WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@p bra MSC_DONE_%=;\n"
+        "bra MSC_WAIT_%=;\n"
+        "MSC_DONE_%=:\n"
+        "}\n" ::"r"(bar),
+        "r"(parity)
+        : "memory");
+}
+// L2 eviction policy for data that is read exactly once (the raw sweeps).
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {
+    uint64_t pol;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+    return pol;
+}
+// 1-D bulk asynchronous copy global -> shared (TMA unit; SASS UBLKCP) of `bytes` (a multiple of 16; both addresses 16-byte aligned),
+// announced on mbarrier `bar` first, whose phase completes when the bytes have landed.  One lane issues it.
+__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint64_t policy) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(dst),
+                 "l"(src), "r"(bytes), "r"(bar), "l"(policy)
+                 : "memory");
+}
+
+// ---------------------------------------------------------------- pieces both streaming kernels share
+// One point of box accumulators acc_s (kAccWords words): count, min s^2 (es2 bits: non-negative floats order as unsigned), and the
+// biased fixed-point coordinates.  Centroid sums are one 32-bit word per axis plus a carry word that takes a rare second atomic when
+// the word wraps (the coordinate is a 24-bit value, so that is at most once per 256 points): order-independent integers.
+__device__ __forceinline__ void box_accumulate(uint32_t acc_s, uint32_t es2, uint32_t fx, uint32_t fy, uint32_t fz) {
+    red_shared_add(acc_s, 1u);
+    asm volatile("red.shared.min.u32 [%0], %1;" ::"r"(acc_s + 4u), "r"(es2) : "memory");
+    const uint32_t ox = atom_shared_add(acc_s + 8u, fx), oy = atom_shared_add(acc_s + 12u, fy), oz = atom_shared_add(acc_s + 16u, fz);
+    if (ox > ~fx) red_shared_add(acc_s + 20u, 1u);
+    if (oy > ~fy) red_shared_add(acc_s + 24u, 1u);
+    if (oz > ~fz) red_shared_add(acc_s + 28u, 1u);
+}
+// Centroid coordinate of a box with cnt > 0 member points from the biased 64-bit sum of its fixed-point coordinates: exact integers and
+// one f64 division, which makes it bit-identical to the scalar definition.  (A box without members has the centroid 0 and the nearest
+// distance +inf.)
+__device__ __forceinline__ float box_centroid(const FusedArgs& A, uint32_t cnt, unsigned long long biased) {
+    const long long sum = (long long)biased - (long long)cnt * (long long)A.centroid_bias;
+    return (float)((double)sum / ((double)cnt * (double)A.cscale));
+}
+// Zero-fill one sample's global BEV layers: ncell (count, isum) pairs and ncell max heights, 16-byte stores by `nthreads` threads.
+__device__ __forceinline__ void zero_bev_layers(uint32_t* ci, float* h, size_t ncell, uint32_t tid, uint32_t nthreads) {
+    uint4* c4 = reinterpret_cast<uint4*>(ci);
+    for (size_t i = tid; i < ncell / 2; i += nthreads) c4[i] = make_uint4(0, 0, 0, 0);
+    uint4* h4 = reinterpret_cast<uint4*>(h);
+    for (size_t i = tid; i < ncell / 4; i += nthreads) h4[i] = make_uint4(0, 0, 0, 0);
+}
+// Edge-table entry (apex.x, apex.y, a, b) of one edge of camera wedge wq (in_wedge's form): q = p - apex, the point passes iff
+// fma(a, q.y, -(b * q.x)) >= 0, with (a, b) = (w4, w5) for the right edge and (-w2, -w3) for the left one.
+__device__ __forceinline__ float4 wedge_edge_entry(const float* wq, bool left) {
+    float4 E;
+    E.x = wq[0]; E.y = wq[1];
+    if (left) { E.z = -wq[2]; E.w = -wq[3]; } else { E.z = wq[4]; E.w = wq[5]; }
+    return E;
+}
+// Camera c's 8-bit counter of a pair of byte-counter words (cam_lo: cameras 0-3, cam_hi: 4-7).
+__device__ __forceinline__ uint32_t cam_byte(uint32_t cam_lo, uint32_t cam_hi, int c) { return ((c < 4 ? cam_lo : cam_hi) >> ((c & 3) * 8)) & 0xffu; }
 
 struct TableLayout {  // offsets (bytes) into the workspace
     size_t counter_off, boxprep_off, wedge_off, cullids_off;
@@ -110,9 +175,9 @@ struct TableLayout {  // offsets (bytes) into the workspace
     size_t total;
 };
 
-// fused_stream.cu (config 7): bytes of its per-CTA state block, and its launcher
-int stream_misc_bytes();
-void stream_shape_info(int* threads, int* tile_pts, int* ring_bytes, int* queue_bytes);
+// fused_stream.cu (config 7): launch shape (1024 threads x 2 points per lane), shared-memory layout (win_w < 0: does not fit), launcher
+constexpr int kStreamThreads = 1024, kStreamTilePts = 64;
+FusedLayout stream_layout(int smem_bytes, int res, int cull_dim, int cull_shift, int box_cap, int opt_window, int inner_dim);
 int launch_stream_kernel(const FusedArgs& args, const TableLayout& T, unsigned char* ws, int grid, bool fov, bool fast, cudaStream_t stream);
 // stream4.cu (config 10)
 int stream4_threads(int ppt);

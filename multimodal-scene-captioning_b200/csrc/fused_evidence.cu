@@ -246,37 +246,6 @@ static TableLayout table_layout(const msc_params& P, int n_samples, int n_boxes,
     return T;
 }
 
-// shared-memory layout of either streaming kernel.  window_cell_bytes / window_extra: bytes per window cell and fixed bytes next to the
-// window (stream4.cu: two arrays + their sink and cull-cell words); inner_dim > 0 reserves a fine class table in smem.
-static int compute_layout(const msc_fused_ctx* X, const msc_params& P, int max_boxes_in_batch, int ring_bytes, int queue_bytes, int misc_bytes,
-                          int inner_dim, bool inner_in_smem, int window_extra, int cull_cell_bytes, FusedLayout* L) {
-    const int cap = max_boxes_in_batch < 1 ? 1 : max_boxes_in_batch;
-    cull_geometry(P, X->opt_cull_shift, &L->cull_shift, &L->cull_dim);
-    L->max_boxes = cap;
-    int off = 0;
-    L->tiles_off = off; off += ring_bytes; off = (off + 127) & ~127;
-    L->queue_off = off; off += queue_bytes; off = (off + 127) & ~127;
-    L->cull_off = off; off += L->cull_dim * L->cull_dim * cull_cell_bytes; off = (off + 127) & ~127;
-    L->boxp_off = off; off += cap * kBoxStride * 4;
-    L->boxacc_off = off; off += cap * kAccWords * 4; off = (off + 127) & ~127;
-    L->misc_off = off; off += (misc_bytes + 127) & ~127;
-    L->inner_dim = inner_dim; L->inner_lo = (P.bev_res - inner_dim) / 2;
-    L->inner_off = off;
-    if (inner_in_smem) off += (inner_dim * inner_dim * 4 + 127) & ~127;
-    L->window_off = off;
-    const int avail = X->smem_optin - off - window_extra;
-    if (avail < 0) return -1;
-    int w = 0;
-    while ((w + 2) * (w + 2) * 8 <= avail && (w + 2) <= P.bev_res) w += 2;
-    if (X->opt_window > 0 && X->opt_window < w) w = X->opt_window & ~1;
-    if (((P.bev_res - w) / 2) & 1) w -= 2;  // keep win_lo even so flush rows stay 16-byte aligned
-    if (w < 0) w = 0;
-    L->win_w = w;
-    L->win_lo = (P.bev_res - w) / 2;
-    L->total_bytes = off + window_extra + w * w * 8;
-    return 0;
-}
-
 // tables (prepared boxes, projection, wedges, housekeeping -> workspace), then the candidate-box ids of every cull cell; the per-cell
 // edge classes of the camera wedges are computed by the streaming kernels themselves, per sample, from the wedges
 static int launch_tables(msc_fused_ctx* X, const FusedArgs& args, const TableLayout& T, unsigned char* ws, int n_boxes_total, int tile_pts,
@@ -440,65 +409,60 @@ int msc_fused_evidence_batch_replicated(msc_fused_ctx* X, const msc_params* para
     args.cscale = (float)(1 << params->centroid_shift);
     args.iscale = (float)(1 << params->intensity_shift);
     args.centroid_bias = 1 << (params->centroid_shift + 6);
-    args.split = 1;
     args.n_replicas = n_replicas;
     for (int r = 0; r < n_replicas; ++r) args.replica[r] = replicas[r];
     const bool fov = X->opt_fov != 0 && params->n_cams > 0;
     const bool fast = X->opt_fastdiv != 0 && fastdiv_verified(args.two_r);
-    // Kernel choice.  stream4.cu: rows read straight into registers, static partition of the batch in warp tiles (any batch size fills the
-    // device evenly).  fused_stream.cu: the TMA-ring generation, one sample per CTA at a time -- the only one with the per-point wedge
+    // Kernel choice.  stream4.cu: raw rows through one TMA slot per warp, static partition of the batch in warp tiles (any batch size fills
+    // the device evenly).  fused_stream.cu: the TMA-ring generation, one sample per CTA at a time -- the only one with the per-point wedge
     // classes a FOV *filter* (fov_keep_mask) needs.
     const bool keepmask = fov && params->fov_keep_mask != 0u;
     MSC_REQUIRE(!(keepmask && n_replicas > 0), "replicated result tables are not available with fov_keep_mask != 0");
     MSC_REQUIRE(!(X->opt_config == 7 && n_replicas > 0), "replicated result tables need the stream4.cu kernel (config 0 or 10)");
     int gen = keepmask ? 7 : X->opt_config;
     if (gen == 0) gen = 10;  // (on batches that fill the device the two kernels measure the same; stream4.cu also fills it on every other batch)
+    const bool s4 = gen == 10;
     X->last_fastdiv = fast ? 1 : 0;
     unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
     // fine edge classes for the kInnerMax x kInnerMax BEV cells around the sensor, where several image-column rays cross a 2 m cull cell
     int inner = fov ? (params->bev_res < kInnerMax ? params->bev_res : kInnerMax) : 0;
     inner &= ~1;
-    int rc = -1;
     bool standard = false;
-    if (gen == 10) {
+    int tile_pts, threads, grid;
+    if (s4) {
         // the box tables are sized for the standard capacity when the batch fits it, so that the layout -- and with it the choice of
         // the compile-time-constant instantiation -- does not depend on the batch
         const int cap = in->max_boxes_per_sample <= stream4_std_boxes() ? stream4_std_boxes() : in->max_boxes_per_sample;
         args.L = stream4_layout(X->smem_optin, X->opt_ppt, params->bev_res, cdim, cshift, cap, X->opt_window, inner);
-        rc = args.L.win_w < 0 ? -1 : 0;
-        standard = rc == 0 && fast && stream4_is_standard(args, X->smem_optin, X->opt_ppt, X->opt_window) && X->opt_std != 0;
-        X->last_tile_pts = 128; X->last_threads = stream4_threads(X->opt_ppt);
+        standard = args.L.win_w >= 0 && fast && stream4_is_standard(args, X->smem_optin, X->opt_ppt, X->opt_window) && X->opt_std != 0;
+        tile_pts = 128; threads = stream4_threads(X->opt_ppt);
+        // every CTA gets the same number of warp tiles; a batch of a few thousand rows is not spread thinner than one tile per warp
+        const long long pts = in->points_per_sample_hint > 0 ? in->points_per_sample_hint : 347200;
+        const long long est_tiles = (long long)in->n_samples * ((pts + tile_pts - 1) / tile_pts);
+        const long long g = X->opt_grid > 0 ? X->opt_grid : 2 * est_tiles / (threads / 32);  // (small batches: down to half a tile per warp)
+        grid = (int)(g < 1 ? 1 : (g > X->sms ? X->sms : g));
+        if (grid > kMaxGrid) grid = kMaxGrid;
     } else {
-        int threads = 0, tile_pts = 0, ring = 0, queue = 0;
-        stream_shape_info(&threads, &tile_pts, &ring, &queue);
-        rc = compute_layout(X, *params, in->max_boxes_per_sample, ring, queue, stream_misc_bytes(), inner, true, 0, 8, &args.L);
-        X->last_tile_pts = tile_pts; X->last_threads = threads;
+        args.L = stream_layout(X->smem_optin, params->bev_res, cdim, cshift, in->max_boxes_per_sample, X->opt_window, inner);
+        tile_pts = kStreamTilePts; threads = kStreamThreads;
+        grid = in->n_samples < X->sms ? in->n_samples : X->sms;
     }
-    if (rc != 0) {
+    X->last_tile_pts = tile_pts; X->last_threads = threads;
+    if (args.L.win_w < 0) {
         set_error("shared-memory layout does not fit (%d bytes available)", X->smem_optin);
         return MSC_ERR_UNSUPPORTED;
     }
     X->last_config = gen;
     X->last_window = args.L.win_w;
     X->last_smem = args.L.total_bytes;
-    if ((rc = launch_tables(X, args, T, ws, in->n_boxes, gen == 10 ? 128 : 0, in->max_boxes_per_sample, stream)) != MSC_OK) return rc;  // stream4.cu: 128-row warp tiles
-    int grid;
-    if (gen == 10) {
-        // every CTA gets the same number of warp tiles; a batch of a few thousand rows is not spread thinner than one tile per warp
-        const long long pts = in->points_per_sample_hint > 0 ? in->points_per_sample_hint : 347200;
-        const int tile_pts = 128, warps = stream4_threads(X->opt_ppt) / 32;
-        const long long est_tiles = (long long)in->n_samples * ((pts + tile_pts - 1) / tile_pts);
-        long long g = X->opt_grid > 0 ? X->opt_grid : 2 * est_tiles / warps;  // (small batches: down to half a tile per warp)
-        grid = (int)(g < 1 ? 1 : (g > X->sms ? X->sms : g));
-        if (grid > kMaxGrid) grid = kMaxGrid;
-        if ((rc = launch_stream4_partition(args, T, ws, grid, stream, &X->last_launches)) != MSC_OK) return rc;
-    } else {
-        grid = in->n_samples < X->sms ? in->n_samples : X->sms;
-    }
+    int rc;
+    // (stream4.cu's static partition: the table kernel prefix-sums the warp tiles of every sample, a pre-kernel zero-fills the samples
+    // that straddle CTAs)
+    if ((rc = launch_tables(X, args, T, ws, in->n_boxes, s4 ? tile_pts : 0, in->max_boxes_per_sample, stream)) != MSC_OK) return rc;
+    if (s4 && (rc = launch_stream4_partition(args, T, ws, grid, stream, &X->last_launches)) != MSC_OK) return rc;
     X->last_grid = grid;
     if ((rc = time_begin(X, stream)) != MSC_OK) return rc;
-    rc = gen == 10 ? launch_stream4_kernel(args, T, ws, grid, X->opt_ppt, fov, fast, standard, stream)
-                   : launch_stream_kernel(args, T, ws, grid, fov, fast, stream);
+    rc = s4 ? launch_stream4_kernel(args, T, ws, grid, X->opt_ppt, fov, fast, standard, stream) : launch_stream_kernel(args, T, ws, grid, fov, fast, stream);
     X->last_standard = standard ? 1 : 0;
     if (rc != MSC_OK) return rc;
     ++X->last_launches;

@@ -52,19 +52,35 @@ struct StreamMisc {  // small per-CTA state at misc_off
     float wq[MSC_MAX_CAMS * 6];         // this sample's camera wedges (fused_tables_kernel), source of the per-cell edge classes
 };
 
-int stream_misc_bytes() { return (int)sizeof(StreamMisc); }
+// launch shape: 1024 threads x 2 points per lane
+using Shape0 = StreamShape<kStreamThreads, kStreamTilePts / 32, false>;
 
-// ---- shared-state-space accesses through 32-bit addresses (no generic-address arithmetic in the loop)
-__device__ __forceinline__ void red_shared_add(uint32_t saddr, uint32_t v) {
-    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(saddr), "r"(v) : "memory");
-}
-__device__ __forceinline__ float4 lds128(uint32_t saddr) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr));
-    return v;
-}
-__device__ __forceinline__ void lds_f64x2(uint32_t saddr, double& a, double& b) {
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"(saddr));
+// Shared-memory layout (bytes): the warps' ring slots, their candidate queues, (box ids, edge classes) per cull cell, the box tables, the
+// per-CTA state, the fine edge classes around the sensor, and last the BEV window of (count, isum) cells, the largest even side that fits.
+FusedLayout stream_layout(int smem_bytes, int res, int cull_dim, int cull_shift, int box_cap, int opt_window, int inner_dim) {
+    FusedLayout L{};
+    L.cull_dim = cull_dim; L.cull_shift = cull_shift; L.max_boxes = box_cap < 1 ? 1 : box_cap;
+    int off = 0;
+    L.tiles_off = off; off += (Shape0::kRingBytes + 127) & ~127;
+    L.queue_off = off; off += (Shape0::kQueueBytes + 127) & ~127;
+    L.cull_off = off; off += (cull_dim * cull_dim * 8 + 127) & ~127;
+    L.boxp_off = off; off += L.max_boxes * kBoxStride * 4;
+    L.boxacc_off = off; off += L.max_boxes * kAccWords * 4; off = (off + 127) & ~127;
+    L.misc_off = off; off += ((int)sizeof(StreamMisc) + 127) & ~127;
+    L.inner_dim = inner_dim; L.inner_lo = (res - inner_dim) / 2;
+    L.inner_off = off; off += (inner_dim * inner_dim * 4 + 127) & ~127;
+    L.window_off = off;
+    const int avail = smem_bytes - off;
+    if (avail < 0) { L.win_w = -1; return L; }
+    int w = 0;
+    while ((w + 2) * (w + 2) * 8 <= avail && (w + 2) <= res) w += 2;
+    if (opt_window > 0 && opt_window < w) w = opt_window & ~1;
+    if (((res - w) / 2) & 1) w -= 2;  // keep win_lo even so flush rows stay 16-byte aligned
+    if (w < 0) w = 0;
+    L.win_w = w;
+    L.win_lo = (res - w) / 2;
+    L.total_bytes = off + w * w * 8;
+    return L;
 }
 
 template <class C, bool FOV, bool FASTDIV, bool KEEPMASK>
@@ -105,8 +121,8 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
     asm volatile("" : "+r"(lt_mask));  // keep it in its register (the compiler would re-derive it from %tid at every use)
 
     if (lane == 0) {
-        mbar_init(&misc->full_bar[warp * 2 + 0], 1);
-        mbar_init(&misc->full_bar[warp * 2 + 1], 1);
+        mbar_init(smem_u32(&misc->full_bar[warp * 2 + 0]), 1);
+        mbar_init(smem_u32(&misc->full_bar[warp * 2 + 1]), 1);
         mbar_fence_init();
     }
     uint32_t wk = 0;  // tiles this warp has consumed since launch: slot = wk & 1, mbarrier parity = (wk >> 1) & 1
@@ -151,14 +167,7 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
             const uint32_t npts = min((uint32_t)TP, n_cnt - n_first);
             const uint32_t bytes = (npts * 20u + 15u) & ~15u;
             const float* src = A.in.points + ((size_t)n_base + n_first) * 5;
-            if (lane == 0) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_s + slot * 8u), "r"(bytes) : "memory");
-                asm volatile(
-                    "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-                        ring_s + slot * (uint32_t)(TF * 4)),
-                    "l"(src), "r"(bytes), "r"(bar_s + slot * 8u), "l"(policy)
-                    : "memory");
-            }
+            if (lane == 0) bulk_load(ring_s + slot * (uint32_t)(TF * 4), src, bytes, bar_s + slot * 8u, policy);
         };
         bool more = next_tile();
         if (more) issue(wk & 1u);  // overlaps the prologue below
@@ -191,19 +200,14 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
                 const int c = tid & (MSC_MAX_CAMS - 1);
                 float4 E = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
                 if (c < n_cams) {
-                    const float* wq = g_wedges + ((size_t)sample * MSC_MAX_CAMS + c) * 6;
-                    // cr = fma(A, qy, -(B * qx)) >= 0 with (A, B) = (w4, w5) for the right edge, (-w2, -w3) for the left one  (in_wedge)
-                    E = (tid >= MSC_MAX_CAMS) ? make_float4(wq[0], wq[1], -wq[2], -wq[3]) : make_float4(wq[0], wq[1], wq[4], wq[5]);
+                    E = wedge_edge_entry(g_wedges + ((size_t)sample * MSC_MAX_CAMS + c) * 6, tid >= MSC_MAX_CAMS);
                 }
                 misc->edge[tid] = E;
                 if (tid == 0) misc->edge_pad = E;
             }
             // zero-fill this sample's global layers (window cells are overwritten by the flush; filling them too
             // keeps the stores fully coalesced)
-            uint4* c4 = reinterpret_cast<uint4*>(g_ci);
-            for (size_t i = tid; i < ncell / 2; i += NT) c4[i] = make_uint4(0, 0, 0, 0);
-            uint4* h4 = reinterpret_cast<uint4*>(g_h);
-            for (size_t i = tid; i < ncell / 4; i += NT) h4[i] = make_uint4(0, 0, 0, 0);
+            zero_bev_layers(g_ci, g_h, ncell, tid, NT);
         }
         __threadfence();
         __syncthreads();
@@ -224,19 +228,8 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
                 const uint32_t fx = (uint32_t)(__float2int_rn(__fmul_rn(e.x, A.cscale)) + A.centroid_bias);
                 const uint32_t fy = (uint32_t)(__float2int_rn(__fmul_rn(e.y, A.cscale)) + A.centroid_bias);
                 const uint32_t fz = (uint32_t)(__float2int_rn(__fmul_rn(e.z, A.cscale)) + A.centroid_bias);
-                // centroid sums: one 32-bit word per axis plus a carry word that takes a rare second atomic when the word wraps
-                // (the coordinate is a 24-bit value, so that is at most once per 256 points); still order-independent integers
                 auto accumulate = [&](int b) {
-                    const uint32_t acc_s = smem_s + (uint32_t)L.boxacc_off + (uint32_t)b * (uint32_t)(kAccWords * 4);
-                    red_shared_add(acc_s, 1u);
-                    asm volatile("red.shared.min.u32 [%0], %1;" ::"r"(acc_s + 4u), "r"(__float_as_uint(es2)) : "memory");
-                    uint32_t ox, oy, oz;
-                    asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(ox) : "r"(acc_s + 8u), "r"(fx) : "memory");
-                    asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(oy) : "r"(acc_s + 12u), "r"(fy) : "memory");
-                    asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(oz) : "r"(acc_s + 16u), "r"(fz) : "memory");
-                    if (ox > ~fx) red_shared_add(acc_s + 20u, 1u);
-                    if (oy > ~fy) red_shared_add(acc_s + 24u, 1u);
-                    if (oz > ~fz) red_shared_add(acc_s + 28u, 1u);
+                    box_accumulate(smem_s + (uint32_t)L.boxacc_off + (uint32_t)b * (uint32_t)(kAccWords * 4), __float_as_uint(es2), fx, fy, fz);
                 };
                 int hit = -1;
                 if (ids == kCullAll) {  // crowded cell (more than four boxes): test every box
@@ -280,20 +273,7 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
             }
             more = next_tile();
             if (more) issue((wk + 1u) & 1u);
-            {
-                const uint32_t bar = bar_s + (wk & 1u) * 8u, parity = (wk >> 1) & 1u;
-                asm volatile(
-                    "{\n"
-                    ".reg .pred p;\n"
-                    "MSC_SWAIT_%=:\n"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-                    "@p bra MSC_SDONE_%=;\n"
-                    "bra MSC_SWAIT_%=;\n"
-                    "MSC_SDONE_%=:\n"
-                    "}\n" ::"r"(bar),
-                    "r"(parity)
-                    : "memory");
-            }
+            mbar_wait_parity(bar_s + (wk & 1u) * 8u, (wk >> 1) & 1u);
             const float* tp = ring + (wk & 1u) * TF + lane * 5;
 
             // ---- phase A: branch-free over the lane's points so their dependency chains interleave
@@ -340,15 +320,14 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
                 const int ix = bev_cell<FASTDIV>(xr[u], P.bev_range, A.two_r, A.rcp_two_r, A.resf, res_m1);
                 const int iy = bev_cell<FASTDIV>(yr[u], P.bev_range, A.two_r, A.rcp_two_r, A.resf, res_m1);
                 const uint32_t ce_s = smem_s + (uint32_t)L.cull_off + (uint32_t)(((iy >> L.cull_shift) * L.cull_dim + (ix >> L.cull_shift)) << 3);
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(cand[u]) : "r"(ce_s));
+                cand[u] = lds32(ce_s);
                 if (FOV) {
                     // edge classes: from the fine grid (one BEV cell) around the sensor, where a 2 m cull cell is crossed by several
                     // image-column rays, else from the cull cell; one load either way
                     const uint32_t jx = (uint32_t)(ix - L.inner_lo), jy = (uint32_t)(iy - L.inner_lo);
                     const bool fine = jx < (uint32_t)L.inner_dim && jy < (uint32_t)L.inner_dim;
                     const uint32_t cls_s = fine ? smem_s + (uint32_t)L.inner_off + ((jy * (uint32_t)L.inner_dim + jx) << 2) : ce_s + 4u;
-                    uint32_t cls;
-                    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(cls) : "r"(cls_s));
+                    const uint32_t cls = lds32(cls_s);
                     in_bits[u] = cls & 0xffu;
                     st[u] = keep[u] ? (cls >> 8) : 0u;  // bit c: right edge of camera c undecided in this cell, bit 8 + c: left edge
                 } else {
@@ -447,7 +426,7 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
                 if (cam_pts > 255u - PPT) {  // spill the byte counters before any of them can wrap
 #pragma unroll
                     for (int c = 0; c < MSC_MAX_CAMS; ++c) {
-                        const uint32_t v = ((c < 4 ? cam_lo : cam_hi) >> ((c & 3) * 8)) & 0xffu;
+                        const uint32_t v = cam_byte(cam_lo, cam_hi, c);
                         if (v) atomicAdd(&misc->stats[5 + c], v);
                     }
                     cam_lo = cam_hi = cam_pts = 0;
@@ -464,7 +443,7 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
             uint32_t v[3 + MSC_MAX_CAMS];
             v[0] = c_close; v[1] = c_kept; v[2] = c_ground;
 #pragma unroll
-            for (int c = 0; c < MSC_MAX_CAMS; ++c) v[3 + c] = FOV ? (((c < 4 ? cam_lo : cam_hi) >> ((c & 3) * 8)) & 0xffu) : 0u;
+            for (int c = 0; c < MSC_MAX_CAMS; ++c) v[3 + c] = FOV ? cam_byte(cam_lo, cam_hi, c) : 0u;
 #pragma unroll
             for (int i = 0; i < 3 + (FOV ? MSC_MAX_CAMS : 0); ++i) {
                 const uint32_t r = __reduce_add_sync(0xffffffffu, v[i]);
@@ -494,13 +473,9 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
                     A.out.box_centroid[o * 3 + 0] = 0.0f; A.out.box_centroid[o * 3 + 1] = 0.0f; A.out.box_centroid[o * 3 + 2] = 0.0f;
                 } else {
                     A.out.box_nearest[o] = __fsqrt_rn(__uint_as_float(acc[1]));
-                    const double den = (double)cnt * (double)A.cscale;
 #pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        const unsigned long long biased = (unsigned long long)acc[2 + k] + ((unsigned long long)acc[5 + k] << 32);
-                        const long long sum = (long long)biased - (long long)cnt * (long long)A.centroid_bias;
-                        A.out.box_centroid[o * 3 + k] = (float)((double)sum / den);
-                    }
+                    for (int k = 0; k < 3; ++k)
+                        A.out.box_centroid[o * 3 + k] = box_centroid(A, cnt, (unsigned long long)acc[2 + k] + ((unsigned long long)acc[5 + k] << 32));
                 }
             }
             if (flags) atomicOr(&misc->stats[13], flags);
@@ -520,9 +495,6 @@ __global__ void __launch_bounds__(C::kThreads, 1) stream_evidence_kernel(const _
     }
 }
 
-// launch shape: 1024 threads x 2 points per lane
-using Shape0 = StreamShape<1024, 2, false>;
-
 template <class C, bool FOV, bool FASTDIV, bool KEEPMASK>
 static int launch_one(const FusedArgs& args, const TableLayout& T, unsigned char* ws, int grid, cudaStream_t stream) {
     auto kern = stream_evidence_kernel<C, FOV, FASTDIV, KEEPMASK>;
@@ -530,10 +502,6 @@ static int launch_one(const FusedArgs& args, const TableLayout& T, unsigned char
     kern<<<grid, C::kThreads, args.L.total_bytes, stream>>>(args, T, ws);
     MSC_CUDA(cudaGetLastError());
     return MSC_OK;
-}
-
-void stream_shape_info(int* threads, int* tile_pts, int* ring_bytes, int* queue_bytes) {
-    *threads = Shape0::kThreads; *tile_pts = Shape0::kTilePts; *ring_bytes = Shape0::kRingBytes; *queue_bytes = Shape0::kQueueBytes;
 }
 
 int launch_stream_kernel(const FusedArgs& args, const TableLayout& T, unsigned char* ws, int grid, bool fov, bool fast, cudaStream_t stream) {

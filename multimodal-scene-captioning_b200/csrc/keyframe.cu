@@ -150,8 +150,8 @@ __global__ void __launch_bounds__(256) kf_bev_raster_kernel(const __grid_constan
     if (i < n) {
         const bool is_obj = i >= n_ground;
         const float4 p = is_obj ? object[i - n_ground] : ground[i];
-        const int ix = bev_index(p.x, P.bev_range, two_r, resf, res - 1);
-        const int iy = bev_index(p.y, P.bev_range, two_r, resf, res - 1);
+        const int ix = bev_cell<false>(p.x, P.bev_range, two_r, 0.0f, resf, res - 1);
+        const int iy = bev_cell<false>(p.y, P.bev_range, two_r, 0.0f, resf, res - 1);
         const size_t cell = (size_t)iy * res + ix;  // [y, x] indexing, :559
         atomicAdd(&count[cell], 1u);                                                   // :559
         if (p.z > 0.0f) atomicMax(reinterpret_cast<int*>(height) + cell, __float_as_int(p.z));  // :560, 0-initialised

@@ -32,44 +32,8 @@ void set_error(const char* fmt, ...);
         }                                                                                   \
     } while (0)
 
-// ---------------------------------------------------------------- mbarrier + bulk-copy (TMA) PTX
+// 32-bit shared-state-space address of a pointer into shared memory
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_parity(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "MSC_WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra MSC_DONE_%=;\n"
-        "bra MSC_WAIT_%=;\n"
-        "MSC_DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-// L2 eviction policy for data that is read exactly once (the raw sweeps).
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-// 1-D bulk asynchronous copy global -> shared (TMA unit; SASS UBLKCP), completion on an mbarrier.
-// dst/src 16-byte aligned, bytes a multiple of 16.
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-        : "memory");
-}
 
 // ---------------------------------------------------------------- f64 pose algebra (no FMA; see header)
 // unit quaternion (w,x,y,z) -> row-major rotation, normalising first
@@ -99,10 +63,21 @@ __device__ __forceinline__ void frame_change(const double* __restrict__ pose7, d
     for (int k = 0; k < 9; ++k) R[k] = T[k];
 }
 
-// BEV cell index (lidar_agent.py:547-552): clip(trunc((c + r) / (2r) * res), 0, res-1), float32 steps
-__device__ __forceinline__ int bev_index(float c, float r, float two_r, float resf, int res_m1) {
-    float t = __fmul_rn(__fdiv_rn(__fadd_rn(c, r), two_r), resf);
-    int i = __float2int_rz(t);
+// BEV cell index (lidar_agent.py:547-552): clip(trunc((c + r) / (2r) * res), 0, res-1), float32 steps.  FASTDIV replaces the IEEE
+// division by the 3-instruction Markstein sequence (rcp_two_r = RN(1/2r); unused without it), which tools/markstein_check.c proves equal
+// to RN(a/b) for every float a outside the subnormal quotient range for the whitelisted divisors (a = fl(c + r) is 0 or >= 2^-24 r here).
+template <bool FASTDIV>
+__device__ __forceinline__ int bev_cell(float c, float r, float two_r, float rcp_two_r, float resf, int res_m1) {
+    const float a = __fadd_rn(c, r);
+    float q;
+    if (FASTDIV) {
+        const float q0 = __fmul_rn(a, rcp_two_r);
+        const float rem = __fmaf_rn(-two_r, q0, a);
+        q = __fmaf_rn(rem, rcp_two_r, q0);
+    } else {
+        q = __fdiv_rn(a, two_r);
+    }
+    const int i = __float2int_rz(__fmul_rn(q, resf));
     return min(max(i, 0), res_m1);
 }
 

@@ -29,14 +29,6 @@
 //     A.replica[]): the gather of a sharded batch without a collective.
 #include "fused_common.cuh"
 
-// Measured alternative, off: lanes of a candidate drain whose points lie in the same box find each other with __match_any_sync, reduce
-// count / nearest / sums with __reduce_*_sync over the group and one lane issues the box's five atomics.  Bit-identical, and 76 %
-// slower (2.86 vs 1.63 ms per 592 samples): MATCH.ANY plus, for masks that differ between lanes, ptxas's per-group loop of WARPSYNC +
-// REDUX cost far more than the same-address ATOMS they save (3 hits per box and drain on this workload).
-#ifndef MSC_S4_AGGREGATE
-#define MSC_S4_AGGREGATE 0
-#endif
-
 namespace msc {
 
 // Two launch shapes: PPT = 2 points per lane and pass (1024 threads x 64 registers, the default: more warps to hide latency) and PPT = 4
@@ -50,16 +42,13 @@ constexpr int kS4PoseSmem = 10;   // sweeps whose transforms / extents are stage
 constexpr int kS4SinkWords = 64;  // per array: [0, 32) remove_close sink of lane l, [32, 64) range / height sink of lane l
 constexpr uint32_t kS4CodeShift = 27, kS4CountMask = (1u << kS4CodeShift) - 1u, kS4CodeMulti = 31u;
 
-struct alignas(16) S4Edge {  // one entry per edge code: the exact test of that image-column ray
-    float ax, ay, a, b;      // q = p - (ax, ay); the point passes iff fma(a, q.y, -(b * q.x)) >= 0
-};
-
 constexpr int kS4PairCodes = 14;  // codes 17..30: cells crossed by exactly two rays of different cameras, assigned per sample as they occur
 
 struct S4Misc {  // small per-CTA state at misc_off
-    // [code]: 0 = pad (the test fails: a = NaN); 1 + c right edge, 9 + c left edge of camera c; 17 + i the first / second edge of pair i
-    // (edge2 is a pad for every other code); 31 = several edges, resolved on a cold path from the cell's class word
-    S4Edge edge1[32], edge2[32];
+    // [code]: the exact test of an image-column ray, wedge_edge_entry(); 0 = pad (the test fails: a = NaN); 1 + c right edge, 9 + c left
+    // edge of camera c; 17 + i the first / second edge of pair i (edge2 is a pad for every other code); 31 = several edges, resolved on a
+    // cold path from the cell's class word
+    float4 edge1[32], edge2[32];
     uint2 inc1[32], inc2[32];  // byte-counter increments (cameras 0-3, 4-7) of the entry's camera
     uint32_t pairs[16];  // pair i: 0 = free, else 0x100 | e1 | e2 << 4 (edge numbers 0-7 right, 8-15 left)
     uint32_t stats[MSC_STATS_STRIDE];
@@ -140,36 +129,6 @@ FusedLayout stream4_layout(int smem_bytes, int ppt, int res, int cull_dim, int c
 }
 int stream4_std_boxes() { return kS4StdBoxes; }
 
-// ---- shared-state-space accesses through 32-bit addresses (no generic-address arithmetic in the loop)
-__device__ __forceinline__ void s4_red_add(uint32_t saddr, uint32_t v) { asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(saddr), "r"(v) : "memory"); }
-__device__ __forceinline__ uint32_t s4_atom_add(uint32_t saddr, uint32_t v) {
-    uint32_t old;
-    asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(old) : "r"(saddr), "r"(v) : "memory");
-    return old;
-}
-__device__ __forceinline__ float4 s4_lds128(uint32_t saddr) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr));
-    return v;
-}
-__device__ __forceinline__ uint2 s4_lds64(uint32_t saddr) {
-    uint2 v;
-    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
-    return v;
-}
-__device__ __forceinline__ uint32_t s4_lds8(uint32_t saddr) {
-    uint32_t v;
-    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(saddr));
-    return v;
-}
-__device__ __forceinline__ uint32_t s4_lds32(uint32_t saddr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(saddr));
-    return v;
-}
-__device__ __forceinline__ void s4_lds_f64x2(uint32_t saddr, double& a, double& b) {
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"(saddr));
-}
 // predicated global reductions (one instruction each, no branch-around sequence)
 __device__ __forceinline__ void s4_red_global_u64_if(unsigned long long* p, unsigned long long v, bool pred) {
     asm volatile("{\n.reg .pred p;\nsetp.ne.u32 p, %2, 0;\n@p red.global.add.u64 [%0], %1;\n}" ::"l"(p), "l"(v), "r"((uint32_t)pred) : "memory");
@@ -218,10 +177,7 @@ __global__ void __launch_bounds__(256) stream4_straddle_kernel(const __grid_cons
     if (n == 0 || !(tile_off[s] < g && g < tile_off[s + 1])) return;
     if (b > 1u && gp > tile_off[s]) return;  // an earlier boundary lies inside the same sample
     const size_t ncell = (size_t)A.P.bev_res * (size_t)A.P.bev_res;
-    uint4* c4 = reinterpret_cast<uint4*>(A.out.bev_ci + (size_t)s * ncell * 2);
-    for (size_t i = threadIdx.x; i < ncell / 2; i += blockDim.x) c4[i] = make_uint4(0, 0, 0, 0);
-    uint4* h4 = reinterpret_cast<uint4*>(A.out.bev_height + (size_t)s * ncell);
-    for (size_t i = threadIdx.x; i < ncell / 4; i += blockDim.x) h4[i] = make_uint4(0, 0, 0, 0);
+    zero_bev_layers(A.out.bev_ci + (size_t)s * ncell * 2, A.out.bev_height + (size_t)s * ncell, ncell, threadIdx.x, blockDim.x);
     uint32_t* st = reinterpret_cast<uint32_t*>(ws + T.splitstats_off) + (size_t)s * MSC_STATS_STRIDE;
     if (threadIdx.x < MSC_STATS_STRIDE) st[threadIdx.x] = 0u;
     unsigned long long* scr = reinterpret_cast<unsigned long long*>(ws + T.boxscr_off);
@@ -297,7 +253,7 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
     const int n_inner = L.inner_dim * L.inner_dim;
 
     if (lane == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar_s), "r"(1) : "memory");
+        mbar_init(bar_s, 1);
         mbar_fence_init();
     }
     uint32_t wk = 0;  // tiles this warp has consumed since launch: mbarrier parity = wk & 1
@@ -367,14 +323,7 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
             const uint32_t npts = min((uint32_t)TP, s_cnt - first);
             const uint32_t bytes = (npts * 20u + 15u) & ~15u;
             const float* src = A.in.points + ((size_t)s_base + first) * 5;
-            if (lane == 0) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_s), "r"(bytes) : "memory");
-                asm volatile(
-                    "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-                        ring_s),
-                    "l"(src), "r"(bytes), "r"(bar_s), "l"(policy)
-                    : "memory");
-            }
+            if (lane == 0) bulk_load(ring_s, src, bytes, bar_s, policy);
         };
         bool more = t < lr1;
         if (more) { seek_sweep(); issue(); }  // overlaps the prologue below
@@ -427,12 +376,8 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
             for (int i = tid; i < n_boxes * kAccWords; i += NT) boxacc[i] = ((i % kAccWords) == 1) ? 0x7f800000u : 0u;
             const float4* bsrc = reinterpret_cast<const float4*>(g_boxprep + (size_t)bx0 * kBoxStride);
             for (int i = tid; i < n_boxes * (kBoxStride / 4); i += NT) reinterpret_cast<float4*>(boxp)[i] = bsrc[i];
-            if (n_parts == 1) {  // zero-fill this sample's global layers (a straddling sample was zero-filled by stream4_straddle_kernel)
-                uint4* c4 = reinterpret_cast<uint4*>(g_ci);
-                for (size_t i = tid; i < ncell / 2; i += NT) c4[i] = make_uint4(0, 0, 0, 0);
-                uint4* h4 = reinterpret_cast<uint4*>(g_h);
-                for (size_t i = tid; i < ncell / 4; i += NT) h4[i] = make_uint4(0, 0, 0, 0);
-            }
+            // zero-fill this sample's global layers (a straddling sample was zero-filled by stream4_straddle_kernel)
+            if (n_parts == 1) zero_bev_layers(g_ci, g_h, ncell, tid, NT);
         }
         __threadfence();
         __syncthreads();  // class tables are in smem
@@ -446,15 +391,11 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
             int e = -1;  // edge tested by this entry
             if (code >= 1 && code <= 2 * MSC_MAX_CAMS) e = second ? -1 : code - 1;
             else if (code >= 17 && code < 17 + kS4PairCodes && misc->pairs[code - 17]) e = (int)((misc->pairs[code - 17] >> (second ? 4 : 0)) & 0xfu);
-            S4Edge E;
-            E.ax = 0.0f; E.ay = 0.0f; E.a = __int_as_float(0x7fc00000); E.b = 0.0f;  // pad: the test fails
+            float4 E = make_float4(0.0f, 0.0f, __int_as_float(0x7fc00000), 0.0f);  // pad: the test fails
             uint2 inc = make_uint2(0u, 0u);
             const int c = e & (MSC_MAX_CAMS - 1);
             if (FOV && e >= 0 && c < n_cams) {
-                const float* wq = misc->wq + c * 6;
-                // cr = fma(a, qy, -(b * qx)) >= 0 with (a, b) = (w4, w5) for a right edge, (-w2, -w3) for a left one  (in_wedge)
-                E.ax = wq[0]; E.ay = wq[1];
-                if (e >= MSC_MAX_CAMS) { E.a = -wq[2]; E.b = -wq[3]; } else { E.a = wq[4]; E.b = wq[5]; }
+                E = wedge_edge_entry(misc->wq + c * 6, e >= MSC_MAX_CAMS);
                 inc.x = c < 4 ? 1u << (8 * c) : 0u;
                 inc.y = c < 4 ? 0u : 1u << (8 * (c - 4));
             }
@@ -476,25 +417,17 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
         // (The 80-register shape drains 32 entries at a time, one per lane: eight 128-bit loads in flight per lane do not fit.)
         constexpr uint32_t kDrain = PPT == 4 ? 64u : 32u;
         auto drain_queue = [&](uint32_t n_take) {  // n_take <= kDrain
-            const float4 e0 = s4_lds128(queue_s + (((q_head + (uint32_t)lane) & (uint32_t)(kS4QueueEntries - 1)) << 4));
+            const float4 e0 = lds128(queue_s + (((q_head + (uint32_t)lane) & (uint32_t)(kS4QueueEntries - 1)) << 4));
             float4 e1 = e0;
-            if (kDrain == 64u) e1 = s4_lds128(queue_s + (((q_head + 32u + (uint32_t)lane) & (uint32_t)(kS4QueueEntries - 1)) << 4));
+            if (kDrain == 64u) e1 = lds128(queue_s + (((q_head + 32u + (uint32_t)lane) & (uint32_t)(kS4QueueEntries - 1)) << 4));
             uint32_t ids0 = (uint32_t)lane < n_take ? __float_as_uint(e0.w) : kCullEmpty;
             uint32_t ids1 = (kDrain == 64u && (uint32_t)lane + 32u < n_take) ? __float_as_uint(e1.w) : kCullEmpty;
-            // centroid sums: one 32-bit word per axis plus a carry word that takes a rare second atomic when the word wraps
-            // (the coordinate is a 24-bit value, so that is at most once per 256 points); still order-independent integers
             auto accumulate = [&](int b, const float4& e) {
                 const float es2 = __fadd_rn(__fmul_rn(e.x, e.x), __fmul_rn(e.y, e.y));
                 const uint32_t fx = (uint32_t)(__float2int_rn(__fmul_rn(e.x, A.cscale)) + A.centroid_bias);
                 const uint32_t fy = (uint32_t)(__float2int_rn(__fmul_rn(e.y, A.cscale)) + A.centroid_bias);
                 const uint32_t fz = (uint32_t)(__float2int_rn(__fmul_rn(e.z, A.cscale)) + A.centroid_bias);
-                const uint32_t acc_s = smem_s + (uint32_t)L.boxacc_off + (uint32_t)b * (uint32_t)(kAccWords * 4);
-                s4_red_add(acc_s, 1u);
-                asm volatile("red.shared.min.u32 [%0], %1;" ::"r"(acc_s + 4u), "r"(__float_as_uint(es2)) : "memory");
-                const uint32_t ox = s4_atom_add(acc_s + 8u, fx), oy = s4_atom_add(acc_s + 12u, fy), oz = s4_atom_add(acc_s + 16u, fz);
-                if (ox > ~fx) s4_red_add(acc_s + 20u, 1u);
-                if (oy > ~fy) s4_red_add(acc_s + 24u, 1u);
-                if (oz > ~fz) s4_red_add(acc_s + 28u, 1u);
+                box_accumulate(smem_s + (uint32_t)L.boxacc_off + (uint32_t)b * (uint32_t)(kAccWords * 4), __float_as_uint(es2), fx, fy, fz);
             };
             int hit0 = -1, hit1 = -1;
             const bool crowded0 = ids0 == kCullAll, crowded1 = ids1 == kCullAll;  // more than four boxes touch the cell: test every box (below)
@@ -523,35 +456,10 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                     if (crowded1 && box_contains(boxp, b, e1.x, e1.y, e1.z)) { if (hit1 >= 0) accumulate(b, e1); else hit1 = b; }
                 }
             }
-#if MSC_S4_AGGREGATE
-            // lanes whose points lie in the same box reduce among themselves (count, nearest, three sums) and one of them updates the
-            // box's accumulators: the same integers, fewer same-address atomics
-            auto accumulate_grouped = [&](int hit, const float4& e) {
-                if (!__any_sync(0xffffffffu, hit >= 0)) return;
-                const uint32_t grp = __match_any_sync(0xffffffffu, hit);
-                const bool in = hit >= 0;
-                const float es2 = __fadd_rn(__fmul_rn(e.x, e.x), __fmul_rn(e.y, e.y));
-                const uint32_t fx = in ? (uint32_t)(__float2int_rn(__fmul_rn(e.x, A.cscale)) + A.centroid_bias) : 0u;
-                const uint32_t fy = in ? (uint32_t)(__float2int_rn(__fmul_rn(e.y, A.cscale)) + A.centroid_bias) : 0u;
-                const uint32_t fz = in ? (uint32_t)(__float2int_rn(__fmul_rn(e.z, A.cscale)) + A.centroid_bias) : 0u;
-                const uint32_t sx = __reduce_add_sync(grp, fx), sy = __reduce_add_sync(grp, fy), sz = __reduce_add_sync(grp, fz);  // < 2^30
-                const uint32_t mn = __reduce_min_sync(grp, __float_as_uint(es2));  // (es2 >= 0 or NaN-free: float order = unsigned order)
-                if (in && (uint32_t)lane == (uint32_t)__ffs((int)grp) - 1u) {
-                    const uint32_t acc_s = smem_s + (uint32_t)L.boxacc_off + (uint32_t)hit * (uint32_t)(kAccWords * 4);
-                    s4_red_add(acc_s, (uint32_t)__popc(grp));
-                    asm volatile("red.shared.min.u32 [%0], %1;" ::"r"(acc_s + 4u), "r"(mn) : "memory");
-                    const uint32_t ox = s4_atom_add(acc_s + 8u, sx), oy = s4_atom_add(acc_s + 12u, sy), oz = s4_atom_add(acc_s + 16u, sz);
-                    if (ox > ~sx) s4_red_add(acc_s + 20u, 1u);
-                    if (oy > ~sy) s4_red_add(acc_s + 24u, 1u);
-                    if (oz > ~sz) s4_red_add(acc_s + 28u, 1u);
-                }
-            };
-            accumulate_grouped(hit0, e0);
-            if (kDrain == 64u) accumulate_grouped(hit1, e1);
-#else
+            // (Aggregating the hits of one box over the warp first, __match_any_sync + __reduce_*_sync, is bit-identical and 76 % slower:
+            // DESIGN.md section 5.)
             if (hit0 >= 0) accumulate(hit0, e0);
             if (hit1 >= 0) accumulate(hit1, e1);
-#endif
             q_head += n_take;
         };
         // ---- exact cross products for the points of cells that image-column rays cross, 32 queued points at a time (one per lane): the
@@ -561,19 +469,19 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
         uint32_t e_head = 0, e_tail = 0;  // warp-uniform
         auto drain_edges = [&](uint32_t n_take) {  // n_take <= 32
             const uint32_t slot = (e_head + (uint32_t)lane) & (uint32_t)(kS4EdgeEntries - 1);
-            const uint2 pw = s4_lds64(eq_s + (slot << 3));
+            const uint2 pw = lds64(eq_s + (slot << 3));
             const float px = __uint_as_float(pw.x), py = __uint_as_float(pw.y);
-            const uint32_t code = (uint32_t)lane < n_take ? s4_lds8(eqc_s + slot) : 0u;
+            const uint32_t code = (uint32_t)lane < n_take ? lds8(eqc_s + slot) : 0u;
             {
-                const float4 E = s4_lds128(edge1_s + (code << 4));
-                const uint2 inc = s4_lds64(edge1_s + kInc1 + (code << 3));
+                const float4 E = lds128(edge1_s + (code << 4));
+                const uint2 inc = lds64(edge1_s + kInc1 + (code << 3));
                 const float qx = __fsub_rn(px, E.x), qy = __fsub_rn(py, E.y);
                 const float cr = __fmaf_rn(E.z, qy, -__fmul_rn(E.w, qx));
                 if (cr >= 0.0f) { cam_lo += inc.x; cam_hi += inc.y; }
             }
             if (__any_sync(0xffffffffu, code > 2u * MSC_MAX_CAMS)) {
-                const float4 E2 = s4_lds128(edge1_s + kEdge2 + (code << 4));
-                const uint2 inc2 = s4_lds64(edge1_s + kInc2 + (code << 3));
+                const float4 E2 = lds128(edge1_s + kEdge2 + (code << 4));
+                const uint2 inc2 = lds64(edge1_s + kInc2 + (code << 3));
                 const float qx2 = __fsub_rn(px, E2.x), qy2 = __fsub_rn(py, E2.y);
                 const float cr2 = __fmaf_rn(E2.z, qy2, -__fmul_rn(E2.w, qx2));
                 if (cr2 >= 0.0f) { cam_lo += inc2.x; cam_hi += inc2.y; }
@@ -589,7 +497,7 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                     while (und) {
                         const int e = __ffs((int)und) - 1;
                         und &= und - 1u;
-                        const float4 E = s4_lds128(edge1_s + ((uint32_t)(e + 1) << 4));
+                        const float4 E = lds128(edge1_s + ((uint32_t)(e + 1) << 4));
                         const float qx = __fsub_rn(px, E.x), qy = __fsub_rn(py, E.y);
                         const float cr = __fmaf_rn(E.z, qy, -__fmul_rn(E.w, qx));
                         if (!(cr >= 0.0f)) pass &= ~(1u << e);
@@ -605,8 +513,8 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
             if (++pstate == 255u) {  // spill the byte counters before any of them can wrap
 #pragma unroll
                 for (int c = 0; c < MSC_MAX_CAMS; ++c) {
-                    const uint32_t v = ((c < 4 ? cam_lo : cam_hi) >> ((c & 3) * 8)) & 0xffu;
-                    if (v) s4_red_add(misc_s + (uint32_t)offsetof(S4Misc, stats) + (uint32_t)(5 + c) * 4u, v);
+                    const uint32_t v = cam_byte(cam_lo, cam_hi, c);
+                    if (v) red_shared_add(misc_s + (uint32_t)offsetof(S4Misc, stats) + (uint32_t)(5 + c) * 4u, v);
                 }
                 cam_lo = cam_hi = pstate = 0;
             }
@@ -623,20 +531,7 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
             }
             // ---- the tile in flight becomes the current one
             const uint32_t npts = min((uint32_t)TP, s_cnt - ((t - s_tb) << TSH));
-            {
-                const uint32_t bar = bar_s, parity = wk & 1u;
-                asm volatile(
-                    "{\n"
-                    ".reg .pred p;\n"
-                    "MSC_S4WAIT_%=:\n"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-                    "@p bra MSC_S4DONE_%=;\n"
-                    "bra MSC_S4WAIT_%=;\n"
-                    "MSC_S4DONE_%=:\n"
-                    "}\n" ::"r"(bar),
-                    "r"(parity)
-                    : "memory");
-            }
+            mbar_wait_parity(bar_s, wk & 1u);
 #pragma unroll 1
           for (int sub = 0; sub < SUB; ++sub) {  // SUB passes of 32 * PPT rows over the slot
             // ---- phase A: branch-free over the lane's points so their dependency chains interleave.  Lane l owns rows l, l + 32, ... of
@@ -650,9 +545,9 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                 const bool partial = npts < (uint32_t)TP;  // (warp-uniform)
 #pragma unroll
                 for (int u = 0; u < PPT; ++u) {
-                    float x = __uint_as_float(s4_lds32(row_s + u * 640u));
-                    const float y = __uint_as_float(s4_lds32(row_s + u * 640u + 4u)), z = __uint_as_float(s4_lds32(row_s + u * 640u + 8u));
-                    const float inten = __uint_as_float(s4_lds32(row_s + u * 640u + 12u));
+                    float x = __uint_as_float(lds32(row_s + u * 640u));
+                    const float y = __uint_as_float(lds32(row_s + u * 640u + 4u)), z = __uint_as_float(lds32(row_s + u * 640u + 8u));
+                    const float inten = __uint_as_float(lds32(row_s + u * 640u + 12u));
                     // last tile of a sweep: rows past its end hold stale data -> NaN fails every compare below
                     if (partial && (uint32_t)lane + (uint32_t)(u + sub * PPT) * 32u >= npts) x = __int_as_float(0x7fc00000);
                     // A.1 remove_close (square, sweep's own sensor frame)
@@ -673,8 +568,8 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
 #pragma unroll
                 for (int r = 0; r < 3; ++r) {
                     double m0, m1, m2, m3;
-                    s4_lds_f64x2(pose_s + r * 32, m0, m1);
-                    s4_lds_f64x2(pose_s + r * 32 + 16, m2, m3);
+                    lds_f64x2(pose_s + r * 32, m0, m1);
+                    lds_f64x2(pose_s + r * 32 + 16, m2, m3);
 #pragma unroll
                     for (int u = 0; u < PPT; ++u) {
                         const float v = (float)__fma_rn(m0, xd[u], __fma_rn(m1, yd[u], __fma_rn(m2, zd[u], m3)));
@@ -703,15 +598,15 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                 uint32_t ix, iy;
                 s4_bev_cell_xy<FASTDIV>(xr[u], yr[u], P.bev_range, two_r, rcp_two_r, resf, (uint32_t)res_m1, ix, iy);
                 const uint32_t ci = (iy >> L.cull_shift) * (uint32_t)L.cull_dim + (ix >> L.cull_shift);
-                const uint32_t ids = s4_lds32(cull_s + (ci << 2));
+                const uint32_t ids = lds32(cull_s + (ci << 2));
                 const uint32_t wx = ix - (uint32_t)win_lo, wy = iy - (uint32_t)win_lo;
                 const bool inwin = max(wx, wy) < (uint32_t)win_w;
                 // ---- phase C: the atomic that counts the point returns its cell's edge code.  Window cells count into the window, cells
                 // outside it into their cull cell's word, dropped points into one of the lane's two sink words (code 0)
                 uint32_t wa = inwin ? wcount_s + ((wy * (uint32_t)win_stride + wx) << 2) : pcnt_s + (ci << 2);
                 wa = keep ? wa : (close[u] ? sink_close_s : sink_gate_s);
-                const uint32_t old = s4_atom_add(wa, 1u);
-                s4_red_add((keep && !inwin) ? sink_close_s + isum_delta : wa + isum_delta, q[u]);
+                const uint32_t old = atom_shared_add(wa, 1u);
+                red_shared_add((keep && !inwin) ? sink_close_s + isum_delta : wa + isum_delta, q[u]);
                 if (keep && zr[u] < P.ground_z) ++c_ground;  // lidar_agent.py:128
                 code[u] = old >> kS4CodeShift;
                 cand[u] = keep ? ids : kCullEmpty;
@@ -774,7 +669,7 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
         // share of the per-camera counts.
         uint32_t kept = 0, removed = 0, flags = 0, camc[MSC_MAX_CAMS];
 #pragma unroll
-        for (int c = 0; c < MSC_MAX_CAMS; ++c) camc[c] = FOV ? (((c < 4 ? cam_lo : cam_hi) >> ((c & 3) * 8)) & 0xffu) : 0u;
+        for (int c = 0; c < MSC_MAX_CAMS; ++c) camc[c] = FOV ? cam_byte(cam_lo, cam_hi, c) : 0u;
         if (tid < 32) removed = arrA[tid];
         for (int i = tid; i < n_cull; i += NT) {  // periphery points, per cull cell
             const uint32_t c0 = pcnt[i] & kS4CountMask;
@@ -878,12 +773,8 @@ __global__ void __launch_bounds__(s4_threads(PPT), 1) stream4_kernel(const __gri
                 float nearest = INFINITY, cen[3] = {0.0f, 0.0f, 0.0f};
                 if (cnt != 0) {
                     nearest = __fsqrt_rn(__uint_as_float(mn));
-                    const double den = (double)cnt * (double)A.cscale;
 #pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        const long long sum = (long long)sum3[k] - (long long)cnt * (long long)A.centroid_bias;
-                        cen[k] = (float)((double)sum / den);
-                    }
+                    for (int k = 0; k < 3; ++k) cen[k] = box_centroid(A, cnt, sum3[k]);
                 }
                 A.out.box_count[o] = cnt;
                 A.out.box_nearest[o] = nearest;

@@ -127,7 +127,7 @@ def load():
 
 DEFAULT_FUSED_CONFIG = 0    # auto (fused_evidence.cu: msc_fused_ctx::opt_config): stream4.cu (fused_stream.cu when fov_keep_mask != 0)
 FUSED_CONFIGS = (10, 7)     # forced: stream4.cu, fused_stream.cu
-DEFAULT_FUSED_PPT = 2       # stream4.cu launch shape: 2 points per lane (768 threads) or 4 (512 threads)
+DEFAULT_FUSED_PPT = 2       # stream4.cu launch shape: 2 points per lane (1024 threads) or 4 (512 threads)
 
 
 def check(status: int, what: str):

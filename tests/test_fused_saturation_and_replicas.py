@@ -39,7 +39,7 @@ def check_stats(st, ref_stats, ref_count, n_boxes, declared_boxes, p):
     (stream4.cu sizes its tables for at least 128, fused_stream.cu for the declared maximum); [14] and [15] are zero."""
     assert np.array_equal(st[:13], ref_stats[:13]), (st, ref_stats)
     w = _capi.get_option("last_window")
-    lo = (p.bev_res - w) // 2                    # stream4.cu s4_layout / fused_evidence.cu compute_layout
+    lo = (p.bev_res - w) // 2                    # stream4.cu s4_layout / fused_stream.cu stream_layout
     crowded = w > 0 and int(ref_count[lo:lo + w, lo:lo + w].max()) >= 65536
     room = max(declared_boxes, 128) if _capi.get_option("last_config") == 10 else max(declared_boxes, 1)
     want = (1 if crowded else 0) | ((1 << 31) if n_boxes > room else 0)

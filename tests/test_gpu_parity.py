@@ -246,7 +246,7 @@ def test_fused_static_partition_over_ctas(engine):
     empty = make_sample(32, n_sweeps=1, n_boxes=3)
     empty["lidar_sweeps"] = [dict(empty["lidar_sweeps"][0], points_raw=empty["lidar_sweeps"][0]["points_raw"][:0])]
     try:
-        for ppt in (4, 2):  # both launch shapes: 512 threads x 4 points per lane, 768 x 2
+        for ppt in (4, 2):  # both launch shapes: 512 threads x 4 points per lane, 1024 x 2
             _capi.set_option("ppt", ppt)
             for grid in (1, 2, 3, 7, 37, 148, 0):
                 _capi.set_option("grid", grid)

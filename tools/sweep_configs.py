@@ -11,7 +11,7 @@ from msc_geom.layout import pack_batch, tile_batch
 from msc_geom.engine import GeometryEngine
 from msc_geom import _capi
 
-configs = [tuple(int(v) for v in a.split(":")) for a in sys.argv[1:]] or [(7,), (9,)]
+configs = [tuple(int(v) for v in a.split(":")) for a in sys.argv[1:]] or [(7,), (10,)]
 n_unique = int(os.environ.get("SWEEP_UNIQUE", "8")); reps = int(os.environ.get("SWEEP_REPS", "74")); iters = int(os.environ.get("SWEEP_ITERS", "10"))
 eng = GeometryEngine()
 t0 = time.time()
