@@ -249,6 +249,41 @@ int msc_project_boxes(int32_t n_boxes, const double* boxes, int32_t n_cams, cons
                       const double* cam_calib, const double* cam_K, int32_t image_w, int32_t image_h,
                       uint8_t* visible, float* extent, void* stream);
 
+/*
+ * [EXT] row e7: LiDAR -> camera projection (devkit NuScenesExplorer.map_pointcloud_to_image), batched.  Per sample and camera a
+ * downsampled depth map -- the minimum depth of the returns that land in each ds x ds pixel block -- and per (box, camera) how much of
+ * the box's projected extent has LiDAR returns on it or in front of it.
+ * Points: the multi-sweep cloud of msc_aggregate_sweeps (remove_close in the sweep's frame, then the f64 fma transform into the keyframe
+ * LIDAR_TOP frame "ref"); no range or height gate.  Per (sample, camera) P = K [R | t] (3x4, f64 composed without FMA, rounded once to
+ * f32) maps ref to the image; a point lands in camera c iff w > min_dist and 1 < u < W-1 and 1 < v < H-1 (all strict), where
+ * (a, b, w) = P (x, y, z, 1) in f32 fmaf chains, u = a / w, v = b / w (IEEE division).  For nuScenes intrinsics (third row of K is
+ * (0, 0, 1)) w is the camera-frame depth.  The pixel is ((int)u, (int)v), its block (px / ds, py / ds); NaN rows land nowhere; a point
+ * may land in several cameras.  The normative definition is orc_camera_depth_sample / orc_box_depth_support of the test oracle.
+ * Outputs (every element is written by the call; the caller does not pre-fill):
+ *   depth       f32 [n_samples, n_cams, ceil(H/ds), ceil(W/ds)]: minimum w per block, +inf where no point lands;
+ *   cam_points  u32 [n_samples, n_cams]: points that land in the camera;
+ *   box_support u32 [n_boxes, n_cams, 4] (may be NULL): n_blocks, n_hit, n_front, n_on over the blocks of the box's clipped image
+ *               extent (the proj_visible / proj_extent of msc_project_boxes): blocks bx in [(int)umin / ds, min((int)umax, W-1) / ds],
+ *               likewise by; n_hit: finite depth; n_front: hit and (double)d < zlo - margin (something nearer hides the box);
+ *               n_on: other hits with (double)d <= zhi + margin, where zlo / zhi are the min / max camera-frame Z of the 8 corners
+ *               (f64).  All four are 0 for a box that is not visible.
+ * From msc_params only remove_close_radius, image_w, image_h and n_cams are used.  The results are bit-reproducible and independent of
+ * the launch shape (the depth minimum and the counts are order-independent integer reductions).  Stream-ordered: no host
+ * synchronisation, no allocation.  n_samples = 0 is a successful no-op.
+ */
+typedef struct {
+    float min_dist;       /* devkit map_pointcloud_to_image min_dist, 1.0; >= 0 */
+    int32_t downsample;   /* ds >= 1: pixel block edge of the depth map, 8 */
+    float support_margin; /* metres, >= 0, 0.5 */
+} msc_depth_params;
+typedef struct {
+    float* depth;
+    uint32_t* cam_points;
+    uint32_t* box_support; /* may be NULL */
+} msc_depth_out;
+int msc_camera_depth_batch(const msc_params* params, const msc_depth_params* dp, const msc_batch_in* in, const msc_depth_out* out,
+                           void* stream);
+
 /* Per-cluster axis-aligned metadata (lidar_agent.py:200-204): out [n_clusters, 11] f32 =
  * min3, max3, center3, distance, num_points.  labels: i32 per row of pts (-1 = noise). */
 int msc_cluster_aabb(const float* pts, uint32_t n, int32_t pitch, const int32_t* labels, int32_t n_clusters,

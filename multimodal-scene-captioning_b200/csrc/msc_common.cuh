@@ -91,10 +91,13 @@ __device__ __forceinline__ uint8_t bearing4(double dx, double dy) {
     return 3;
 }
 
-// box -> camera projection of one (box, camera) pair, devkit box_in_image(BoxVisibility.ANY) (App. A.3)
-__device__ __forceinline__ void project_box(const double* __restrict__ box, const double* __restrict__ cam_ego_pose,
-                                            const double* __restrict__ cam_calib, const double* __restrict__ K,
-                                            double W, double H, uint8_t* visible, float* extent4) {
+// box -> camera projection of one (box, camera) pair, devkit box_in_image(BoxVisibility.ANY) (App. A.3).
+// ZRANGE also returns the smallest and largest camera-frame Z of the 8 corners in zrange[0..1] (the LiDAR support of
+// csrc/camera_depth.cu); without it the body is the projection alone.
+template <bool ZRANGE>
+__device__ __forceinline__ void project_box_z(const double* __restrict__ box, const double* __restrict__ cam_ego_pose,
+                                              const double* __restrict__ cam_calib, const double* __restrict__ K,
+                                              double W, double H, uint8_t* visible, float* extent4, double* zrange) {
     double c[3] = {box[0], box[1], box[2]};
     double R[9];
     quat_to_rot(box + 6, R);
@@ -103,6 +106,7 @@ __device__ __forceinline__ void project_box(const double* __restrict__ box, cons
     const double hl = box[4] / 2.0, hw = box[3] / 2.0, hh = box[5] / 2.0;
     bool any_vis = false, all_front = true;
     double umin = INFINITY, vmin = INFINITY, umax = -INFINITY, vmax = -INFINITY;
+    double zlo = INFINITY, zhi = -INFINITY;
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
         const double lx = (k < 4) ? hl : -hl;
@@ -121,7 +125,12 @@ __device__ __forceinline__ void project_box(const double* __restrict__ box, cons
         if (u > umax) umax = u;
         if (v < vmin) vmin = v;
         if (v > vmax) vmax = v;
+        if (ZRANGE) {
+            if (Z < zlo) zlo = Z;
+            if (Z > zhi) zhi = Z;
+        }
     }
+    if (ZRANGE) { zrange[0] = zlo; zrange[1] = zhi; }
     bool ok = any_vis && all_front;
     *visible = ok ? 1 : 0;
     if (ok) {
@@ -133,6 +142,11 @@ __device__ __forceinline__ void project_box(const double* __restrict__ box, cons
     } else {
         extent4[0] = extent4[1] = extent4[2] = extent4[3] = 0.0f;
     }
+}
+__device__ __forceinline__ void project_box(const double* __restrict__ box, const double* __restrict__ cam_ego_pose,
+                                            const double* __restrict__ cam_calib, const double* __restrict__ K,
+                                            double W, double H, uint8_t* visible, float* extent4) {
+    project_box_z<false>(box, cam_ego_pose, cam_calib, K, W, H, visible, extent4, nullptr);
 }
 
 }  // namespace msc

@@ -20,6 +20,7 @@ class MscError(RuntimeError):
         self.status = status
 
 
+MSC_ERR_BAD_ARGUMENT = -1
 MSC_ERR_UNSUPPORTED = -3
 
 
@@ -47,6 +48,14 @@ class MscBatchOut(C.Structure):
         ("box_count", C.c_void_p), ("box_nearest", C.c_void_p), ("box_centroid", C.c_void_p), ("proj_visible", C.c_void_p),
         ("proj_extent", C.c_void_p), ("bev_ci", C.c_void_p), ("bev_height", C.c_void_p), ("stats", C.c_void_p),
     ]
+
+
+class MscDepthParams(C.Structure):
+    _fields_ = [("min_dist", C.c_float), ("downsample", C.c_int32), ("support_margin", C.c_float)]
+
+
+class MscDepthOut(C.Structure):
+    _fields_ = [("depth", C.c_void_p), ("cam_points", C.c_void_p), ("box_support", C.c_void_p)]
 
 
 class MscJpegComp(C.Structure):
@@ -89,6 +98,8 @@ _PROTOS = {
     "msc_relation_table_batch": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msc_project_boxes": (C.c_int, [C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
+    "msc_camera_depth_batch": (C.c_int, [C.POINTER(MscParams), C.POINTER(MscDepthParams), C.POINTER(MscBatchIn), C.POINTER(MscDepthOut),
+                                         C.c_void_p]),
     "msc_cluster_aabb": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "msc_dbscan_workspace_bytes": (C.c_size_t, [C.c_uint32, C.POINTER(C.c_int32)]),
     "msc_dbscan": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int32, C.c_double, C.c_int32, C.POINTER(C.c_double), C.c_double, C.POINTER(C.c_int32), C.c_void_p,

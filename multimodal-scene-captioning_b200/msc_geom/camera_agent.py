@@ -10,7 +10,7 @@ import numpy as np
 
 from . import ops
 from .engine import GeometryEngine
-from .layout import boxes_from_annotations
+from .layout import DepthParams, GeomParams, boxes_from_annotations
 
 
 def projection_evidence(engine: GeometryEngine, sample: Dict[str, Any], image_size=(1600, 900)) -> Dict[str, Any]:
@@ -27,16 +27,42 @@ def projection_evidence(engine: GeometryEngine, sample: Dict[str, Any], image_si
     vis, ext = ops.project_boxes(engine, boxes, pose, calib, K, image_size[0], image_size[1])
     out: Dict[str, Any] = {}
     for ci, c in enumerate(cams):
-        rows = [{"annotation": i, "category": anns[i].get("category_name", "unknown"), "bbox": [round(float(v), 1) for v in ext[i, ci]]}
+        rows = [{"annotation": int(i), "category": anns[i].get("category_name", "unknown"), "bbox": [round(float(v), 1) for v in ext[i, ci]]}
                 for i in np.nonzero(vis[:, ci])[0]]
         out[c.get("channel", f"CAM_{ci}")] = {"visible_objects": len(rows), "objects": rows}
     return out
 
 
-def evidence_context(engine: GeometryEngine, sample: Dict[str, Any], image_size=(1600, 900)) -> Dict[str, Any]:
-    """The `context` argument for CameraAgent.process: the projection evidence under one key, JSON-serialisable."""
+def lidar_evidence(engine: GeometryEngine, sample: Dict[str, Any], dp: Optional[DepthParams] = None, image_size=(1600, 900)) -> Dict[str, Any]:
+    """[EXT] what LiDAR sees in each camera (devkit map_pointcloud_to_image over the sample's multi-sweep cloud, ops.camera_depth):
+    per camera the number of returns that land in the image and, per visible annotation, how many ds x ds pixel blocks its projected
+    box covers, how many of them hold returns, in how many the nearest return lies on the box (`on_object`) and in how many something
+    nearer hides it (`occluded`).  Needs the additive `cameras` key; returns {} for plain reference-style samples."""
+    cams = sample.get("cameras") or []
+    if not cams:
+        return {}
+    anns = sample.get("annotations") or []
+    res = ops.camera_depth(engine, sample, dp, GeomParams(image_w=image_size[0], image_h=image_size[1], n_cams=len(cams)))
+    sup = res["box_support"]
+    out: Dict[str, Any] = {}
+    for ci, c in enumerate(cams):
+        rows = [{"annotation": int(i), "category": anns[i].get("category_name", "unknown"), "blocks": int(sup[i, ci, 0]),
+                 "blocks_with_returns": int(sup[i, ci, 1]), "on_object": int(sup[i, ci, 3]), "occluded": int(sup[i, ci, 2])}
+                for i in np.nonzero(sup[:, ci, 0])[0]]
+        out[c.get("channel", f"CAM_{ci}")] = {"lidar_returns": int(res["cam_points"][ci]), "objects": rows}
+    return out
+
+
+def evidence_context(engine: GeometryEngine, sample: Dict[str, Any], image_size=(1600, 900), lidar: bool = False) -> Dict[str, Any]:
+    """The `context` argument for CameraAgent.process: the projection evidence under one key, JSON-serialisable.  lidar=True adds
+    lidar_evidence under "lidar_in_camera"."""
     ev = projection_evidence(engine, sample, image_size)
-    return {"box_projection": ev} if ev else {}
+    out = {"box_projection": ev} if ev else {}
+    if lidar:
+        lev = lidar_evidence(engine, sample, image_size=image_size)
+        if lev:
+            out["lidar_in_camera"] = lev
+    return out
 
 
 def split_camera_sections(response: str, camera_names: List[str]) -> Dict[str, str]:
@@ -71,9 +97,11 @@ class CameraAgent:
     reference renders any context (:43-47).  The VLM call is the injected `llm(messages, temperature=...)`; without one the reply is
     empty and every camera gets it, like the reference's unparsed-reply branch."""
 
-    def __init__(self, client, model: str, agent_name: str, engine: Optional[GeometryEngine] = None, llm: Optional[Callable[..., str]] = None):
+    def __init__(self, client, model: str, agent_name: str, engine: Optional[GeometryEngine] = None, llm: Optional[Callable[..., str]] = None,
+                 lidar: bool = False):
         self.client, self.model, self.agent_name = client, model, agent_name
         self.engine = engine
+        self.lidar = lidar  # opt-in: process(sample=...) also puts lidar_evidence into the context
         self.llm = llm
 
     def call_llm(self, messages, temperature: float = 0.7, **kw) -> str:
@@ -99,9 +127,10 @@ class CameraAgent:
         return content
 
     def process(self, images: List[np.ndarray], camera_names: List[str], context: Optional[Dict] = None, sample: Optional[Dict] = None) -> Dict[str, Any]:
-        """`sample` (additive): a loader sample with the `cameras` key; its projection evidence is merged into `context`."""
+        """`sample` (additive): a loader sample with the `cameras` key; its projection evidence is merged into `context` (for an agent
+        made with lidar=True also what LiDAR sees in each camera, lidar_evidence).  The parameter list stays the reference's."""
         if sample is not None and self.engine is not None:
-            context = {**(context or {}), **evidence_context(self.engine, sample)}
+            context = {**(context or {}), **evidence_context(self.engine, sample, lidar=self.lidar)}
         messages = [{"role": "user", "content": self.user_content(images, camera_names, context)}]
         response = self.call_llm(messages, temperature=0.3)
         return {"agent": self.agent_name, "modality": "camera", "camera_views": camera_names,

@@ -11,8 +11,8 @@ import numpy as np
 import torch
 
 from . import _capi
-from ._capi import MscBatchIn, MscBatchOut, MscParams
-from .layout import GeomParams, HostBatch, pack_batch
+from ._capi import MscBatchIn, MscBatchOut, MscDepthOut, MscDepthParams, MscParams
+from .layout import DepthParams, GeomParams, HostBatch, pack_batch
 
 _IN_FIELDS = ("points", "sample_sweep_off", "sweep_start", "sweep_count", "sweep_pose", "sample_box_off", "boxes", "ego_pose",
               "lidar_calib", "cam_ego_pose", "cam_calib", "cam_K")
@@ -121,6 +121,31 @@ class BatchResult:
             out["bev_isum_q"] = np.ascontiguousarray(ci[..., 1])
             out["bev_intensity_sum"] = (ci[..., 1].astype(np.float64) / float(1 << self.intensity_shift)).astype(np.float32)
             out["bev_height"] = self.bev_height.cpu().numpy()
+        return out
+
+
+@dataclass
+class DepthResult:
+    """Outputs of msc_camera_depth_batch ([EXT] row e7), still on the device.  Depth maps stay sharded like the BEV grids."""
+    n_samples: int
+    n_cams: int
+    image_w: int
+    image_h: int
+    downsample: int
+    sample_box_off: np.ndarray
+    depth: torch.Tensor                      # f32 [S, C, ceil(H/ds), ceil(W/ds)], +inf where no return lands
+    cam_points: torch.Tensor                 # u32 bits in i32 [S, C]
+    box_support: Optional[torch.Tensor]      # u32 bits in i32 [B, C, 4]: blocks, blocks with returns, in front, on the box; None: skipped
+
+    def struct(self) -> MscDepthOut:
+        return MscDepthOut(self.depth.data_ptr(), self.cam_points.data_ptr(),
+                           self.box_support.data_ptr() if self.box_support is not None else None)
+
+    def to_host(self) -> Dict[str, np.ndarray]:
+        out = {"depth": self.depth.cpu().numpy(), "cam_points": self.cam_points.cpu().numpy().view(np.uint32),
+               "sample_box_off": self.sample_box_off}
+        if self.box_support is not None:
+            out["box_support"] = self.box_support.cpu().numpy().view(np.uint32)
         return out
 
 
@@ -310,6 +335,44 @@ class GeometryEngine:
             _capi.check(self.lib.msc_fused_evidence_batch(self.ctx.handle, C.byref(mp), C.byref(bi), C.byref(bo), ws.data_ptr(), ws.numel(),
                                                           C.c_void_p(stream)), "msc_fused_evidence_batch")
         self.kernel_launches += self.ctx.get_option("last_launches")  # table kernels + the streaming kernel, counted by the library
+        return out
+
+    # ------------------------------------------------------------------ LiDAR -> camera projection ([EXT] e7)
+    def alloc_depth(self, hb: HostBatch, dp: Optional[DepthParams] = None, params: Optional[GeomParams] = None,
+                    box_support: bool = True) -> DepthResult:
+        """Output buffers of run_camera_depth for `hb` (image size and camera count from `params`); box_support=False skips the
+        per-box counts."""
+        p = params or self.params
+        dp = dp or DepthParams()
+        hbk, wbk = dp.block_shape(p.image_w, p.image_h)
+        d = self.device
+        S, Cn = hb.n_samples, p.n_cams
+        return DepthResult(S, Cn, p.image_w, p.image_h, int(dp.downsample), hb.sample_box_off.copy(),
+                           torch.empty((S, Cn, hbk, wbk), dtype=torch.float32, device=d), torch.empty((S, Cn), dtype=torch.int32, device=d),
+                           torch.empty((hb.n_boxes, Cn, 4), dtype=torch.int32, device=d) if box_support else None)
+
+    def run_camera_depth(self, db: DeviceBatch, out: Optional[DepthResult] = None, dp: Optional[DepthParams] = None,
+                         params: Optional[GeomParams] = None) -> DepthResult:
+        """Per-camera depth maps, per-camera return counts and per-(box, camera) LiDAR support of a device-resident batch
+        (msc_camera_depth_batch): the devkit's map_pointcloud_to_image over every sample's multi-sweep cloud, in one pass."""
+        p = params or self.params
+        dp = dp or DepthParams()
+        if p.n_cams != db.host.n_cams:
+            raise _capi.MscError(f"params.n_cams={p.n_cams} but the batch was packed for {db.host.n_cams} cameras")
+        if out is None:
+            out = self.alloc_depth(db.host, dp, p)
+        hbk, wbk = dp.block_shape(p.image_w, p.image_h)
+        if out.n_samples != db.host.n_samples or tuple(out.depth.shape) != (db.host.n_samples, p.n_cams, hbk, wbk) or (
+                out.box_support is not None and tuple(out.box_support.shape) != (db.host.n_boxes, p.n_cams, 4)):
+            raise _capi.MscError("run_camera_depth: the output buffers do not match the batch, parameters and downsample")
+        mp = make_params(p)
+        mdp = MscDepthParams(dp.min_dist, int(dp.downsample), dp.support_margin)
+        bi, bo = db.struct(), out.struct()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _capi.check(self.lib.msc_camera_depth_batch(C.byref(mp), C.byref(mdp), C.byref(bi), C.byref(bo), C.c_void_p(stream)),
+                    "msc_camera_depth_batch")
+        if db.host.n_samples > 0:  # fill + depth pass (+ the support scan)
+            self.kernel_launches += 2 + int(out.box_support is not None and db.host.n_boxes > 0)
         return out
 
     # ------------------------------------------------------------------ batched pairwise relation tables ([EXT] e6)

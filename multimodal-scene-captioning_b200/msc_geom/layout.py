@@ -44,6 +44,21 @@ class GeomParams:
         return sqrt_thresholds(self.range_min, self.range_max)
 
 
+@dataclass
+class DepthParams:
+    """Parameters of the [EXT] LiDAR -> camera projection (msc_camera_depth_batch).  Kept apart from GeomParams, whose values key the
+    fused path's parameter cache.  min_dist: devkit map_pointcloud_to_image's (m, >= 0); downsample: pixel block edge of the depth
+    maps; support_margin: metres of slack around a box's depth range when its blocks are classed as in front of / on the box."""
+    min_dist: float = 1.0
+    downsample: int = 8
+    support_margin: float = 0.5
+
+    def block_shape(self, image_w: int, image_h: int):
+        """(rows, columns) of one depth map."""
+        ds = max(int(self.downsample), 1)  # the library refuses downsample < 1
+        return (int(image_h) + ds - 1) // ds, (int(image_w) + ds - 1) // ds
+
+
 def boxes_from_annotations(annotations: List[dict]) -> np.ndarray:
     """(B,10) f64: translation, size (w,l,h), rotation (w,x,y,z) exactly as the loader's dicts hold them
     (nuscenes_loader.py:183-185)."""

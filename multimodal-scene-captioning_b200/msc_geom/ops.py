@@ -11,7 +11,7 @@ import torch
 
 from . import _capi
 from .engine import GeometryEngine, make_params
-from .layout import GeomParams
+from .layout import DepthParams, GeomParams, pack_batch
 
 
 def _stream(eng: GeometryEngine):
@@ -166,6 +166,18 @@ def project_boxes(eng: GeometryEngine, boxes: np.ndarray, cam_ego_pose: np.ndarr
                                           ext.data_ptr(), _stream(eng)), "msc_project_boxes")
     eng.kernel_launches += 1
     return vis.cpu().numpy(), ext.cpu().numpy()
+
+
+def camera_depth(eng: GeometryEngine, sample: dict, dp: Optional[DepthParams] = None, params: Optional[GeomParams] = None) -> Dict[str, np.ndarray]:
+    """[EXT] LiDAR -> camera projection of one loader sample (devkit map_pointcloud_to_image over its multi-sweep cloud): depth
+    [C, ceil(H/ds), ceil(W/ds)] f32 (minimum depth per ds x ds pixel block, +inf where no return lands), cam_points [C] u32 and
+    box_support [B, C, 4] u32 (blocks of the box's image extent, blocks with returns, blocks with a return in front of the box, blocks
+    whose nearest return lies on the box).  Cameras, image size and remove_close radius come from `params` (default: the engine's)."""
+    p = params or eng.params
+    hb = pack_batch([sample], n_cams=p.n_cams)
+    res = eng.run_camera_depth(eng.upload(hb), dp=dp, params=p)
+    out = res.to_host()
+    return {"depth": out["depth"][0], "cam_points": out["cam_points"][0], "box_support": out["box_support"]}
 
 
 def aggregate_sweeps(eng: GeometryEngine, sweeps, remove_close_radius: float = 1.0):

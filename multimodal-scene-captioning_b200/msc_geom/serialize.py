@@ -75,9 +75,11 @@ def jpeg_base64(img: np.ndarray) -> str:
 
 def ext_evidence(annotations: Sequence[Dict], box_count: np.ndarray, box_nearest: np.ndarray, box_centroid: np.ndarray,
                  proj_visible: np.ndarray, camera_names: Sequence[str], relations: Optional[Dict[str, Any]] = None,
-                 max_pairs: int = 20) -> Dict[str, Any]:
+                 max_pairs: int = 20, camera_support: Optional[np.ndarray] = None) -> Dict[str, Any]:
     """[EXT] evidence of one sample (rows e3, e5, e6 of SURVEY.md section 8a) as a JSON-serialisable dict: the `context` a caller
-    hands to CameraAgent.process / SceneGraphAgent.process.  Floats are rounded the way the reference rounds distances (1 decimal)."""
+    hands to CameraAgent.process / SceneGraphAgent.process.  Floats are rounded the way the reference rounds distances (1 decimal).
+    camera_support: the sample's box_support [B, C, 4] of msc_camera_depth_batch (row e7); adds per object "lidar_in_camera" with the
+    block counts of every camera the box is visible in."""
     objs = []
     for i, a in enumerate(annotations):
         n = int(box_count[i])
@@ -85,6 +87,10 @@ def ext_evidence(annotations: Sequence[Dict], box_count: np.ndarray, box_nearest
         objs.append({"id": f"obj_{i}", "category": str(a.get("category_name", "unknown")), "lidar_points": n,
                      "nearest_point_m": None if n == 0 else round(float(box_nearest[i]), 1),
                      "centroid": None if n == 0 else [round(float(v), 1) for v in box_centroid[i]], "visible_in": cams})
+        if camera_support is not None:
+            objs[-1]["lidar_in_camera"] = {camera_names[c]: {"blocks": int(camera_support[i, c, 0]), "blocks_with_returns": int(camera_support[i, c, 1]),
+                                                             "on_object": int(camera_support[i, c, 3]), "occluded": int(camera_support[i, c, 2])}
+                                           for c in range(len(camera_names)) if camera_support[i, c, 0]}
     out: Dict[str, Any] = {"objects": objs}
     if relations is not None:
         labels = relations.get("labels", ("ahead", "left", "behind", "right"))
