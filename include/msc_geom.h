@@ -308,6 +308,41 @@ size_t msc_dbscan_workspace_bytes(uint32_t n, const int32_t dims[3]);
 int msc_dbscan(const float* pts, uint32_t n, int32_t pitch, double eps, int32_t min_samples, const double origin[3], double cell,
                const int32_t dims[3], int32_t* labels, int32_t* n_clusters_host, void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * The reference's own LiDAR evidence (LiDARAgent.process up to the classifier, lidar_agent.py:103-209) for every sample of a packed
+ * batch in one stream-ordered call.  The keyframe of sample s is sweep sample_sweep_off[s] (raw rows, sensor frame); a sample without
+ * sweeps has an empty keyframe.  Per sample, bit-identical to the single-keyframe path run on that keyframe:
+ *   ground / object rows (x, y, z, intensity) in input order, as msc_keyframe_filter_split; counts [s] = kept, ground, object;
+ *   labels of the object rows, as msc_dbscan(eps, min_samples) (scikit-learn's labelling; points of different samples are never
+ *   neighbours), numbered per sample from 0;
+ *   the cluster table, as msc_cluster_aabb: record k of sample s at row object_off[s] + k (k < n_clusters[s] <= object rows), plus
+ *   cluster_first, the smallest object-row index (within the sample) labelled k, and noise_first[s], that of the first noise row
+ *   (-1: none).
+ * Only the keyframe's gate and split parameters of msc_params are used (range_min, range_max, z_min, z_max, ground_z); the DBSCAN grid
+ * is derived from them.  Row arrays are sized by row_capacity >= the batch's total keyframe rows; ground and object rows of sample s
+ * start at ground_off[s] / object_off[s].  status (device u32[1]) is written by the call: 0 on success, bit 0 if the component merge
+ * left an edge unmerged, bit 1 if the keyframes hold more than row_capacity rows (every sample then reads as empty).  A set bit means
+ * the results must not be used.  No host synchronisation, no allocation: workspace >= msc_lidar_batch_workspace_bytes(...), 256-byte
+ * aligned.  eps <= 0, min_samples < 1, NULL outputs or a short workspace: MSC_ERR_BAD_ARGUMENT.  n_samples = 0 is a successful no-op.
+ */
+typedef struct {
+    uint32_t row_capacity;
+    uint32_t* counts;         /* [n_samples, 3] kept, ground, object            */
+    uint32_t* ground_off;     /* [n_samples]                                     */
+    uint32_t* object_off;     /* [n_samples]                                     */
+    float* ground;            /* [row_capacity, 4]                               */
+    float* object;            /* [row_capacity, 4]                               */
+    int32_t* labels;          /* [row_capacity] per object row, -1 noise        */
+    int32_t* n_clusters;      /* [n_samples]                                     */
+    float* clusters;          /* [row_capacity, 11] min3 max3 center3 distance num_points */
+    int32_t* cluster_first;   /* [row_capacity]                                  */
+    int32_t* noise_first;     /* [n_samples]                                     */
+    uint32_t* status;         /* [1]                                             */
+} msc_lidar_batch_out;
+size_t msc_lidar_batch_workspace_bytes(const msc_params* params, double eps, int32_t n_samples, uint32_t row_capacity);
+int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, const msc_batch_in* in, const msc_lidar_batch_out* out,
+                    void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

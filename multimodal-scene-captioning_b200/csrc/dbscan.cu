@@ -14,7 +14,7 @@
 // relation -- and therefore every label -- is identical to scikit-learn's whenever scikit-learn uses a tree (n >= 12 points).
 // For n <= 11 scikit-learn brute-forces the neighbour search with a BLAS expansion |a|^2 - 2ab + |b|^2 that can drop a pair at
 // exactly eps; this file keeps the rule above there too, so labels can differ from scikit-learn's only through such pairs.
-#include "msc_common.cuh"
+#include "lidar_common.cuh"
 
 namespace msc {
 
@@ -95,12 +95,7 @@ __device__ __forceinline__ void for_each_neighbour(const float* __restrict__ pts
                 const uint32_t b = cell_start[c], e = b + cell_count[c];
                 for (uint32_t k = b; k < e; ++k) {
                     const uint32_t j = sorted[k];
-                    const float* q = pts + (size_t)j * pitch;
-                    const double dx = px - (double)q[0], dy = py - (double)q[1], dz = pz - (double)q[2];
-                    double d = dx * dx;
-                    d = d + dy * dy;
-                    d = d + dz * dz;
-                    if (d <= eps2) f(j);
+                    if (db_dist2(px, py, pz, pts + (size_t)j * pitch) <= eps2) f(j);
                 }
             }
 }
@@ -116,12 +111,6 @@ __global__ void __launch_bounds__(128) db_core_kernel(const float* __restrict__ 
     parent[i] = i;
 }
 
-__device__ __forceinline__ uint32_t db_find(const uint32_t* parent, uint32_t a) {
-    uint32_t p = ((const volatile uint32_t*)parent)[a];
-    while (p != a) { a = p; p = ((const volatile uint32_t*)parent)[a]; }
-    return a;
-}
-
 // one round of hooking over core-core edges: the larger root is hung under the smaller one (atomicMin), so a component's
 // root converges to its smallest index.  *changed is set when any hook happened.
 __global__ void __launch_bounds__(128) db_hook_kernel(const float* __restrict__ pts, uint32_t n, int pitch, DbscanGrid G, double eps2,
@@ -132,15 +121,7 @@ __global__ void __launch_bounds__(128) db_hook_kernel(const float* __restrict__ 
     if (i >= n || !core[i]) return;
     for_each_neighbour(pts, pitch, G, eps2, cell_start, cell_count, sorted, i, [&](uint32_t j) {
         if (j >= i || !core[j]) return;
-        uint32_t a = db_find(parent, i), b = db_find(parent, j);
-        while (a != b) {
-            const uint32_t hi = max(a, b), lo = min(a, b);
-            const uint32_t old = atomicMin(&parent[hi], lo);
-            *changed = 1u;
-            if (old == hi) break;   // hi was a root and now hangs under lo
-            a = db_find(parent, old);  // hi already had a smaller parent: merge that tree with lo
-            b = db_find(parent, lo);
-        }
+        db_union(parent, i, j, [&] { *changed = 1u; });
     });
 }
 

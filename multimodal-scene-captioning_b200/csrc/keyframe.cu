@@ -5,30 +5,9 @@
 // These are the latency path behind the drop-in LiDARAgent methods: one keyframe (35k points) at a time,
 // many CTAs per cloud, global (L2) atomics into an 800x800 grid that cannot be privatised in shared memory
 // (5 MB), order-preserving compaction through block counts + a scan + an ordered scatter.
-#include "msc_common.cuh"
+#include "lidar_common.cuh"
 
 namespace msc {
-
-constexpr int kCompactThreads = 1024;
-
-// monotonic float <-> uint mapping so integer atomicMin/Max order floats correctly (including negatives)
-__device__ __forceinline__ uint32_t f2ord(float f) {
-    uint32_t b = __float_as_uint(f);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(uint32_t u) {
-    uint32_t b = (u & 0x80000000u) ? (u & 0x7fffffffu) : ~u;
-    return __uint_as_float(b);
-}
-
-// lidar_agent.py:106-110 (float32, separate roundings, strict compares) and :128
-// split_only: _segment_ground alone (no gate; a NaN z compares false and lands in `object`, like pc[~mask])
-__device__ __forceinline__ uint32_t keyframe_class(const float* __restrict__ p, const msc_params& P, bool split_only) {
-    const float d = __fsqrt_rn(__fadd_rn(__fmul_rn(p[0], p[0]), __fmul_rn(p[1], p[1])));
-    const bool ok = split_only || ((d > P.range_min) && (d < P.range_max) && (p[2] < P.z_max) && (p[2] > P.z_min));
-    if (!ok) return 0u;
-    return (p[2] < P.ground_z) ? 1u : 2u;  // 1 ground, 2 object
-}
 
 // pass 1: per-block counts of kept / ground / object rows
 __global__ void __launch_bounds__(kCompactThreads) kf_count_kernel(const __grid_constant__ msc_params P, const float* __restrict__ pts,
@@ -241,16 +220,7 @@ __global__ void cluster_init_kernel(uint32_t* __restrict__ scratch11, int n_clus
 __global__ void cluster_finish_kernel(uint32_t* __restrict__ scratch11, int n_clusters) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n_clusters) return;
-    uint32_t* s = scratch11 + (size_t)c * 11;
-    float* o = reinterpret_cast<float*>(s);
-    float mn[3], mx[3];
-    const uint32_t cnt = s[10];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) { mn[k] = cnt ? ord2f(s[k]) : INFINITY; mx[k] = cnt ? ord2f(s[3 + k]) : -INFINITY; }
-#pragma unroll
-    for (int k = 0; k < 3; ++k) { o[k] = mn[k]; o[3 + k] = mx[k]; o[6 + k] = __fdiv_rn(__fadd_rn(mn[k], mx[k]), 2.0f); }  // :203
-    o[9] = __fsqrt_rn(__fadd_rn(__fmul_rn(o[6], o[6]), __fmul_rn(o[7], o[7])));                                             // :204
-    o[10] = (float)cnt;
+    cluster_finish(scratch11 + (size_t)c * 11);
 }
 
 // ---------------------------------------------------------------- materialised multi-sweep aggregation (App. A.1)

@@ -58,6 +58,12 @@ class MscDepthOut(C.Structure):
     _fields_ = [("depth", C.c_void_p), ("cam_points", C.c_void_p), ("box_support", C.c_void_p)]
 
 
+class MscLidarBatchOut(C.Structure):
+    _fields_ = [("row_capacity", C.c_uint32), ("counts", C.c_void_p), ("ground_off", C.c_void_p), ("object_off", C.c_void_p), ("ground", C.c_void_p),
+                ("object", C.c_void_p), ("labels", C.c_void_p), ("n_clusters", C.c_void_p), ("clusters", C.c_void_p), ("cluster_first", C.c_void_p),
+                ("noise_first", C.c_void_p), ("status", C.c_void_p)]
+
+
 class MscJpegComp(C.Structure):
     _fields_ = [("h", C.c_int32), ("v", C.c_int32), ("blocks_x", C.c_int32), ("blocks_y", C.c_int32), ("ds_w", C.c_int32), ("ds_h", C.c_int32),
                 ("coef_off", C.c_int64), ("plane_off", C.c_int64), ("qt", C.c_uint16 * 64)]
@@ -104,6 +110,9 @@ _PROTOS = {
     "msc_dbscan_workspace_bytes": (C.c_size_t, [C.c_uint32, C.POINTER(C.c_int32)]),
     "msc_dbscan": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int32, C.c_double, C.c_int32, C.POINTER(C.c_double), C.c_double, C.POINTER(C.c_int32), C.c_void_p,
                              C.POINTER(C.c_int32), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "msc_lidar_batch_workspace_bytes": (C.c_size_t, [C.POINTER(MscParams), C.c_double, C.c_int32, C.c_uint32]),
+    "msc_lidar_batch": (C.c_int, [C.POINTER(MscParams), C.c_double, C.c_int32, C.POINTER(MscBatchIn), C.POINTER(MscLidarBatchOut), C.c_void_p,
+                                  C.c_size_t, C.c_void_p]),
     "msc_jpeg_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc)]),
     "msc_jpeg_entropy_decode_host": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc), C.c_void_p]),
     "msc_jpeg_reconstruct": (C.c_int, [C.POINTER(MscJpegDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

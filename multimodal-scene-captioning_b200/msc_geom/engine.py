@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _capi
-from ._capi import MscBatchIn, MscBatchOut, MscDepthOut, MscDepthParams, MscParams
+from ._capi import MscBatchIn, MscBatchOut, MscDepthOut, MscDepthParams, MscLidarBatchOut, MscParams
 from .layout import DepthParams, GeomParams, HostBatch, pack_batch
 
 _IN_FIELDS = ("points", "sample_sweep_off", "sweep_start", "sweep_count", "sweep_pose", "sample_box_off", "boxes", "ego_pose",
@@ -147,6 +147,75 @@ class DepthResult:
         if self.box_support is not None:
             out["box_support"] = self.box_support.cpu().numpy().view(np.uint32)
         return out
+
+
+@dataclass
+class LidarBatchResult:
+    """Outputs of msc_lidar_batch (the reference's keyframe evidence for every sample of a batch), still on the device.  `small` holds
+    the status word and the per-sample tables in one buffer, so reading them is one copy."""
+    n_samples: int
+    row_capacity: int
+    small: torch.Tensor          # i32 [1 + 7 S]: status, counts [S, 3], ground_off, object_off, n_clusters, noise_first
+    ground: torch.Tensor         # f32 [cap, 4]; sample s at ground_off[s]
+    object: torch.Tensor         # f32 [cap, 4]; sample s at object_off[s]
+    labels: torch.Tensor         # i32 [cap] per object row, numbered per sample, -1 noise
+    clusters: torch.Tensor       # f32 [cap, 11]; cluster k of sample s at object_off[s] + k
+    cluster_first: torch.Tensor  # i32 [cap] smallest object row (within the sample) of that cluster
+
+    def _view(self, k: int, n: int) -> torch.Tensor:
+        return self.small[1 + k * self.n_samples: 1 + (k + n) * self.n_samples]
+
+    @property
+    def counts(self) -> torch.Tensor:
+        return self._view(0, 3).view(self.n_samples, 3)
+
+    @property
+    def ground_off(self) -> torch.Tensor:
+        return self._view(3, 1)
+
+    @property
+    def object_off(self) -> torch.Tensor:
+        return self._view(4, 1)
+
+    def struct(self) -> MscLidarBatchOut:
+        p = lambda t: t.data_ptr() or None
+        return MscLidarBatchOut(self.row_capacity, p(self.counts), p(self.ground_off), p(self.object_off), p(self.ground), p(self.object),
+                                p(self.labels), p(self._view(5, 1)), p(self.clusters), p(self.cluster_first), p(self._view(6, 1)),
+                                p(self.small[:1]))
+
+    def to_host(self) -> List[Dict[str, np.ndarray]]:
+        """Per sample: ground / object rows (n, 4) f32 and where they start in the device buffers, counts (kept, ground, object), labels of the object rows (int64, like
+        ops.dbscan), clusters (n_clusters, 11) f32 as ops.cluster_aabb, cluster_first (n_clusters,) and noise_first (-1: no noise row).
+        This is the synchronisation point; a set status word raises MscError."""
+        S = self.n_samples
+        small = self.small.cpu().numpy()
+        status = int(small[0]) if small.size else 0
+        if status:
+            why = []
+            if status & 1:
+                why.append("the component merge left an edge unmerged")
+            if status & 2:
+                why.append("the keyframes hold more rows than row_capacity (%d)" % self.row_capacity)
+            raise _capi.MscError("msc_lidar_batch: status 0x%x: %s" % (status, "; ".join(why)), status)
+        tab = small[1:].reshape(7, S) if S else np.zeros((7, 0), np.int32)
+        counts = tab[0:3].reshape(S, 3).astype(np.int64)
+        goff, ooff, ncl, nfirst = (tab[k].astype(np.int64) for k in (3, 4, 5, 6))
+        G, M = int(counts[:, 1].sum()), int(counts[:, 2].sum())
+        ground, obj = self.ground[:G].cpu().numpy(), self.object[:M].cpu().numpy()
+        labels, clusters, first = self.labels[:M].cpu().numpy(), self.clusters[:M].cpu().numpy(), self.cluster_first[:M].cpu().numpy()
+        out = []
+        for s in range(S):
+            g0, o0, ng, no, k = goff[s], ooff[s], counts[s, 1], counts[s, 2], ncl[s]
+            out.append({"counts": counts[s], "ground_off": int(g0), "object_off": int(o0), "ground": ground[g0:g0 + ng], "object": obj[o0:o0 + no], "labels": labels[o0:o0 + no].astype(np.int64),
+                        "clusters": clusters[o0:o0 + k], "cluster_first": first[o0:o0 + k], "noise_first": int(nfirst[s])})
+        return out
+
+
+def keyframe_rows(hb: HostBatch) -> int:
+    """Total keyframe rows of a batch (sweep sample_sweep_off[s] of every sample that has sweeps): the row capacity of run_lidar."""
+    sso = hb.sample_sweep_off
+    first = sso[:-1][sso[1:] > sso[:-1]]
+    return int(hb.sweep_count[first].astype(np.int64).sum())
 
 
 class InputArena:
@@ -373,6 +442,36 @@ class GeometryEngine:
                     "msc_camera_depth_batch")
         if db.host.n_samples > 0:  # fill + depth pass (+ the support scan)
             self.kernel_launches += 2 + int(out.box_support is not None and db.host.n_boxes > 0)
+        return out
+
+    # ------------------------------------------------------------------ the reference's keyframe evidence, batched
+    def alloc_lidar(self, hb: HostBatch) -> LidarBatchResult:
+        """Output buffers of run_lidar for `hb`: row arrays sized by the batch's total keyframe rows (known on the host)."""
+        S, cap, d = hb.n_samples, keyframe_rows(hb), self.device
+        return LidarBatchResult(S, cap, torch.zeros(1 + 7 * S, dtype=torch.int32, device=d), torch.empty((cap, 4), dtype=torch.float32, device=d),
+                                torch.empty((cap, 4), dtype=torch.float32, device=d), torch.empty(cap, dtype=torch.int32, device=d),
+                                torch.empty((cap, 11), dtype=torch.float32, device=d), torch.empty(cap, dtype=torch.int32, device=d))
+
+    def run_lidar(self, db: DeviceBatch, out: Optional[LidarBatchResult] = None, params: Optional[GeomParams] = None, eps: float = 0.5,
+                  min_samples: int = 10) -> LidarBatchResult:
+        """The reference's LiDAR evidence for every sample of a device-resident batch in one stream-ordered call (msc_lidar_batch): the
+        keyframe filter and ground split, DBSCAN(eps, min_samples) over each sample's object rows and the per-cluster boxes.  Only the
+        gate / split parameters of `params` are used (LiDARAgent._params()).  Nothing is synchronised; out.to_host() reads the results."""
+        p = params or self.params
+        hb = db.host
+        if out is None:
+            out = self.alloc_lidar(hb)
+        if out.n_samples != hb.n_samples or out.row_capacity < keyframe_rows(hb):
+            raise _capi.MscError("run_lidar: the output buffers do not match the batch")
+        mp = make_params(p)
+        need = int(self.lib.msc_lidar_batch_workspace_bytes(C.byref(mp), C.c_double(float(eps)), hb.n_samples, out.row_capacity))
+        ws = torch.empty(max(need, 256), dtype=torch.uint8, device=self.device)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        bi, bo = db.struct(), out.struct()
+        _capi.check(self.lib.msc_lidar_batch(C.byref(mp), C.c_double(float(eps)), int(min_samples), C.byref(bi), C.byref(bo), ws.data_ptr(),
+                                             need, C.c_void_p(stream)), "msc_lidar_batch")
+        if hb.n_samples > 0:
+            self.kernel_launches += 15  # 13 own kernels + the CUB sort and scan (each of those launches several kernels of its own)
         return out
 
     # ------------------------------------------------------------------ batched pairwise relation tables ([EXT] e6)

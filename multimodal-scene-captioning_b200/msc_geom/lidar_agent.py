@@ -16,13 +16,13 @@ from __future__ import annotations
 
 import json
 from dataclasses import dataclass
-from typing import Any, Callable, Dict, List, Optional, Tuple
+from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
 from . import ops
-from .engine import GeometryEngine
-from .layout import GeomParams
+from .engine import DeviceBatch, GeometryEngine
+from .layout import GeomParams, pack_batch
 
 DIRECTION_LABELS = ("front_right", "front", "front_left", "left", "back_left", "back", "back_right", "right")
 
@@ -108,6 +108,22 @@ def cluster_mosaic(images: List[np.ndarray]) -> np.ndarray:
     return sheet
 
 
+def set_order(cluster_first, noise_first: int) -> List[int]:
+    """The cluster labels (noise excluded) in the order `s = set(labels); s.discard(-1)` iterates them (lidar_agent.py:154-159), from
+    each label's first row alone: cluster_first[k] is the smallest index of a row labelled k (a sequence over k = 0..K-1, or a dict
+    label -> row), noise_first that of the first noise row (-1: none).  CPython lays a set out from the sequence of NEW keys inserted, so
+    set(labels) iterates like the set of the distinct labels inserted in first-appearance order -- noise included, since -1 takes a slot
+    before it is discarded.  O(K log K), with no pass over the labels."""
+    items = cluster_first.items() if isinstance(cluster_first, dict) else enumerate(cluster_first)
+    firsts = [(int(f), int(k)) for k, f in items]
+    if noise_first >= 0:
+        firsts.append((int(noise_first), -1))
+    firsts.sort()
+    uniq = set(label for _, label in firsts)
+    uniq.discard(-1)
+    return list(uniq)
+
+
 class LiDARAgent:
     def __init__(self, client, model: str, agent_name: str, engine: Optional[GeometryEngine] = None,
                  llm: Optional[Callable[..., str]] = None, cluster_classifier: Optional[Callable[..., List[dict]]] = None):
@@ -156,7 +172,11 @@ class LiDARAgent:
 
     def _cluster_metadata(self, object_points: np.ndarray, labels: np.ndarray, order: List[int]) -> List[dict]:
         n_clusters = int(labels.max()) + 1 if labels.size else 0
-        table = ops.cluster_aabb(self.engine, object_points, labels, n_clusters)
+        return self._metadata_of(ops.cluster_aabb(self.engine, object_points, labels, n_clusters), order)
+
+    @staticmethod
+    def _metadata_of(table: np.ndarray, order: List[int]) -> List[dict]:
+        """Cluster metadata (lidar_agent.py:198-209) of the clusters in `order` from their msc_cluster_aabb rows."""
         meta = []
         for i, lab in enumerate(order):
             row = table[lab]
@@ -180,10 +200,14 @@ class LiDARAgent:
         labels = labels.astype(np.int32)
         meta = self._cluster_metadata(object_points, labels, order)
         images = self._cluster_visualizations(object_points, labels, order)
+        return self._classified_objects(meta, lambda a, b: images[a:b])
+
+    def _classified_objects(self, meta: List[dict], images_of: Callable[[int, int], List[np.ndarray]]) -> List[DetectedObject]:
+        """The classifier loop of lidar_agent.py:189-239; images_of(a, b) gives the images of clusters a..b-1 of `meta`."""
         out: List[DetectedObject] = []
         for start in range(0, len(meta), 10):  # the reference classifies in batches of 10 (:189)
             batch = meta[start:start + 10]
-            cls = self._classify_batch_with_llm(images[start:start + 10], batch)
+            cls = self._classify_batch_with_llm(images_of(start, start + len(batch)), batch)
             for m, c in zip(batch, cls):
                 if c["category"] != "unknown" and c["confidence"] > 0.3:
                     out.append(DetectedObject(c["category"], m["center"], m["dimensions"], m["num_points"], m["distance"], m["direction"],
@@ -255,6 +279,47 @@ class LiDARAgent:
         kept, ground, obj = ops.keyframe_filter_split(self.engine, point_cloud, self._params())
         detected = self._detect_objects_3d(obj)
         bev = self._generate_multi_layer_bev(ground, obj)
+        return self._result(detected, ground, obj, bev, context)
+
+    def process_batch(self, samples: Optional[Sequence[dict]] = None, device_batch: Optional[DeviceBatch] = None,
+                      contexts: Optional[Sequence[Optional[Dict]]] = None) -> List[Dict[str, Any]]:
+        """[process(sample["point_cloud"], context) for each sample], with the filter, the ground split, DBSCAN and the cluster boxes of
+        every sample's keyframe (sweep 0) in one device pass (GeometryEngine.run_lidar).  `device_batch` (e.g. engine.upload of
+        io.stage_batch over lazy-loader samples, whose point_cloud is None) is used as it is; otherwise `samples` are packed and uploaded.
+        The classifier sees the same images, mosaics and metadata in the same order as process's; the 800 x 800 BEV, which only the
+        scene interpretation reads, is drawn only when an llm is injected, and cluster images only when a classifier is."""
+        eng = self.engine
+        if device_batch is None:
+            if samples is None:
+                raise ValueError("process_batch needs samples or a device_batch")
+            device_batch = eng.upload(pack_batch(list(samples), n_cams=eng.params.n_cams))
+        res = eng.run_lidar(device_batch, params=self._params(), eps=self.dbscan_eps, min_samples=self.dbscan_min_samples)
+        per = res.to_host()
+        contexts = list(contexts) if contexts is not None else [None] * len(per)
+        out = []
+        for s, r in enumerate(per):
+            ground, obj = r["ground"], r["object"]
+            detected: List[DetectedObject] = []
+            if len(obj) >= self.dbscan_min_samples:  # the guard of _detect_objects_3d
+                table = r["clusters"]
+                order = [l for l in set_order(r["cluster_first"], r["noise_first"]) if int(table[l, 10]) >= 5]
+                if order:
+                    labels = r["labels"]
+                    images_of = ((lambda a, b, obj=obj, labels=labels, order=order: self._cluster_visualizations(obj, labels, order[a:b]))
+                                 if self.cluster_classifier is not None else (lambda a, b: []))
+                    detected = self._classified_objects(self._metadata_of(table, order), images_of)
+            bev = None
+            if self.llm is not None:
+                res_px, rng = int(self.bev_resolution), self.bev_range
+                ng, no = len(ground), len(obj)
+                g0, o0 = r["ground_off"], r["object_off"]
+                count, height, sem = ops.keyframe_bev_layers_device(eng, res.ground[g0:g0 + ng], ng, res.object[o0:o0 + no], no, res_px, float(rng))
+                bev = finish_bev_layers(count, height, sem, res_px, rng)
+            out.append(self._result(detected, ground, obj, bev, contexts[s]))
+        return out
+
+    def _result(self, detected: List[DetectedObject], ground: np.ndarray, obj: np.ndarray, bev: Optional[Dict[str, np.ndarray]],
+                context: Optional[Dict]) -> Dict[str, Any]:
         features = self._extract_semantic_features(detected, ground, obj)
         report = self._generate_structured_report(features, detected)
         observations = self._scene_interpretation(report, bev, context)

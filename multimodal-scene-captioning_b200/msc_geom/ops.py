@@ -68,17 +68,24 @@ def keyframe_filter_split(eng: GeometryEngine, pc: np.ndarray, params: Optional[
 
 def keyframe_bev_layers(eng: GeometryEngine, ground: np.ndarray, obj: np.ndarray, res: int = 800, bev_range: float = 50.0):
     """Raster half of _generate_multi_layer_bev (lidar_agent.py:539-597): count u32, height f32, semantic BGR u8 (unflipped)."""
-    p = GeomParams(bev_res=res, bev_range=bev_range)
     d = eng.device
     g = torch.from_numpy(np.ascontiguousarray(ground[:, :4], np.float32)).to(d) if len(ground) else torch.zeros((1, 4), device=d)
     o = torch.from_numpy(np.ascontiguousarray(obj[:, :4], np.float32)).to(d) if len(obj) else torch.zeros((1, 4), device=d)
+    return keyframe_bev_layers_device(eng, g, len(ground), o, len(obj), res, bev_range)
+
+
+def keyframe_bev_layers_device(eng: GeometryEngine, ground: torch.Tensor, n_ground: int, obj: torch.Tensor, n_object: int, res: int = 800,
+                               bev_range: float = 50.0):
+    """keyframe_bev_layers on dense (n, 4) f32 device rows, e.g. one sample's slices of a LidarBatchResult."""
+    p = GeomParams(bev_res=res, bev_range=bev_range)
+    d = eng.device
     count = torch.empty((res, res), dtype=torch.int32, device=d)
     height = torch.empty((res, res), dtype=torch.float32, device=d)
     sem = torch.empty((res, res, 3), dtype=torch.uint8, device=d)
     winner = torch.empty((res, res), dtype=torch.int32, device=d)
     zr = torch.empty(2, dtype=torch.int32, device=d)
     mp = make_params(p)
-    _capi.check(eng.lib.msc_keyframe_bev(C.byref(mp), g.data_ptr(), len(ground), o.data_ptr(), len(obj), count.data_ptr(), height.data_ptr(),
+    _capi.check(eng.lib.msc_keyframe_bev(C.byref(mp), ground.data_ptr(), n_ground, obj.data_ptr(), n_object, count.data_ptr(), height.data_ptr(),
                                          sem.data_ptr(), winner.data_ptr(), zr.data_ptr(), _stream(eng)), "msc_keyframe_bev")
     eng.kernel_launches += 2
     return count.cpu().numpy().view(np.uint32), height.cpu().numpy(), sem.cpu().numpy()
