@@ -244,6 +244,23 @@ int msc_jpeg_entropy_decode_host(const uint8_t* jpeg_host, size_t nbytes, const 
  * planes: device scratch of desc->plane_bytes bytes. */
 int msc_jpeg_reconstruct(const msc_jpeg_desc* desc_host, const int16_t* coef, uint8_t* planes, uint8_t* out, void* stream);
 
+/*
+ * Camera-frame encode (CameraAgent._encode_image, camera_agent.py:128-137): image i of the batch becomes, byte for byte, the file
+ * `PIL.Image.fromarray(rgb[i]).save(buf, "JPEG", quality=quality)` writes -- libjpeg-turbo's default compression: JFIF 1.01, 4:2:0, the
+ * Annex K tables (quantisation scaled by jpeg_set_quality, standard Huffman tables), slow-integer FDCT, no restart markers.
+ * rgb: device [n_images][height][width][3] u8, contiguous.  The files go back to back into the device arena `out`; image i is
+ * out[out_off[i] .. out_off[i + 1]) (out_off: device i64[n_images + 1]).  status (device i32[1]) is written by the call: 0, or 1 when
+ * the files need more than out_bytes -- then nothing is written to `out`, but out_off is still exact, so out_off[n_images] is the arena
+ * size a second call needs.  Stream-ordered: no host synchronisation, no allocation; the results do not depend on the other images of the
+ * batch.  workspace: >= msc_jpeg_encode_workspace_bytes(...) bytes, 256-byte aligned (the size does not depend on out_bytes: each
+ * image's scan is packed in a region sized for its worst case before its stuffed size is known; 0 = arguments out of range).
+ * quality outside 1..100, height or width outside 1..65535, a NULL pointer with n_images > 0 or a short workspace: MSC_ERR_BAD_ARGUMENT
+ * before anything is launched.  n_images = 0 is a successful no-op.
+ */
+size_t msc_jpeg_encode_workspace_bytes(int32_t n_images, int32_t height, int32_t width, size_t out_bytes);
+int msc_jpeg_encode_batch(int32_t n_images, int32_t height, int32_t width, int32_t quality, const uint8_t* rgb, uint8_t* out, size_t out_bytes,
+                          int64_t* out_off, int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
+
 /* [EXT] standalone box -> camera projection (also fused into msc_fused_evidence_batch). */
 int msc_project_boxes(int32_t n_boxes, const double* boxes, int32_t n_cams, const double* cam_ego_pose,
                       const double* cam_calib, const double* cam_K, int32_t image_w, int32_t image_h,

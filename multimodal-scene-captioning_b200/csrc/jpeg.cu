@@ -11,6 +11,7 @@
 // files and other sampling layouts return MSC_ERR_UNSUPPORTED (nuScenes camera frames are baseline 4:2:0 JFIF).
 #include <vector>
 
+#include "jpeg_common.cuh"
 #include "msc_common.cuh"
 
 namespace msc {
@@ -108,9 +109,6 @@ struct BitReader {
     }
     void reset_to(const uint8_t* q) { p = q; acc = 0; n = 0; hit_marker = false; }
 };
-
-static const uint8_t kZigzag[64] = {0, 1, 8, 16, 9, 2, 3, 10, 17, 24, 32, 25, 18, 11, 4, 5, 12, 19, 26, 33, 40, 48, 41, 34, 27, 20, 13, 6, 7, 14, 21, 28,
-                                    35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23, 30, 37, 44, 51, 58, 59, 52, 45, 38, 31, 39, 46, 53, 60, 61, 54, 47, 55, 62, 63};
 
 struct ParsedJpeg {
     msc_jpeg_desc d;

@@ -116,6 +116,9 @@ _PROTOS = {
     "msc_jpeg_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc)]),
     "msc_jpeg_entropy_decode_host": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc), C.c_void_p]),
     "msc_jpeg_reconstruct": (C.c_int, [C.POINTER(MscJpegDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "msc_jpeg_encode_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_size_t]),
+    "msc_jpeg_encode_batch": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_size_t, C.c_void_p]),
     "msc_cluster_views": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 

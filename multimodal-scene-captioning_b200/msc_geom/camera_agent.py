@@ -3,10 +3,12 @@ its `process(images, camera_names, context=None)` JSON-dumps `context` into the 
 for the [EXT] box -> camera projection evidence built here (devkit get_sample_data + view_points + box_in_image, App. A.3)."""
 from __future__ import annotations
 
+import base64
 import json
 from typing import Any, Callable, Dict, List, Optional
 
 import numpy as np
+import torch
 
 from . import ops
 from .engine import GeometryEngine
@@ -114,16 +116,44 @@ class CameraAgent:
             return None
         return {"type": "text", "text": f"Context from other sensors:\n{json.dumps(context, indent=2)}\n\n"}
 
+    def device_jpegs(self, images: List[Any]) -> Dict[int, str]:
+        """Base64 JPEG of every (H, W, 3) frame of `images` (after the reference's uint8 conversion), encoded in one device call per frame
+        shape (ops.encode_jpeg_batch), keyed by position.  Other frames -- grayscale, RGBA -- are left to serialize.jpeg_base64."""
+        picked, where = [], []
+        for k, img in enumerate(images):
+            if isinstance(img, torch.Tensor) and img.is_cuda:
+                if img.dtype == torch.uint8 and img.dim() == 3 and img.shape[2] == 3:
+                    picked.append(img)
+                    where.append(k)
+                continue
+            a = np.asarray(img)
+            if a.dtype != np.uint8:
+                a = (a * 255).astype(np.uint8)
+            if a.ndim == 3 and a.shape[2] == 3:
+                picked.append(a)
+                where.append(k)
+        files = ops.encode_jpeg_batch(self.engine, picked, quality=85) if picked else []
+        return {k: base64.b64encode(f).decode() for k, f in zip(where, files)}
+
     def user_content(self, images: List[np.ndarray], camera_names: List[str], context: Optional[Dict] = None) -> List[Dict[str, Any]]:
+        """The reference's user message: the context block, the instruction, then every camera's name and base64 JPEG.  With an
+        engine, the (H, W, 3) frames are JPEG-encoded on the device in one batch, with the same bytes as Pillow's; `images` may then also
+        hold CUDA tensors (e.g. ops.decode_jpeg_batch(..., to_host=False)), so no raw frame crosses PCIe."""
         from . import serialize
         content = []
         block = self.context_block(context)
         if block:
             content.append(block)
         content.append({"type": "text", "text": f"Analyze all {len(camera_names)} camera views. For each view, provide detailed observations:\n\n"})
-        for img, name in zip(images, camera_names):
+        frames = list(zip(images, camera_names))
+        encoded = self.device_jpegs([img for img, _ in frames]) if self.engine is not None else {}
+        for k, (img, name) in enumerate(frames):
+            if k in encoded:
+                b64 = encoded[k]
+            else:
+                b64 = serialize.jpeg_base64(img.cpu().numpy() if self.engine is not None and isinstance(img, torch.Tensor) else img)
             content.append({"type": "text", "text": f"Camera: {name}"})
-            content.append({"type": "image_url", "image_url": {"url": f"data:image/jpeg;base64,{serialize.jpeg_base64(img)}", "detail": "low"}})
+            content.append({"type": "image_url", "image_url": {"url": f"data:image/jpeg;base64,{b64}", "detail": "low"}})
         return content
 
     def process(self, images: List[np.ndarray], camera_names: List[str], context: Optional[Dict] = None, sample: Optional[Dict] = None) -> Dict[str, Any]:

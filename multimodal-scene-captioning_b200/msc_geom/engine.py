@@ -211,6 +211,37 @@ class LidarBatchResult:
         return out
 
 
+JPEG_HEADER_BYTES = 625  # SOI .. SOS (623 bytes) and EOI of every file msc_jpeg_encode_batch writes
+
+
+@dataclass
+class JpegBatchResult:
+    """Files of msc_jpeg_encode_batch, still on the device: image i is arena[out_off[i] : out_off[i + 1]].  `small` holds the status
+    word and out_off in one buffer, so reading them is one copy."""
+    n_images: int
+    height: int
+    width: int
+    small: torch.Tensor       # i64 [n + 2]: status (low 32 bits of word 0), out_off [n + 1]
+    arena: torch.Tensor       # u8 [out_bytes]
+    workspace: torch.Tensor   # u8, msc_jpeg_encode_workspace_bytes
+    needed: Optional[int] = None  # arena bytes the last call needed, known after to_host()
+
+    @property
+    def out_off(self) -> torch.Tensor:
+        return self.small[1:]
+
+    def to_host(self) -> List[bytes]:
+        """The files as bytes.  This is the synchronisation point: one copy of status and offsets, then one copy of the used prefix of
+        the arena.  A set status word (the files need more than the arena) raises MscError with status 1 and the size they need."""
+        small = self.small.cpu().numpy()
+        off = small[1:].astype(np.int64)
+        self.needed = int(off[-1])
+        if int(small[0]) & 0xffffffff:
+            raise _capi.MscError("msc_jpeg_encode_batch: the files need %d bytes, the arena holds %d" % (self.needed, self.arena.numel()), 1)
+        data = self.arena[:self.needed].cpu().numpy().tobytes()
+        return [data[off[i]:off[i + 1]] for i in range(self.n_images)]
+
+
 def keyframe_rows(hb: HostBatch) -> int:
     """Total keyframe rows of a batch (sweep sample_sweep_off[s] of every sample that has sweeps): the row capacity of run_lidar."""
     sso = hb.sample_sweep_off
@@ -472,6 +503,38 @@ class GeometryEngine:
                                              need, C.c_void_p(stream)), "msc_lidar_batch")
         if hb.n_samples > 0:
             self.kernel_launches += 15  # 13 own kernels + the CUB sort and scan (each of those launches several kernels of its own)
+        return out
+
+    # ------------------------------------------------------------------ camera frames -> JPEG files (CameraAgent._encode_image)
+    def alloc_jpeg(self, n: int, h: int, w: int, out_bytes: Optional[int] = None) -> JpegBatchResult:
+        """Buffers of run_jpeg_encode for n frames of h x w: the file arena (default: half the raw RGB bytes plus header and EOI per
+        image), offsets and status, and the workspace."""
+        if out_bytes is None:
+            out_bytes = n * (h * w * 3 // 2 + JPEG_HEADER_BYTES)
+        need = int(self.lib.msc_jpeg_encode_workspace_bytes(n, h, w, out_bytes))
+        if need == 0:
+            raise _capi.MscError("alloc_jpeg: %d frames of %d x %d cannot be encoded in one call" % (n, h, w), _capi.MSC_ERR_BAD_ARGUMENT)
+        d = self.device
+        return JpegBatchResult(n, h, w, torch.zeros(n + 2, dtype=torch.int64, device=d), torch.empty(max(out_bytes, 1), dtype=torch.uint8, device=d),
+                               torch.empty(need, dtype=torch.uint8, device=d))
+
+    def run_jpeg_encode(self, images: torch.Tensor, quality: int = 85, out: Optional[JpegBatchResult] = None) -> JpegBatchResult:
+        """JPEG files of a device batch of RGB frames (uint8 [N, H, W, 3]), byte-identical to Pillow's save(..., "JPEG", quality=q), in
+        one stream-ordered call (msc_jpeg_encode_batch).  With `out` given nothing is allocated; out.to_host() reads the files."""
+        if not (isinstance(images, torch.Tensor) and images.is_cuda and images.dtype == torch.uint8 and images.dim() == 4 and images.shape[3] == 3):
+            raise _capi.MscError("run_jpeg_encode: images must be a uint8 CUDA tensor [N, H, W, 3]", _capi.MSC_ERR_BAD_ARGUMENT)
+        n, h, w = (int(v) for v in images.shape[:3])
+        if out is None:
+            out = self.alloc_jpeg(n, h, w)
+        if (out.n_images, out.height, out.width) != (n, h, w):
+            raise _capi.MscError("run_jpeg_encode: the output buffers do not match the batch", _capi.MSC_ERR_BAD_ARGUMENT)
+        images = images.contiguous()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _capi.check(self.lib.msc_jpeg_encode_batch(n, h, w, int(quality), images.data_ptr(), out.arena.data_ptr(), out.arena.numel(),
+                                                   out.out_off.data_ptr(), out.small.data_ptr(), out.workspace.data_ptr(), out.workspace.numel(),
+                                                   C.c_void_p(stream)), "msc_jpeg_encode_batch")
+        if n > 0:
+            self.kernel_launches += 6
         return out
 
     # ------------------------------------------------------------------ batched pairwise relation tables ([EXT] e6)

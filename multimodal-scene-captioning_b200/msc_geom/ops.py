@@ -4,7 +4,7 @@ are torch tensors that live for the duration of the call."""
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Tuple
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 import torch
@@ -329,3 +329,59 @@ def decode_jpeg_batch(eng: GeometryEngine, streams, threads: int = 8, to_host: b
 
 def decode_jpeg(eng: GeometryEngine, stream) -> np.ndarray:
     return decode_jpeg_batch(eng, [stream], threads=1)[0]
+
+
+def _jpeg_frame(img):
+    """One frame for encode_jpeg_batch: a uint8 (H, W, 3) CUDA tensor or host array; host arrays of another dtype are converted the way
+    the reference converts them, (img * 255).astype(np.uint8)."""
+    if isinstance(img, torch.Tensor) and img.is_cuda:
+        ok = img.dtype == torch.uint8 and img.dim() == 3 and img.shape[2] == 3
+    else:
+        img = img.numpy() if isinstance(img, torch.Tensor) else np.asarray(img)
+        if img.dtype != np.uint8:
+            img = (img * 255).astype(np.uint8)
+        ok = img.ndim == 3 and img.shape[2] == 3
+    if not ok:
+        raise _capi.MscError("encode_jpeg_batch: frames must be (H, W, 3) uint8, got %s %s" % (tuple(img.shape), img.dtype), _capi.MSC_ERR_BAD_ARGUMENT)
+    return img
+
+
+JPEG_WORKSPACE_PER_CALL = 4 << 30  # workspace bytes one device call of encode_jpeg_batch may use (a 1600 x 900 frame reserves 7.1 MB)
+
+
+def encode_jpeg_batch(eng: GeometryEngine, images, quality: int = 85) -> List[bytes]:
+    """JPEG files of RGB frames, byte-identical to `Image.fromarray(img).save(buf, "JPEG", quality=quality)` (CameraAgent._encode_image,
+    camera_agent.py:128-137), encoded on the device.  `images`: a list of host arrays or CUDA tensors, or one uint8 [N, H, W, 3] CUDA
+    tensor.  Frames are grouped by shape, one device call per shape and per JPEG_WORKSPACE_PER_CALL bytes of workspace (every frame
+    reserves room for its worst-case scan); a call whose files outgrow the default arena is encoded once more into an arena of the
+    exact size."""
+    if isinstance(images, torch.Tensor) and images.dim() == 4:
+        groups = {tuple(images.shape[1:3]): list(range(images.shape[0]))}
+        frames = images
+    else:
+        frames = [_jpeg_frame(img) for img in images]
+        groups = {}
+        for k, f in enumerate(frames):
+            groups.setdefault(tuple(f.shape[:2]), []).append(k)
+    out: List[Optional[bytes]] = [None] * len(frames)
+    for (h, w), group in groups.items():
+        per_frame = int(eng.lib.msc_jpeg_encode_workspace_bytes(1, h, w, 0))
+        step = max(1, JPEG_WORKSPACE_PER_CALL // per_frame) if per_frame else len(group)
+        for a in range(0, len(group), step):
+            idx = group[a:a + step]
+            if isinstance(frames, torch.Tensor):
+                batch = frames[idx[0]:idx[-1] + 1]
+            elif all(isinstance(frames[k], np.ndarray) for k in idx):
+                batch = torch.from_numpy(np.stack([frames[k] for k in idx])).to(eng.device)
+            else:
+                batch = torch.stack([frames[k] if isinstance(frames[k], torch.Tensor) else torch.from_numpy(frames[k]).to(eng.device) for k in idx])
+            res = eng.run_jpeg_encode(batch, quality)
+            try:
+                files = res.to_host()
+            except _capi.MscError as e:
+                if e.status != 1:
+                    raise
+                files = eng.run_jpeg_encode(batch, quality, out=eng.alloc_jpeg(len(idx), h, w, out_bytes=res.needed)).to_host()
+            for k, f in zip(idx, files):
+                out[k] = f
+    return out
