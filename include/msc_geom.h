@@ -318,9 +318,10 @@ int msc_cluster_views(const float* pts_xyzi, const uint32_t* order, const int32_
 
 /* DBSCAN with scikit-learn's labelling (reference call site LiDARAgent._detect_objects_3d, lidar_agent.py:148-153):
  * float64 neighbour relation, clusters numbered by their smallest core index, border points take the smallest adjacent
- * cluster number, noise = -1.  pts: rows of `pitch` floats (xyz first).  origin / cell / dims describe a host-chosen grid
- * of cubic cells (cell >= eps) covering the points.  labels: device i32[n]; n_clusters_host: host int.  SYNCHRONOUS on
- * `stream`.  workspace >= msc_dbscan_workspace_bytes(n, dims). */
+ * cluster number, noise = -1.  pts: rows of `pitch` floats (xyz first), n < 2^31 - 1.  origin / cell / dims describe a
+ * host-chosen grid of cubic cells (cell >= eps, fewer than 2^31 cells) covering the points; it sets only the width of the sorted
+ * cell keys, the workspace is O(n).  labels: device i32[n]; n_clusters_host: host int.  SYNCHRONOUS on `stream` (one host
+ * synchronisation).  workspace >= msc_dbscan_workspace_bytes(n, dims), which is 0 for n or dims out of range. */
 size_t msc_dbscan_workspace_bytes(uint32_t n, const int32_t dims[3]);
 int msc_dbscan(const float* pts, uint32_t n, int32_t pitch, double eps, int32_t min_samples, const double origin[3], double cell,
                const int32_t dims[3], int32_t* labels, int32_t* n_clusters_host, void* workspace, size_t workspace_bytes, void* stream);

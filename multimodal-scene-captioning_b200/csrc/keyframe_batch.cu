@@ -1,29 +1,17 @@
 // keyframe_batch.cu -- the reference's LiDAR evidence (keyframe filter + ground split, DBSCAN, per-cluster boxes; lidar_agent.py:103-209)
 // for every sample of a packed batch in one stream-ordered pass (DESIGN.md section 4.5).
 //
-// Per sample the results are those of the single-keyframe path (keyframe.cu, dbscan.cu) on the sample's keyframe; the device helpers
-// that define them (gate / split, neighbour relation, union-find, cluster-box arithmetic) are the same code, in lidar_common.cuh.
+// Per sample the results are those of msc_keyframe_filter_split, msc_dbscan and msc_cluster_aabb on the sample's keyframe: the gate /
+// split rule and the cluster-box arithmetic are the same code (lidar_common.cuh), and DBSCAN is the same pipeline (dbscan.cu).
 //   1. filter / split: 1024-row tiles of keyframe rows, never spanning two samples; per-tile counts, one exclusive scan over the tiles
 //      (tile order is sample order, so the scan also gives each sample's ground / object offset), an ordered scatter.
-//   2. DBSCAN over the object rows of all samples at once: 64-bit keys (sample, cell) sorted with CUB, cells found by binary search, so
-//      memory is O(object rows) whatever the number of samples; one hooking sweep, one verify sweep, flatten, an exclusive scan of the
-//      root flags (per-sample numbering = global rank minus the rank at the sample's first object row), labelling.
+//   2. DBSCAN over the object rows of all samples at once (db_enqueue).
 //   3. cluster table: ordered-int min / max, count and first row per (sample, cluster) slot object_off[s] + k, then the finish pass.
 #include "lidar_common.cuh"
 
 #include <cub/block/block_scan.cuh>
-#include <cub/device/device_radix_sort.cuh>
-#include <cub/device/device_scan.cuh>
 
 namespace msc {
-
-constexpr uint32_t kLbUnmerged = 1u, kLbOverflow = 2u;  // status bits (include/msc_geom.h)
-
-struct LbGrid {
-    double ox, oy, oz, inv_cell;
-    int nx, ny, nz;
-    uint64_t ncells;
-};
 
 // ---------------------------------------------------------------- 1. keyframe filter / split
 // one block of 256: keyframe rows per sample, tile offsets (exclusive scan of ceil(rows / 1024)), status and noise_first initialised
@@ -168,159 +156,9 @@ __global__ void __launch_bounds__(kCompactThreads) lb_scatter_kernel(const __gri
     }
 }
 
-// ---------------------------------------------------------------- 2. segmented DBSCAN
-__device__ __forceinline__ void lb_cell(const LbGrid& G, float4 p, int* cx, int* cy, int* cz) {
-    *cx = min(max((int)floor(((double)p.x - G.ox) * G.inv_cell), 0), G.nx - 1);
-    *cy = min(max((int)floor(((double)p.y - G.oy) * G.inv_cell), 0), G.ny - 1);
-    *cz = min(max((int)floor(((double)p.z - G.oz) * G.inv_cell), 0), G.nz - 1);
-}
-
-// key of every object row (rows past the batch's object count get the largest key, so they sort last)
-__global__ void __launch_bounds__(256) lb_key_kernel(const float4* __restrict__ object, const uint32_t* __restrict__ object_sample,
-                                                    const uint32_t* __restrict__ totals, uint32_t cap, LbGrid G, uint64_t pad_key,
-                                                    uint64_t* __restrict__ keys, uint32_t* __restrict__ vals) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= cap) return;
-    uint64_t k = pad_key;
-    if (i < totals[2]) {
-        int cx, cy, cz;
-        lb_cell(G, object[i], &cx, &cy, &cz);
-        k = (uint64_t)object_sample[i] * G.ncells + ((uint64_t)cz * G.ny + cy) * G.nx + cx;
-    }
-    keys[i] = k;
-    vals[i] = i;
-}
-
-// visit every neighbour j of object row i (same sample, squared distance <= eps2 in float64, x -> y -> z) and call f(j).  The three
-// cells along x of one (z, y) row are consecutive keys: one binary search per row, nine per point.
-template <class F>
-__device__ __forceinline__ void lb_for_each_neighbour(const float4* __restrict__ object, const LbGrid& G, double eps2, uint32_t s,
-                                                      const uint64_t* __restrict__ skey, const uint32_t* __restrict__ sidx, uint32_t m,
-                                                      uint32_t i, F f) {
-    const float4 p = object[i];
-    const double px = (double)p.x, py = (double)p.y, pz = (double)p.z;
-    int cx, cy, cz;
-    lb_cell(G, p, &cx, &cy, &cz);
-    const uint64_t base = (uint64_t)s * G.ncells;
-    for (int z = max(cz - 1, 0); z <= min(cz + 1, G.nz - 1); ++z)
-        for (int y = max(cy - 1, 0); y <= min(cy + 1, G.ny - 1); ++y) {
-            const uint64_t row = base + ((uint64_t)z * G.ny + y) * G.nx;
-            const uint64_t k0 = row + max(cx - 1, 0), k1 = row + min(cx + 1, G.nx - 1);
-            uint32_t lo = 0, hi = m;
-            while (lo < hi) {
-                const uint32_t mid = (lo + hi) >> 1;
-                if (skey[mid] < k0) lo = mid + 1; else hi = mid;
-            }
-            for (uint32_t k = lo; k < m && skey[k] <= k1; ++k) {
-                const uint32_t j = sidx[k];
-                if (db_dist2(px, py, pz, &object[j].x) <= eps2) f(j);
-            }
-        }
-}
-
-// the four neighbour-search kernels are declared with a minimum of 8 blocks per SM (<= 64 registers): without it ptxas picks 32
-// registers for the hook and label kernels and spills
-struct LbDb {
-    const float4* object;
-    const uint32_t* object_sample;
-    const uint32_t* totals;  // [2] = object rows of the batch
-    const uint64_t* skey;
-    const uint32_t* sidx;
-    LbGrid G;
-    double eps2;
-};
-
-__global__ void __launch_bounds__(128, 8) lb_core_kernel(const LbDb a, uint32_t min_samples, uint8_t* __restrict__ core, uint32_t* __restrict__ parent) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t m = a.totals[2];
-    if (i >= m) return;
-    uint32_t cnt = 0;
-    lb_for_each_neighbour(a.object, a.G, a.eps2, a.object_sample[i], a.skey, a.sidx, m, i, [&](uint32_t) { ++cnt; });
-    core[i] = cnt >= min_samples ? 1 : 0;
-    parent[i] = i;
-}
-
-// the one hooking sweep: every thread completes the union of each of its edges before it moves on (DESIGN.md section 4.5)
-__global__ void __launch_bounds__(128, 8) lb_hook_kernel(const LbDb a, const uint8_t* __restrict__ core, uint32_t* __restrict__ parent) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t m = a.totals[2];
-    if (i >= m || !core[i]) return;
-    lb_for_each_neighbour(a.object, a.G, a.eps2, a.object_sample[i], a.skey, a.sidx, m, i, [=](uint32_t j) {
-        if (j < i && core[j]) db_union(parent, i, j, [] {});
-    });
-}
-
-// the verify sweep over the same edges: two endpoints with different roots set kLbUnmerged, never a silently under-merged labelling
-__global__ void __launch_bounds__(128, 8) lb_verify_kernel(const LbDb a, const uint8_t* __restrict__ core, const uint32_t* __restrict__ parent,
-                                                       uint32_t* __restrict__ status) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t m = a.totals[2];
-    if (i >= m || !core[i]) return;
-    const uint32_t ri = db_find(parent, i);
-    bool bad = false;
-    lb_for_each_neighbour(a.object, a.G, a.eps2, a.object_sample[i], a.skey, a.sidx, m, i, [=, &bad](uint32_t j) {
-        if (j < i && core[j] && db_find(parent, j) != ri) bad = true;
-    });
-    if (bad) atomicOr(status, kLbUnmerged);
-}
-
-// parent -> root for core rows; is_root has cap + 1 entries (zero past the object rows) so its exclusive scan also gives the totals
-__global__ void __launch_bounds__(256) lb_flatten_kernel(uint32_t cap, const uint32_t* __restrict__ totals, const uint8_t* __restrict__ core,
-                                                        uint32_t* __restrict__ parent, uint32_t* __restrict__ is_root) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i > cap) return;
-    uint32_t root = 0;
-    if (i < totals[2] && core[i]) {
-        const uint32_t r = db_find(parent, i);
-        parent[i] = r;  // roots keep pointing at themselves, so concurrent finds stay valid
-        root = r == i;
-    }
-    is_root[i] = root;
-}
-
-struct LbTable {
-    const uint32_t* object_off;
-    const uint32_t* rank;     // exclusive scan of is_root
-    uint32_t* slots;          // [cap, 11]: ordered min3, max3, -, -, -, -, count; finished in place
-    uint32_t* first;          // [cap]: smallest row of the slot's cluster (the caller's cluster_first)
-    int32_t* labels;
-    int32_t* noise_first;
-};
-
-// labels numbered per sample (the smallest core index of a component is its root; roots in row order give scikit-learn's numbering);
-// a border row takes the smallest adjacent cluster number.  The root of cluster k initialises the k-th slot of its sample.
-__global__ void __launch_bounds__(128, 8) lb_label_kernel(const LbDb a, const uint8_t* __restrict__ core, const uint32_t* __restrict__ parent,
-                                                      const LbTable t) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t m = a.totals[2];
-    if (i >= m) return;
-    const uint32_t s = a.object_sample[i], off = t.object_off[s], base = t.rank[off];
-    if (core[i]) {
-        const uint32_t r = parent[i], k = t.rank[r] - base;
-        t.labels[i] = (int32_t)k;
-        if (r == i) {
-            uint32_t* o = t.slots + (size_t)(off + k) * 11;
-#pragma unroll
-            for (int w = 0; w < 11; ++w) o[w] = (w < 3) ? 0xffffffffu : 0u;
-            t.first[off + k] = 0xffffffffu;
-        }
-        return;
-    }
-    uint32_t best = 0xffffffffu;
-    lb_for_each_neighbour(a.object, a.G, a.eps2, s, a.skey, a.sidx, m, i, [=, &best](uint32_t j) {
-        if (core[j]) best = min(best, t.rank[parent[j]]);
-    });
-    if (best == 0xffffffffu) {
-        t.labels[i] = -1;
-        atomicMin(&t.noise_first[s], (int32_t)(i - off));
-    } else {
-        t.labels[i] = (int32_t)(best - base);
-    }
-}
-
 // ---------------------------------------------------------------- 3. per-sample cluster table
 __global__ void __launch_bounds__(256) lb_minmax_kernel(const float4* __restrict__ object, const uint32_t* __restrict__ object_sample,
-                                                       const uint32_t* __restrict__ totals, const LbTable t) {
+                                                       const uint32_t* __restrict__ totals, const ClusterTable t) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= totals[2]) return;
     const int c = t.labels[i];
@@ -338,7 +176,7 @@ __global__ void __launch_bounds__(256) lb_minmax_kernel(const float4* __restrict
 // rows: finish the slot of every root; samples: cluster count and the noise marker
 __global__ void __launch_bounds__(256) lb_finish_kernel(uint32_t n_threads, int n_samples, const uint32_t* __restrict__ object_sample,
                                                        const uint32_t* __restrict__ totals, const uint32_t* __restrict__ is_root,
-                                                       const uint32_t* __restrict__ counts, const LbTable t, int32_t* __restrict__ n_clusters) {
+                                                       const uint32_t* __restrict__ counts, const ClusterTable t, int32_t* __restrict__ n_clusters) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_threads) return;
     if (i < totals[2] && is_root[i]) {
@@ -355,8 +193,8 @@ __global__ void __launch_bounds__(256) lb_finish_kernel(uint32_t n_threads, int 
 // ---------------------------------------------------------------- host side
 // cubic cells a hair above eps (as ops.dbscan) over the box every object row lies in: |x|, |y| < range_max (the gate's
 // sqrt(x^2 + y^2) < range_max), max(ground_z, z_min) <= z < z_max; coarser cells while one sample's grid would not fit 32 bits
-static LbGrid lb_grid(const msc_params& P, double eps) {
-    LbGrid G;
+static DbGrid lb_grid(const msc_params& P, double eps) {
+    DbGrid G;
     double cell = eps * (1.0 + 1e-6);
     const double r = (double)P.range_max, zlo = (double)fmaxf(P.ground_z, P.z_min), zhi = (double)P.z_max;
     G.ox = -r; G.oy = -r; G.oz = zlo;
@@ -374,25 +212,17 @@ static LbGrid lb_grid(const msc_params& P, double eps) {
     return G;
 }
 
-static int lb_bits(uint64_t v) {  // bits needed to hold v
-    int b = 0;
-    while (b < 64 && (v >> b) != 0) ++b;
-    return b;
-}
-
 struct LbWs {
-    size_t kf_n, tile_off, block_counts, totals, object_sample, keys_in, keys_out, vals_in, sidx, core, parent, is_root, rank, temp,
-        temp_bytes, total;
+    size_t kf_n, tile_off, block_counts, totals, object_sample;
     uint32_t n_tiles;
-    int end_bit;
-    LbGrid G;
+    DbGrid G;
+    DbWs db;  // DBSCAN's buffers follow; db.end is the total
 };
 
 static cudaError_t lb_layout(const msc_params& P, double eps, int n_samples, uint32_t cap, LbWs* W) {
     auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
     W->G = lb_grid(P, eps);
     W->n_tiles = (uint32_t)((cap + (uint64_t)kCompactThreads - 1) / kCompactThreads + (uint64_t)n_samples);
-    W->end_bit = lb_bits((uint64_t)n_samples * W->G.ncells);  // the largest key, S * ncells, pads the sort
     const size_t S = (size_t)n_samples, n = cap;
     size_t o = 0;
     W->kf_n = o; o = al(o + S * 4);
@@ -400,25 +230,7 @@ static cudaError_t lb_layout(const msc_params& P, double eps, int n_samples, uin
     W->block_counts = o; o = al(o + (size_t)W->n_tiles * 8);
     W->totals = o; o = al(o + 16);
     W->object_sample = o; o = al(o + n * 4);
-    W->keys_in = o; o = al(o + n * 8);
-    W->keys_out = o; o = al(o + n * 8);
-    W->vals_in = o; o = al(o + n * 4);
-    W->sidx = o; o = al(o + n * 4);
-    W->core = o; o = al(o + n);
-    W->parent = o; o = al(o + n * 4);
-    W->is_root = o; o = al(o + (n + 1) * 4);
-    W->rank = o; o = al(o + (n + 1) * 4);
-    size_t sort_bytes = 0, scan_bytes = 0;
-    cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const uint32_t*)nullptr,
-                                                    (uint32_t*)nullptr, (int)n, 0, W->end_bit);
-    if (e != cudaSuccess) return e;
-    e = cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n + 1);
-    if (e != cudaSuccess) return e;
-    W->temp = o;
-    W->temp_bytes = al(sort_bytes > scan_bytes ? sort_bytes : scan_bytes);
-    o = al(o + W->temp_bytes);
-    W->total = o;
-    return cudaSuccess;
+    return db_layout(o, cap, n_samples, W->G, &W->db);
 }
 
 static bool lb_args_ok(const msc_params* params, double eps, int32_t n_samples, uint32_t cap) {
@@ -434,7 +246,7 @@ size_t msc_lidar_batch_workspace_bytes(const msc_params* params, double eps, int
     if (!lb_args_ok(params, eps, n_samples, row_capacity)) return 0;
     LbWs W;
     if (lb_layout(*params, eps, n_samples, row_capacity, &W) != cudaSuccess) return 0;
-    return W.total;
+    return W.db.end;
 }
 
 int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, const msc_batch_in* in, const msc_lidar_batch_out* out,
@@ -455,17 +267,13 @@ int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, c
     MSC_REQUIRE(workspace, "msc_lidar_batch: null workspace");
     LbWs W;
     MSC_CUDA(lb_layout(*params, eps, S, cap, &W));
-    MSC_REQUIRE(workspace_bytes >= W.total, "msc_lidar_batch: workspace too small: need %zu bytes, got %zu", W.total, workspace_bytes);
+    MSC_REQUIRE(workspace_bytes >= W.db.end, "msc_lidar_batch: workspace too small: need %zu bytes, got %zu", W.db.end, workspace_bytes);
     cudaStream_t stream = (cudaStream_t)stream_v;
     unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
     uint32_t* kf_n = (uint32_t*)(ws + W.kf_n); uint32_t* tile_off = (uint32_t*)(ws + W.tile_off);
     uint32_t* block_counts = (uint32_t*)(ws + W.block_counts); uint32_t* totals = (uint32_t*)(ws + W.totals);
     uint32_t* object_sample = (uint32_t*)(ws + W.object_sample);
-    uint64_t* keys_in = (uint64_t*)(ws + W.keys_in); uint64_t* keys_out = (uint64_t*)(ws + W.keys_out);
-    uint32_t* vals_in = (uint32_t*)(ws + W.vals_in); uint32_t* sidx = (uint32_t*)(ws + W.sidx);
-    uint8_t* core = (uint8_t*)(ws + W.core); uint32_t* parent = (uint32_t*)(ws + W.parent);
-    uint32_t* is_root = (uint32_t*)(ws + W.is_root); uint32_t* rank = (uint32_t*)(ws + W.rank);
-    void* temp = ws + W.temp;
+    const uint32_t* is_root = (const uint32_t*)(ws + W.db.is_root); const uint32_t* rank = (const uint32_t*)(ws + W.db.rank);
     const float4* object = reinterpret_cast<const float4*>(out->object);
 
     // 1. filter / split
@@ -481,21 +289,11 @@ int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, c
     MSC_CUDA(cudaGetLastError());
 
     // 2. DBSCAN over every sample's object rows
-    const unsigned nb256 = (cap + 255) / 256 + 1, nb128 = (cap + 127) / 128 + 1;
-    lb_key_kernel<<<nb256, 256, 0, stream>>>(object, object_sample, totals, cap, W.G, (uint64_t)S * W.G.ncells, keys_in, vals_in);
-    size_t temp_bytes = W.temp_bytes;
-    MSC_CUDA(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys_in, keys_out, vals_in, sidx, (int)cap, 0, W.end_bit, stream));
-    const LbDb a{object, object_sample, totals, keys_out, sidx, W.G, eps * eps};
-    lb_core_kernel<<<nb128, 128, 0, stream>>>(a, (uint32_t)min_samples, core, parent);
-    lb_hook_kernel<<<nb128, 128, 0, stream>>>(a, core, parent);
-    lb_verify_kernel<<<nb128, 128, 0, stream>>>(a, core, parent, out->status);
-    lb_flatten_kernel<<<nb256, 256, 0, stream>>>(cap, totals, core, parent, is_root);
-    temp_bytes = W.temp_bytes;
-    MSC_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, is_root, rank, (int)cap + 1, stream));
-    const LbTable t{out->object_off, rank, reinterpret_cast<uint32_t*>(out->clusters), reinterpret_cast<uint32_t*>(out->cluster_first), out->labels, out->noise_first};
-    lb_label_kernel<<<nb128, 128, 0, stream>>>(a, core, parent, t);
+    const ClusterTable t{out->object_off, rank, reinterpret_cast<uint32_t*>(out->clusters), reinterpret_cast<uint32_t*>(out->cluster_first), out->labels, out->noise_first};
+    MSC_CUDA(db_enqueue(W.db, ws, W.G, object, object_sample, totals, eps, (uint32_t)min_samples, t, out->status, stream));
 
     // 3. cluster table
+    const unsigned nb256 = (cap + 255) / 256 + 1;
     lb_minmax_kernel<<<nb256, 256, 0, stream>>>(object, object_sample, totals, t);
     const uint32_t n_fin = cap > (uint32_t)S ? cap : (uint32_t)S;
     lb_finish_kernel<<<(n_fin + 255) / 256, 256, 0, stream>>>(n_fin, S, object_sample, totals, is_root, out->counts, t, out->n_clusters);

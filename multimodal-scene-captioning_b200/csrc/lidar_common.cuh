@@ -1,6 +1,5 @@
-// lidar_common.cuh -- device helpers of the keyframe path that both the single-keyframe kernels (keyframe.cu, dbscan.cu) and
-// the batched ones (keyframe_batch.cu) use: one copy of the gate / split rule, of the neighbour relation, of the union-find
-// and of the cluster-box arithmetic, so the two paths cannot drift apart.
+// lidar_common.cuh -- what the single-keyframe path (keyframe.cu, dbscan.cu) and the batched one (keyframe_batch.cu) share: one
+// copy of the gate / split rule, of the cluster-box arithmetic and of the DBSCAN pipeline, so the two paths cannot drift apart.
 #pragma once
 #include "msc_common.cuh"
 
@@ -30,36 +29,44 @@ __device__ __forceinline__ uint32_t keyframe_class(const float* __restrict__ p, 
 // exclusive scan of per-block (ground, object) counts, single block; defined in keyframe.cu
 __global__ void __launch_bounds__(1024) kf_scan_kernel(uint32_t* __restrict__ block_counts, uint32_t n_blocks, uint32_t* __restrict__ counts);
 
-// DBSCAN neighbour relation: squared distance in float64, accumulated x -> y -> z (scikit-learn's KD-tree reduced distance)
-__device__ __forceinline__ double db_dist2(double px, double py, double pz, const float* __restrict__ q) {
-    const double dx = px - (double)q[0], dy = py - (double)q[1], dz = pz - (double)q[2];
-    double d = dx * dx;
-    d = d + dy * dy;
-    d = d + dz * dz;
-    return d;
-}
+// ---------------------------------------------------------------- DBSCAN over the rows of many samples (dbscan.cu)
+constexpr uint32_t kDbUnmerged = 1u, kLbOverflow = 2u;  // bits of msc_lidar_batch's status word (include/msc_geom.h)
 
-__device__ __forceinline__ uint32_t db_find(const uint32_t* parent, uint32_t a) {
-    uint32_t p = ((const volatile uint32_t*)parent)[a];
-    while (p != a) { a = p; p = ((const volatile uint32_t*)parent)[a]; }
-    return a;
-}
+// cubic cells of side 1 / inv_cell from (ox, oy, oz); a row's key is sample * ncells + its cell
+struct DbGrid {
+    double ox, oy, oz, inv_cell;
+    int nx, ny, nz;
+    uint64_t ncells;
+};
 
-// union of the trees of i and j: the larger root is hung under the smaller one (atomicMin), so a component's root converges to its
-// smallest index.  When the atomicMin finds hi already relinked (by another thread) to old < hi, hi's subtree moves under lo and this
-// thread goes on to merge old's tree with lo's, so the edge it cut is restored before it returns.  on_hook() runs on every atomic.
-template <class F>
-__device__ __forceinline__ void db_union(uint32_t* parent, uint32_t i, uint32_t j, F on_hook) {
-    uint32_t a = db_find(parent, i), b = db_find(parent, j);
-    while (a != b) {
-        const uint32_t hi = max(a, b), lo = min(a, b);
-        const uint32_t old = atomicMin(&parent[hi], lo);
-        on_hook();
-        if (old == hi) break;   // hi was a root and now hangs under lo
-        a = db_find(parent, old);  // hi already had a smaller parent: merge that tree with lo
-        b = db_find(parent, lo);
-    }
-}
+// the per-sample cluster table: the label kernel initialises the slot of every cluster, msc_lidar_batch fills and finishes them
+struct ClusterTable {
+    const uint32_t* object_off;
+    const uint32_t* rank;     // exclusive scan of is_root
+    uint32_t* slots;          // [cap, 11]: ordered min3, max3, -, -, -, -, count; finished in place
+    uint32_t* first;          // [cap]: smallest row of the slot's cluster (the caller's cluster_first)
+    int32_t* labels;
+    int32_t* noise_first;
+};
+
+// byte offsets of DBSCAN's buffers in a caller's workspace, for `cap` rows whose keys lie below pad_key
+struct DbWs {
+    size_t keys_in, keys_out, vals_in, sidx, core, parent, is_root, rank, temp, temp_bytes, end;
+    uint32_t cap;
+    uint64_t pad_key;  // n_samples * ncells: the key of the rows past the last object row
+    int end_bit;
+};
+// lays the buffers out from byte `base` (256-aligned) on; W->end is the first byte past them
+cudaError_t db_layout(size_t base, uint32_t cap, int n_samples, const DbGrid& G, DbWs* W);
+
+// Enqueues on `stream`: key -> radix sort -> core -> hook -> verify -> flatten -> exclusive scan of is_root into W.rank -> label, over
+// rows [0, totals[2]) of `object`; row i belongs to sample object_sample[i], and rows of different samples are never neighbours.
+// Writes t.labels (numbered per sample from 0), t.noise_first and the initial slot of every cluster of t; sets kDbUnmerged in
+// *status if the merge left an edge unmerged.  is_root and rank (cap + 1 entries each; rank[cap] is the number of clusters) stay
+// in the workspace.  t.rank must point at W.rank.
+cudaError_t db_enqueue(const DbWs& W, unsigned char* ws, const DbGrid& G, const float4* object, const uint32_t* object_sample,
+                       const uint32_t* totals, double eps, uint32_t min_samples, const ClusterTable& t, uint32_t* status,
+                       cudaStream_t stream);
 
 // per-cluster box (lidar_agent.py:200-204) from 11 words: ordered-int min3, max3, -, -, -, -, count -> f32 min3, max3, center3,
 // distance, num_points, in place

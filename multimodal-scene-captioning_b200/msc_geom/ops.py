@@ -286,7 +286,7 @@ def dbscan(eng: GeometryEngine, xyz: np.ndarray, eps: float = 0.5, min_samples: 
     k = C.c_int32(0)
     _capi.check(eng.lib.msc_dbscan(src.data_ptr(), n, pitch, C.c_double(float(eps)), int(min_samples), c_org, C.c_double(cell), c_dims,
                                    labels.data_ptr(), C.byref(k), ws.data_ptr(), need, _stream(eng)), "msc_dbscan")
-    eng.kernel_launches += 8
+    eng.kernel_launches += 9  # 7 own kernels + the CUB sort and scan
     return labels.cpu().numpy().astype(np.int64)
 
 

@@ -6,7 +6,7 @@ keyframe, sweep 0 with 34,720 rows, is read), against the per-sample loop of the
 
 The batched call is timed with CUDA events on the current stream, median over --calls after --warmup; it stays on the device (to_host is
 not in the timed window).  The per-sample loop is ops.keyframe_filter_split + ops.dbscan + ops.cluster_aabb on host arrays (host in,
-host out, one host synchronisation per DBSCAN sweep), timed with a host clock over all samples once after one warm-up sample, and its
+host out, one host synchronisation per DBSCAN call), timed with a host clock over all samples once after one warm-up sample, and its
 outputs are compared with the batch's sample by sample.  The card's name and power limit are read in the same run."""
 import argparse
 import json
