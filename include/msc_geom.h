@@ -361,6 +361,47 @@ size_t msc_lidar_batch_workspace_bytes(const msc_params* params, double eps, int
 int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, const msc_batch_in* in, const msc_lidar_batch_out* out,
                     void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * The finished BEV of LiDARAgent._generate_multi_layer_bev (lidar_agent.py:539-634) for samples [first, first + n) of an
+ * msc_lidar_batch result of n_samples samples, in one stream-ordered call.  From `rows` only ground, object, ground_off, object_off and
+ * counts are read; from msc_params only bev_res (res) and bev_range.  Image i (sample first + i), byte-identical to the host path
+ * finish_bev_layers(msc_keyframe_bev(...)) on that sample's rows:
+ *   semantic u8 [n, res, res, 3] BGR: the raster colours, flipped vertically, with the overlays written over them;
+ *   height   f32 [n, res, res]: the largest z > 0 per cell (0 elsewhere), flipped;
+ *   density  u8 [n, res, res]: (u8)(lut[c] / lut[cmax] * 255) in float32 (round to nearest per step, truncated), c the cell's rows and
+ *            cmax the sample's largest c, flipped; all 0 when cmax = 0.
+ * lut f32 [lut_len]: the density table, entry c = NumPy's float32 log1p(c).  A sample whose cmax >= lut_len sets bit 0 of *status
+ * (device u32, OR-ed into: the caller clears it) and gets density 0; the results must then not be used.
+ * stamp u32 [stamp_len, 2]: the overlays as (pixel index y * res + x, B | G << 8 | R << 16), written last; pixels >= res * res are
+ * skipped.  Nothing outside the n images is written.  No host synchronisation, no allocation: workspace >=
+ * msc_keyframe_bev_batch_workspace_bytes(res, n) (8 res^2 bytes per sample and 16 more), 256-byte aligned.  res outside
+ * [1, 8192], a window outside [0, n_samples), n > 65535, lut_len < 1, NULL buffers or a short workspace: MSC_ERR_BAD_ARGUMENT.
+ * n = 0 is a successful no-op.
+ */
+size_t msc_keyframe_bev_batch_workspace_bytes(int32_t bev_res, int32_t n);
+int msc_keyframe_bev_batch(const msc_params* params, const msc_lidar_batch_out* rows, int32_t n_samples, int32_t first, int32_t n,
+                           const float* lut, int32_t lut_len, const uint32_t* stamp, int32_t stamp_len, uint8_t* semantic, float* height,
+                           uint8_t* density, uint32_t* status, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * The finished 4-view images of LiDARAgent._generate_cluster_visualization (lidar_agent.py:241-356) for n_views clusters in one
+ * stream-ordered call.  rows: f32 [*, 4] (x, y, z, intensity) and labels i32 [*] on the device; views: HOST i32 [n_views, 3] =
+ * (row_begin, row_end, label), copied into the workspace.  The points of view v are the rows r in [row_begin, row_end) with
+ * labels[r] == label, in row order (for msc_lidar_batch's output: (object_off[s], object_off[s] + object count, k) is cluster k of
+ * sample s).  Image v, out_bgr u8 [n_views, 512, 512, 3], is byte-identical to the host path: msc_cluster_views with the cluster mean
+ * (NumPy's float32 mean: a sequential sum in row order over n) and scale (fl32(89.6 / max_range), 1 when max_range is 0), then the
+ * axes and titles given as stamp u32 [stamp_len, 2] (pixel y * 512 + x, B | G << 8 | R << 16), written last.  A view of more than
+ * max_view_points points sets bit 0 of *status (device u32, OR-ed into: the caller clears it); its image must not be used.
+ * No host synchronisation, no allocation: workspace >= msc_cluster_views_batch_workspace_bytes(n_views, max_view_points) (1 MiB of
+ * keys and 4 max_view_points bytes per view, plus a few words), 256-byte aligned.  n_views outside [0, 65535], max_view_points outside
+ * [0, 2^24), an empty or inverted row range, NULL buffers or a short workspace: MSC_ERR_BAD_ARGUMENT.  n_views = 0 is a successful
+ * no-op.
+ */
+size_t msc_cluster_views_batch_workspace_bytes(int32_t n_views, int32_t max_view_points);
+int msc_cluster_views_batch(const float* rows, const int32_t* labels, const int32_t* views, int32_t n_views, int32_t max_view_points,
+                            const uint32_t* stamp, int32_t stamp_len, uint8_t* out_bgr, uint32_t* status, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

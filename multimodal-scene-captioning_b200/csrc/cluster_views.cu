@@ -7,11 +7,9 @@
 // key grid over the 13-pixel footprint of cv2's filled radius-2 circle (|dx|+|dy| <= 2, clipped to the 512x512 grid),
 // then one pass that turns each pixel's winner into its grey value.  Axes, titles (cv2.line / cv2.putText) and the
 // batch mosaic stay on the host: they are drawn after the points and never overlap another view's discs.
-#include "msc_common.cuh"
+#include "lidar_common.cuh"
 
 namespace msc {
-
-constexpr int kView = 256, kGrid = 512;  // img_size and the 2x2 grid (lidar_agent.py:242, :267)
 
 __device__ __forceinline__ uint32_t f2ord_cv(float f) {
     uint32_t b = __float_as_uint(f);

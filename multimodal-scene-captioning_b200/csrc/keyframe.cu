@@ -129,8 +129,8 @@ __global__ void __launch_bounds__(256) kf_bev_raster_kernel(const __grid_constan
     if (i < n) {
         const bool is_obj = i >= n_ground;
         const float4 p = is_obj ? object[i - n_ground] : ground[i];
-        const int ix = bev_cell<false>(p.x, P.bev_range, two_r, 0.0f, resf, res - 1);
-        const int iy = bev_cell<false>(p.y, P.bev_range, two_r, 0.0f, resf, res - 1);
+        int ix, iy;
+        bev_xy(p, P.bev_range, two_r, resf, res, &ix, &iy);
         const size_t cell = (size_t)iy * res + ix;  // [y, x] indexing, :559
         atomicAdd(&count[cell], 1u);                                                   // :559
         if (p.z > 0.0f) atomicMax(reinterpret_cast<int*>(height) + cell, __float_as_int(p.z));  // :560, 0-initialised
@@ -149,20 +149,8 @@ __global__ void __launch_bounds__(256) kf_bev_colour_kernel(const float4* __rest
                                                            uint8_t* __restrict__ semantic_bgr) {
     const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncell) return;
-    const uint32_t w = winner[c];
-    uint8_t b = 0, g = 0, r = 0;
-    if (w == 1u) { b = 80; g = 80; r = 120; }  // :572
-    else if (w >= 2u) {
-        const float hmin = ord2f(zrange[0]), hmax = ord2f(zrange[1]);
-        int gv;
-        if (!(hmax > hmin)) gv = 255;  // :581-582 norm = 0.5 -> int(255 * (1 - (0.5 - 0.5) * 2))
-        else {
-            const float hn = __fdiv_rn(__fsub_rn(object[w - 2u].z, hmin), __fsub_rn(hmax, hmin));  // :580
-            if (hn < 0.5f) gv = __float2int_rz(__fmul_rn(255.0f, __fsub_rn(1.0f, __fmul_rn(hn, 2.0f))));  // :589
-            else gv = __float2int_rz(__fmul_rn(255.0f, __fsub_rn(1.0f, __fmul_rn(__fsub_rn(hn, 0.5f), 2.0f))));  // :594
-        }
-        b = 0; g = (uint8_t)gv; r = 255;  // :597 BGR
-    }
+    uint8_t b, g, r;
+    bev_colour(winner[c], object, zrange, &b, &g, &r);
     semantic_bgr[(size_t)c * 3 + 0] = b; semantic_bgr[(size_t)c * 3 + 1] = g; semantic_bgr[(size_t)c * 3 + 2] = r;
 }
 

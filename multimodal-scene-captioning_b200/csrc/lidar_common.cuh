@@ -29,6 +29,40 @@ __device__ __forceinline__ uint32_t keyframe_class(const float* __restrict__ p, 
 // exclusive scan of per-block (ground, object) counts, single block; defined in keyframe.cu
 __global__ void __launch_bounds__(1024) kf_scan_kernel(uint32_t* __restrict__ block_counts, uint32_t n_blocks, uint32_t* __restrict__ counts);
 
+// ---------------------------------------------------------------- keyframe BEV (lidar_agent.py:539-597): keyframe.cu and lidar_images.cu
+// cell of a row: x and y cells of :547-552, [y, x] indexing (:559)
+__device__ __forceinline__ void bev_xy(const float4& p, float bev_range, float two_r, float resf, int res, int* ix, int* iy) {
+    *ix = bev_cell<false>(p.x, bev_range, two_r, 0.0f, resf, res - 1);
+    *iy = bev_cell<false>(p.y, bev_range, two_r, 0.0f, resf, res - 1);
+}
+// semantic BGR of a cell from its winner key (0 empty, 1 ground, 2 + i object row i of `object`) and the ordered-int min / max
+// of the object heights in zrange[0..1]
+__device__ __forceinline__ void bev_colour(uint32_t w, const float4* __restrict__ object, const uint32_t* __restrict__ zrange, uint8_t* b,
+                                           uint8_t* g, uint8_t* r) {
+    *b = 0; *g = 0; *r = 0;
+    if (w == 1u) { *b = 80; *g = 80; *r = 120; }  // :572
+    else if (w >= 2u) {
+        const float hmin = ord2f(zrange[0]), hmax = ord2f(zrange[1]);
+        int gv;
+        if (!(hmax > hmin)) gv = 255;  // :581-582 norm = 0.5 -> int(255 * (1 - (0.5 - 0.5) * 2))
+        else {
+            const float hn = __fdiv_rn(__fsub_rn(object[w - 2u].z, hmin), __fsub_rn(hmax, hmin));  // :580
+            if (hn < 0.5f) gv = __float2int_rz(__fmul_rn(255.0f, __fsub_rn(1.0f, __fmul_rn(hn, 2.0f))));  // :589
+            else gv = __float2int_rz(__fmul_rn(255.0f, __fsub_rn(1.0f, __fmul_rn(__fsub_rn(hn, 0.5f), 2.0f))));  // :594
+        }
+        *b = 0; *g = (uint8_t)gv; *r = 255;  // :597 BGR
+    }
+}
+
+// ---------------------------------------------------------------- cluster 4-view raster (cluster_views.cu), also run by lidar_images.cu
+constexpr int kView = 256, kGrid = 512;  // img_size and the 2x2 grid (lidar_agent.py:242, :267)
+__global__ void __launch_bounds__(256) cluster_splat_kernel(const float4* __restrict__ pts, const uint32_t* __restrict__ order,
+                                                           const int32_t* __restrict__ cluster_off, int n_clusters, const float* __restrict__ center_scale,
+                                                           uint32_t* __restrict__ keys, uint32_t* __restrict__ irange);
+__global__ void __launch_bounds__(256) cluster_colour_kernel(const float4* __restrict__ pts, const uint32_t* __restrict__ order,
+                                                            const int32_t* __restrict__ cluster_off, const uint32_t* __restrict__ keys,
+                                                            const uint32_t* __restrict__ irange, uint8_t* __restrict__ out);
+
 // ---------------------------------------------------------------- DBSCAN over the rows of many samples (dbscan.cu)
 constexpr uint32_t kDbUnmerged = 1u, kLbOverflow = 2u;  // bits of msc_lidar_batch's status word (include/msc_geom.h)
 

@@ -120,6 +120,12 @@ _PROTOS = {
     "msc_jpeg_encode_batch": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_size_t, C.c_void_p]),
     "msc_cluster_views": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "msc_keyframe_bev_batch_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "msc_keyframe_bev_batch": (C.c_int, [C.POINTER(MscParams), C.POINTER(MscLidarBatchOut), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
+                                         C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "msc_cluster_views_batch_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "msc_cluster_views_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_size_t, C.c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_PROTOS)

@@ -161,6 +161,7 @@ class LidarBatchResult:
     labels: torch.Tensor         # i32 [cap] per object row, numbered per sample, -1 noise
     clusters: torch.Tensor       # f32 [cap, 11]; cluster k of sample s at object_off[s] + k
     cluster_first: torch.Tensor  # i32 [cap] smallest object row (within the sample) of that cluster
+    sample_rows: Optional[int] = None  # most keyframe rows of one sample (sizes run_lidar_bev's density table); None: row_capacity
 
     def _view(self, k: int, n: int) -> torch.Tensor:
         return self.small[1 + k * self.n_samples: 1 + (k + n) * self.n_samples]
@@ -211,6 +212,44 @@ class LidarBatchResult:
         return out
 
 
+@dataclass
+class LidarBevResult:
+    """Finished BEVs of msc_keyframe_bev_batch for samples first .. first + n_samples - 1 of a LidarBatchResult, still on the device."""
+    first: int
+    n_samples: int
+    res: int
+    semantic: torch.Tensor  # u8 [n, res, res, 3] BGR, flipped, overlays drawn
+    height: torch.Tensor    # f32 [n, res, res], flipped
+    density: torch.Tensor   # u8 [n, res, res], flipped
+    status: torch.Tensor    # i32 [1]
+
+    def to_host(self, layers: Sequence[str] = ("semantic", "height", "density")) -> List[Dict[str, np.ndarray]]:
+        """Per sample, the layers asked for (finish_bev_layers' dict); only those are copied.  This is the synchronisation point; a set
+        status word (a cell count beyond the density table) raises MscError."""
+        if int(self.status.cpu()[0]):
+            raise _capi.MscError("msc_keyframe_bev_batch: a cell count has no entry in the density table", 1)
+        host = {k: getattr(self, k).cpu().numpy() for k in layers}
+        return [{k: host[k][i] for k in layers} for i in range(self.n_samples)]
+
+
+@dataclass
+class ClusterViewsResult:
+    """Finished cluster images of msc_cluster_views_batch, still on the device."""
+    n_views: int
+    images: torch.Tensor  # u8 [n, 512, 512, 3]
+    status: torch.Tensor  # i32 [1]
+
+    def to_host(self) -> np.ndarray:
+        """u8 [n, 512, 512, 3].  This is the synchronisation point; a view above the maximum view size raises MscError."""
+        if int(self.status.cpu()[0]):
+            raise _capi.MscError("msc_cluster_views_batch: a view holds more points than max_view_points", 1)
+        return self.images.cpu().numpy()
+
+
+BEV_WORKSPACE_PER_CALL = 2 << 30            # workspace bytes of one msc_keyframe_bev_batch call (8 res^2 bytes per sample)
+CLUSTER_VIEWS_WORKSPACE_PER_CALL = 2 << 30  # workspace bytes of one msc_cluster_views_batch call (1 MiB + 4 max_view_points per view)
+
+
 JPEG_HEADER_BYTES = 625  # SOI .. SOS (623 bytes) and EOI of every file msc_jpeg_encode_batch writes
 
 
@@ -242,11 +281,16 @@ class JpegBatchResult:
         return [data[off[i]:off[i + 1]] for i in range(self.n_images)]
 
 
-def keyframe_rows(hb: HostBatch) -> int:
-    """Total keyframe rows of a batch (sweep sample_sweep_off[s] of every sample that has sweeps): the row capacity of run_lidar."""
+def _keyframe_row_counts(hb: HostBatch) -> np.ndarray:
+    """Keyframe rows (sweep sample_sweep_off[s]) of every sample that has sweeps."""
     sso = hb.sample_sweep_off
     first = sso[:-1][sso[1:] > sso[:-1]]
-    return int(hb.sweep_count[first].astype(np.int64).sum())
+    return hb.sweep_count[first].astype(np.int64)
+
+
+def keyframe_rows(hb: HostBatch) -> int:
+    """Total keyframe rows of a batch: the row capacity of run_lidar."""
+    return int(_keyframe_row_counts(hb).sum())
 
 
 class InputArena:
@@ -308,6 +352,8 @@ class GeometryEngine:
         self._workspaces: Dict[int, torch.Tensor] = {}  # one work counter per stream (kernels on different streams overlap)
         self._ws_need: Dict[tuple, int] = {}
         self._params_cache: Dict[tuple, tuple] = {}
+        self._stamps: Dict[object, torch.Tensor] = {}  # overlay stamps of the LiDAR agent's images, per image geometry
+        self._bev_lut: Optional[torch.Tensor] = None    # the BEV density table
         self.kernel_launches = 0
 
     # ------------------------------------------------------------------ transfers
@@ -478,10 +524,12 @@ class GeometryEngine:
     # ------------------------------------------------------------------ the reference's keyframe evidence, batched
     def alloc_lidar(self, hb: HostBatch) -> LidarBatchResult:
         """Output buffers of run_lidar for `hb`: row arrays sized by the batch's total keyframe rows (known on the host)."""
-        S, cap, d = hb.n_samples, keyframe_rows(hb), self.device
+        rows = _keyframe_row_counts(hb)
+        S, cap, d = hb.n_samples, int(rows.sum()), self.device
         return LidarBatchResult(S, cap, torch.zeros(1 + 7 * S, dtype=torch.int32, device=d), torch.empty((cap, 4), dtype=torch.float32, device=d),
                                 torch.empty((cap, 4), dtype=torch.float32, device=d), torch.empty(cap, dtype=torch.int32, device=d),
-                                torch.empty((cap, 11), dtype=torch.float32, device=d), torch.empty(cap, dtype=torch.int32, device=d))
+                                torch.empty((cap, 11), dtype=torch.float32, device=d), torch.empty(cap, dtype=torch.int32, device=d),
+                                int(rows.max()) if rows.size else 0)
 
     def run_lidar(self, db: DeviceBatch, out: Optional[LidarBatchResult] = None, params: Optional[GeomParams] = None, eps: float = 0.5,
                   min_samples: int = 10) -> LidarBatchResult:
@@ -503,6 +551,108 @@ class GeometryEngine:
                                              need, C.c_void_p(stream)), "msc_lidar_batch")
         if hb.n_samples > 0:
             self.kernel_launches += 15  # 13 own kernels + the CUB sort and scan (each of those launches several kernels of its own)
+        return out
+
+    # ------------------------------------------------------------------ the LiDAR agent's images, batched
+    def _stamp(self, key, make) -> torch.Tensor:
+        """The device copy of an overlay stamp (lidar_agent.overlay_stamp), derived once per image geometry."""
+        t = self._stamps.get(key)
+        if t is None:
+            t = self._stamps[key] = torch.from_numpy(make().view(np.int32)).to(self.device)
+        return t
+
+    def _density_table(self, cmax: int) -> torch.Tensor:
+        """lidar_agent.density_table on the device, at least cmax + 1 entries (a longer table has the same prefix)."""
+        if self._bev_lut is None or self._bev_lut.numel() < cmax + 1:
+            from .lidar_agent import density_table
+            self._bev_lut = torch.from_numpy(density_table(cmax)).to(self.device)
+        return self._bev_lut
+
+    def alloc_bev(self, n: int, res: int) -> LidarBevResult:
+        """Output buffers of run_lidar_bev for n samples at res x res."""
+        d = self.device
+        return LidarBevResult(0, n, res, torch.empty((n, res, res, 3), dtype=torch.uint8, device=d), torch.empty((n, res, res), dtype=torch.float32, device=d),
+                              torch.empty((n, res, res), dtype=torch.uint8, device=d), torch.zeros(1, dtype=torch.int32, device=d))
+
+    def run_lidar_bev(self, lr: LidarBatchResult, bev_res: int, bev_range: float, first: int = 0, n: Optional[int] = None,
+                      out: Optional[LidarBevResult] = None) -> LidarBevResult:
+        """The finished BEV of LiDARAgent._generate_multi_layer_bev (semantic with its overlays, height, density) for samples
+        first .. first + n - 1 of a run_lidar result, stream-ordered after it (msc_keyframe_bev_batch, one call per
+        BEV_WORKSPACE_PER_CALL bytes of workspace).  Nothing is synchronised; out.to_host() reads the results."""
+        n = lr.n_samples - first if n is None else n
+        if first < 0 or n < 0 or first + n > lr.n_samples:
+            raise _capi.MscError("run_lidar_bev: samples [%d, %d) outside the batch of %d" % (first, first + n, lr.n_samples), _capi.MSC_ERR_BAD_ARGUMENT)
+        res = int(bev_res)
+        if out is None:
+            out = self.alloc_bev(n, res)
+        if out.n_samples != n or out.res != res:
+            raise _capi.MscError("run_lidar_bev: the output buffers do not match the window", _capi.MSC_ERR_BAD_ARGUMENT)
+        out.first = first
+        out.status.zero_()
+        if n == 0:
+            return out
+        from .lidar_agent import bev_stamp
+        lut = self._density_table(lr.sample_rows if lr.sample_rows is not None else lr.row_capacity)
+        stamp = self._stamp(("bev", res, float(bev_range)), lambda: bev_stamp(res, bev_range))
+        per = int(self.lib.msc_keyframe_bev_batch_workspace_bytes(res, 1))
+        if per == 0:
+            raise _capi.MscError("run_lidar_bev: bev_res %d out of range" % res, _capi.MSC_ERR_BAD_ARGUMENT)
+        step = max(1, min(n, 65535, BEV_WORKSPACE_PER_CALL // per))
+        need = int(self.lib.msc_keyframe_bev_batch_workspace_bytes(res, step))
+        ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        mp = make_params(GeomParams(bev_res=res, bev_range=float(bev_range)))
+        rows = lr.struct()
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        for a in range(0, n, step):
+            k = min(step, n - a)
+            _capi.check(self.lib.msc_keyframe_bev_batch(C.byref(mp), C.byref(rows), lr.n_samples, first + a, k, lut.data_ptr(), lut.numel(),
+                                                        stamp.data_ptr(), stamp.shape[0], out.semantic[a].data_ptr(), out.height[a].data_ptr(),
+                                                        out.density[a].data_ptr(), out.status.data_ptr(), ws.data_ptr(), need, stream),
+                        "msc_keyframe_bev_batch")
+            self.kernel_launches += 3
+        return out
+
+    def run_cluster_views(self, rows: torch.Tensor, labels: torch.Tensor, views, max_view_points: Optional[int] = None,
+                          out: Optional[ClusterViewsResult] = None) -> ClusterViewsResult:
+        """The finished 4-view image of LiDARAgent._generate_cluster_visualization (discs, axes, titles) of every view, in one
+        stream-ordered call per CLUSTER_VIEWS_WORKSPACE_PER_CALL bytes of workspace (msc_cluster_views_batch).  rows: f32 [*, 4] and
+        labels: i32 [*] CUDA tensors (e.g. a LidarBatchResult's object and labels); views: (row_begin, row_end, label) triples, the
+        points of a view being the rows of its range with its label, in row order.  max_view_points bounds the points of one view
+        (default: the longest range); a larger view raises in to_host().  Nothing is synchronised."""
+        v = np.ascontiguousarray(np.asarray(views, dtype=np.int64).reshape(-1, 3))
+        n = v.shape[0]
+        if not (isinstance(rows, torch.Tensor) and rows.is_cuda and rows.dtype == torch.float32 and rows.dim() == 2 and rows.shape[1] == 4
+                and isinstance(labels, torch.Tensor) and labels.is_cuda and labels.dtype == torch.int32):
+            raise _capi.MscError("run_cluster_views: rows must be f32 [*, 4] and labels i32 [*] CUDA tensors", _capi.MSC_ERR_BAD_ARGUMENT)
+        if n and (v[:, 0].min() < 0 or (v[:, 1] <= v[:, 0]).any() or v[:, 1].max() > min(rows.shape[0], labels.numel())):
+            raise _capi.MscError("run_cluster_views: a view's row range is empty, inverted or outside the rows", _capi.MSC_ERR_BAD_ARGUMENT)
+        if max_view_points is None:
+            max_view_points = int((v[:, 1] - v[:, 0]).max()) if n else 0
+        if out is None:
+            out = ClusterViewsResult(n, torch.empty((n, 512, 512, 3), dtype=torch.uint8, device=self.device),
+                                     torch.zeros(1, dtype=torch.int32, device=self.device))
+        if out.n_views != n:
+            raise _capi.MscError("run_cluster_views: the output buffers do not match the views", _capi.MSC_ERR_BAD_ARGUMENT)
+        out.status.zero_()
+        if n == 0:
+            return out
+        from .lidar_agent import cluster_view_stamp
+        stamp = self._stamp("cluster_view", cluster_view_stamp)
+        per = int(self.lib.msc_cluster_views_batch_workspace_bytes(1, int(max_view_points)))
+        if per == 0:
+            raise _capi.MscError("run_cluster_views: max_view_points %d out of range" % max_view_points, _capi.MSC_ERR_BAD_ARGUMENT)
+        step = max(1, min(n, 65535, CLUSTER_VIEWS_WORKSPACE_PER_CALL // per))
+        need = int(self.lib.msc_cluster_views_batch_workspace_bytes(step, int(max_view_points)))
+        ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        v32 = v.astype(np.int32)
+        rows, labels = rows.contiguous(), labels.contiguous()
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        for a in range(0, n, step):
+            k = min(step, n - a)
+            _capi.check(self.lib.msc_cluster_views_batch(rows.data_ptr(), labels.data_ptr(), v32[a:a + k].ctypes.data, k, int(max_view_points),
+                                                         stamp.data_ptr(), stamp.shape[0], out.images[a].data_ptr(), out.status.data_ptr(),
+                                                         ws.data_ptr(), need, stream), "msc_cluster_views_batch")
+            self.kernel_launches += 6
         return out
 
     # ------------------------------------------------------------------ camera frames -> JPEG files (CameraAgent._encode_image)

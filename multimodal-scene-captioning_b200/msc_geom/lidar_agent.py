@@ -8,7 +8,8 @@ What stays on the host, and why:
   * the cluster LIST ORDER follows CPython set iteration over the labels, like the reference (lidar_agent.py:154-159);
     DBSCAN itself runs on the device with scikit-learn's exact labelling (csrc/dbscan.cu).
   * the cv2 overlays drawn after the raster (lidar_agent.py:599-634) and the log1p density normalisation, which is
-    evaluated with NumPy's own float32 log1p through a count -> value table so the uint8 layer is bit-identical.
+    evaluated with NumPy's own float32 log1p through a count -> value table so the uint8 layer is bit-identical.  process_batch
+    draws both on the device for the whole batch, from the same table and from stamps of these same cv2 calls (overlay_stamp).
   * every remote LLM call: injected as callables (`llm`, `cluster_classifier`); absent callables yield the
     reference's own fallbacks ('unknown' clusters are dropped, lidar_agent.py:228).
 """
@@ -24,6 +25,7 @@ from . import ops
 from .engine import DeviceBatch, GeometryEngine
 from .layout import GeomParams, pack_batch
 
+CLUSTER_IMAGES_PER_CALL = 1024  # cluster images process_batch draws per device call and holds on the host (768 KiB each)
 DIRECTION_LABELS = ("front_right", "front", "front_left", "left", "back_left", "back", "back_right", "right")
 
 
@@ -53,12 +55,18 @@ def direction_label(position_2d) -> str:
     return DIRECTION_LABELS[7]
 
 
+def density_table(cmax: int) -> np.ndarray:
+    """log1p(c) for c = 0..cmax with NumPy's own float32 log1p (lidar_agent.py:563): the BEV density of a cell of c rows, on the host and
+    through msc_keyframe_bev_batch.  NumPy may pick a CPU-dependent SIMD log1p, so the table is always computed here, never on the device."""
+    return np.log1p(np.arange(cmax + 1, dtype=np.float32))
+
+
 def finish_bev_layers(count: np.ndarray, height: np.ndarray, semantic: np.ndarray, res: int, bev_range) -> Dict[str, np.ndarray]:
     """Host half of _generate_multi_layer_bev: density normalisation (lidar_agent.py:563-564), ego cross, vertical
     flips, range rings and labels (:599-634).  `count`/`height`/`semantic` are the unflipped GPU raster layers."""
     import cv2
     cmax = int(count.max()) if count.size else 0
-    lut = np.log1p(np.arange(cmax + 1, dtype=np.float32))  # NumPy's float32 log1p, one value per distinct count
+    lut = density_table(cmax)
     dens = lut[count.astype(np.int64)]
     density = (dens / dens.max() * 255).astype(np.uint8) if cmax > 0 else dens.astype(np.uint8)
     vis = np.ascontiguousarray(semantic)
@@ -90,6 +98,30 @@ def finish_cluster_view(grid: np.ndarray, img_size: int = 256) -> np.ndarray:
             cv2.line(grid, (ox + half, oy + half), (ox + half, oy + half - 30), (0, 255, 0), 2)   # y axis, green
         cv2.putText(grid, title, (ox + 10, oy + 20), cv2.FONT_HERSHEY_SIMPLEX, 0.5, (0, 0, 0), 1)
     return grid
+
+
+def overlay_stamp(draw: Callable[[np.ndarray], np.ndarray], h: int, w: int) -> np.ndarray:
+    """The pixels an opaque overlay sets, as u32 [m, 2] = (pixel y * w + x, B | G << 8 | R << 16): what `draw(canvas)` changes on an all-0
+    or an all-255 BGR canvas of h x w, with the colour it leaves there.  cv2's line / circle / putText with the default LINE_8 are opaque
+    (pixels and colours do not depend on the canvas), so writing the stamp over any raster equals drawing on it."""
+    lo, hi = draw(np.zeros((h, w, 3), np.uint8)), draw(np.full((h, w, 3), 255, np.uint8))
+    mask = (lo != 0).any(-1) | (hi != 255).any(-1)
+    if not np.array_equal(lo[mask], hi[mask]):
+        raise ValueError("overlay_stamp: the overlay depends on the canvas")
+    px = np.flatnonzero(mask.ravel())
+    c = lo.reshape(-1, 3)[px].astype(np.uint32)
+    return np.stack([px.astype(np.uint32), c[:, 0] | (c[:, 1] << 8) | (c[:, 2] << 16)], 1)
+
+
+def bev_stamp(res: int, bev_range) -> np.ndarray:
+    """The overlays of finish_bev_layers (ego cross, rings, labels) on a res x res BEV, as an overlay_stamp."""
+    zero = np.zeros((res, res), np.uint32)
+    return overlay_stamp(lambda canvas: finish_bev_layers(zero, zero.view(np.float32), canvas, res, bev_range)["semantic"], res, res)
+
+
+def cluster_view_stamp() -> np.ndarray:
+    """The axes and titles of finish_cluster_view on a 512 x 512 cluster image, as an overlay_stamp."""
+    return overlay_stamp(finish_cluster_view, 512, 512)
 
 
 def cluster_mosaic(images: List[np.ndarray]) -> np.ndarray:
@@ -287,36 +319,53 @@ class LiDARAgent:
         every sample's keyframe (sweep 0) in one device pass (GeometryEngine.run_lidar).  `device_batch` (e.g. engine.upload of
         io.stage_batch over lazy-loader samples, whose point_cloud is None) is used as it is; otherwise `samples` are packed and uploaded.
         The classifier sees the same images, mosaics and metadata in the same order as process's; the 800 x 800 BEV, which only the
-        scene interpretation reads, is drawn only when an llm is injected, and cluster images only when a classifier is."""
+        scene interpretation reads, is drawn only when an llm is injected (GeometryEngine.run_lidar_bev, enqueued behind run_lidar), and
+        cluster images only when a classifier is (GeometryEngine.run_cluster_views, CLUSTER_IMAGES_PER_CALL clusters at a time)."""
         eng = self.engine
         if device_batch is None:
             if samples is None:
                 raise ValueError("process_batch needs samples or a device_batch")
             device_batch = eng.upload(pack_batch(list(samples), n_cams=eng.params.n_cams))
         res = eng.run_lidar(device_batch, params=self._params(), eps=self.dbscan_eps, min_samples=self.dbscan_min_samples)
+        bev = eng.run_lidar_bev(res, int(self.bev_resolution), float(self.bev_range)) if self.llm is not None else None
         per = res.to_host()
+        bevs = bev.to_host(("semantic",)) if bev is not None else [None] * len(per)
+        orders = []
+        for r in per:
+            table = r["clusters"]
+            orders.append([l for l in set_order(r["cluster_first"], r["noise_first"]) if int(table[l, 10]) >= 5]
+                          if len(r["object"]) >= self.dbscan_min_samples else [])  # the guard of _detect_objects_3d
+        images = self._batch_cluster_images(res, per, orders) if self.cluster_classifier is not None else None
         contexts = list(contexts) if contexts is not None else [None] * len(per)
-        out = []
-        for s, r in enumerate(per):
-            ground, obj = r["ground"], r["object"]
+        out, base = [], 0
+        for s, (r, order) in enumerate(zip(per, orders)):
             detected: List[DetectedObject] = []
-            if len(obj) >= self.dbscan_min_samples:  # the guard of _detect_objects_3d
-                table = r["clusters"]
-                order = [l for l in set_order(r["cluster_first"], r["noise_first"]) if int(table[l, 10]) >= 5]
-                if order:
-                    labels = r["labels"]
-                    images_of = ((lambda a, b, obj=obj, labels=labels, order=order: self._cluster_visualizations(obj, labels, order[a:b]))
-                                 if self.cluster_classifier is not None else (lambda a, b: []))
-                    detected = self._classified_objects(self._metadata_of(table, order), images_of)
-            bev = None
-            if self.llm is not None:
-                res_px, rng = int(self.bev_resolution), self.bev_range
-                ng, no = len(ground), len(obj)
-                g0, o0 = r["ground_off"], r["object_off"]
-                count, height, sem = ops.keyframe_bev_layers_device(eng, res.ground[g0:g0 + ng], ng, res.object[o0:o0 + no], no, res_px, float(rng))
-                bev = finish_bev_layers(count, height, sem, res_px, rng)
-            out.append(self._result(detected, ground, obj, bev, contexts[s]))
+            if order:
+                images_of = (lambda a, b, o=base: images(o + a, o + b)) if images is not None else (lambda a, b: [])
+                detected = self._classified_objects(self._metadata_of(r["clusters"], order), images_of)
+            base += len(order)
+            out.append(self._result(detected, r["ground"], r["object"], bevs[s], contexts[s]))
         return out
+
+    def _batch_cluster_images(self, res, per: List[Dict[str, Any]], orders: List[List[int]]) -> Callable[[int, int], List[np.ndarray]]:
+        """images(a, b): the 4-view images of clusters a..b-1 of all samples' orders laid end to end, drawn on the device
+        CLUSTER_IMAGES_PER_CALL at a time as they are asked for (in increasing order)."""
+        views = np.array([(r["object_off"], r["object_off"] + len(r["object"]), l) for r, order in zip(per, orders) for l in order],
+                         np.int64).reshape(-1, 3)
+        sizes = np.array([int(r["clusters"][l, 10]) for r, order in zip(per, orders) for l in order], np.int64)
+        k, held = CLUSTER_IMAGES_PER_CALL, {}
+
+        def images(a: int, b: int) -> List[np.ndarray]:
+            got = []
+            for i in range(a, b):
+                c = i // k
+                if c not in held:
+                    held.clear()
+                    held[c] = self.engine.run_cluster_views(res.object, res.labels, views[c * k:(c + 1) * k],
+                                                            max_view_points=int(sizes[c * k:(c + 1) * k].max())).to_host()
+                got.append(held[c][i - c * k])
+            return got
+        return images
 
     def _result(self, detected: List[DetectedObject], ground: np.ndarray, obj: np.ndarray, bev: Optional[Dict[str, np.ndarray]],
                 context: Optional[Dict]) -> Dict[str, Any]:
