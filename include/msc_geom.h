@@ -362,6 +362,33 @@ int msc_lidar_batch(const msc_params* params, double eps, int32_t min_samples, c
                     void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * [EXT] LiDAR clusters -> annotated boxes, for every sample of an msc_lidar_batch result in one stream-ordered call.  `in` is the batch
+ * given to msc_lidar_batch and `rows` its output; n_samples must equal in->n_samples.  Box b of sample s is prepared as in the fused
+ * path (global -> ego_pose[s] -> lidar_calib[s] in f64, the points_in_box vectors rounded to f32) and an object row (x, y, z) of
+ * sample s -- as msc_lidar_batch wrote it, in the keyframe's sensor frame -- lies in it iff the devkit points_in_box test (App. A.2,
+ * f32 fmaf chains, closed intervals) holds; NaN rows lie in no box.  The normative definition is orc_cluster_match_sample of the test
+ * oracle.  Outputs (only these elements are written; the caller does not pre-fill):
+ *   cluster i32 [row_capacity, 3]: cluster k of sample s at row object_off[s] + k (k < n_clusters[s], the cluster table's indexing):
+ *           match_box (the sample-local box holding most of the cluster's rows; ties: the smaller index; -1: no row in any box),
+ *           match_points (its rows in that box), in_any_box (its rows inside at least one box);
+ *   box     i32 [in->n_boxes, 5]: rows (object rows inside, noise included), cluster_rows (rows inside with a label >= 0), clusters
+ *           (labels with a row inside), best_cluster (the label with most rows inside; ties: the smaller label; -1: none),
+ *           best_points (its rows inside).
+ * Any number of clusters and boxes per sample: work items of 128 boxes x 64 labels re-read the sample's rows.  Results are integers and do
+ * not depend on the launch shape or the row order.  A set msc_lidar_batch status means the rows, and so these results, must not be used.
+ * No host synchronisation, no allocation: workspace >= msc_cluster_match_batch_workspace_bytes(...) (O(row_capacity + n_boxes)),
+ * 256-byte aligned.  NULL arguments or buffers, a short workspace, n_samples different from the batch's and negative counts:
+ * MSC_ERR_BAD_ARGUMENT before anything is launched.  n_samples = 0 is a successful no-op.
+ */
+typedef struct {
+    int32_t* cluster; /* [row_capacity, 3] match_box, match_points, in_any_box                    */
+    int32_t* box;     /* [n_boxes, 5] rows, cluster_rows, clusters, best_cluster, best_points   */
+} msc_cluster_match_out;
+size_t msc_cluster_match_batch_workspace_bytes(int32_t n_samples, int32_t n_boxes, uint32_t row_capacity);
+int msc_cluster_match_batch(const msc_batch_in* in, const msc_lidar_batch_out* rows, int32_t n_samples, const msc_cluster_match_out* out,
+                            void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * The finished BEV of LiDARAgent._generate_multi_layer_bev (lidar_agent.py:539-634) for samples [first, first + n) of an
  * msc_lidar_batch result of n_samples samples, in one stream-ordered call.  From `rows` only ground, object, ground_off, object_off and
  * counts are read; from msc_params only bev_res (res) and bev_range.  Image i (sample first + i), byte-identical to the host path

@@ -303,6 +303,28 @@ static __device__ __noinline__ void rasterise_box(const FusedArgs& A, const floa
     }
 }
 
+// Prepared box record o[kBoxStride] (App. A.2) of a box already moved into the sensor frame -- centre c and rotation R, f64 without FMA
+// from the global frame through ego_pose (frame_change) and lidar_calib (frame_change) -- with box = center3, size (w, l, h), quat: the
+// devkit points_in_box vectors rounded to f32 (corner 0, the three edge vectors, their squared lengths) and the centre, for the cull
+// rasterisation.  fused_tables_kernel and csrc/cluster_match.cu share it; the frame changes stay at the call sites, because
+// fused_tables_kernel's instruction schedule changes when they move into a helper.
+__device__ __forceinline__ void box_record(const double* box, const double c[3], const double R[9], float* o) {
+    const double w = box[3], l = box[4], h = box[5];
+    const double hl = l / 2.0, hw = w / 2.0, hh = h / 2.0;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        o[r] = (float)(((R[r * 3 + 0] * hl + R[r * 3 + 1] * hw) + R[r * 3 + 2] * hh) + c[r]);
+        o[3 + r] = (float)(-(l * R[r * 3 + 0]));
+        o[6 + r] = (float)(-(w * R[r * 3 + 1]));
+        o[9 + r] = (float)(-(h * R[r * 3 + 2]));
+    }
+    o[12] = __fmaf_rn(o[5], o[5], __fmaf_rn(o[4], o[4], __fmul_rn(o[3], o[3])));
+    o[13] = __fmaf_rn(o[8], o[8], __fmaf_rn(o[7], o[7], __fmul_rn(o[6], o[6])));
+    o[14] = __fmaf_rn(o[11], o[11], __fmaf_rn(o[10], o[10], __fmul_rn(o[9], o[9])));
+    o[15] = 0.0f;
+    o[16] = (float)c[0]; o[17] = (float)c[1]; o[18] = (float)c[2]; o[19] = 0.0f;
+}
+
 // A.2 exact membership test of one point against one prepared box (closed intervals, float32 with fmaf chains).
 __device__ __forceinline__ bool box_contains(const float* __restrict__ boxp, int b, float xr, float yr, float zr) {
     const float4* bp = reinterpret_cast<const float4*>(boxp + b * kBoxStride);

@@ -73,21 +73,7 @@ __global__ void __launch_bounds__(256) fused_tables_kernel(const __grid_constant
         quat_to_rot(box + 6, R);
         frame_change(A.in.ego_pose + (size_t)sample * 7, c, R);
         frame_change(A.in.lidar_calib + (size_t)sample * 7, c, R);
-        const double w = box[3], l = box[4], h = box[5];
-        const double hl = l / 2.0, hw = w / 2.0, hh = h / 2.0;
-        float* o = boxprep + (size_t)gid * kBoxStride;
-#pragma unroll
-        for (int r = 0; r < 3; ++r) {
-            o[r] = (float)(((R[r * 3 + 0] * hl + R[r * 3 + 1] * hw) + R[r * 3 + 2] * hh) + c[r]);
-            o[3 + r] = (float)(-(l * R[r * 3 + 0]));
-            o[6 + r] = (float)(-(w * R[r * 3 + 1]));
-            o[9 + r] = (float)(-(h * R[r * 3 + 2]));
-        }
-        o[12] = __fmaf_rn(o[5], o[5], __fmaf_rn(o[4], o[4], __fmul_rn(o[3], o[3])));
-        o[13] = __fmaf_rn(o[8], o[8], __fmaf_rn(o[7], o[7], __fmul_rn(o[6], o[6])));
-        o[14] = __fmaf_rn(o[11], o[11], __fmaf_rn(o[10], o[10], __fmul_rn(o[9], o[9])));
-        o[15] = 0.0f;
-        o[16] = (float)c[0]; o[17] = (float)c[1]; o[18] = (float)c[2]; o[19] = 0.0f;  // centre, for the cull rasterisation
+        box_record(box, c, R, boxprep + (size_t)gid * kBoxStride);
     }
     // (2) box -> camera projection (App. A.3): one thread per (box, camera)
     if (n_cams > 0 && gid < n_boxes_total * n_cams) {

@@ -64,6 +64,10 @@ class MscLidarBatchOut(C.Structure):
                 ("noise_first", C.c_void_p), ("status", C.c_void_p)]
 
 
+class MscClusterMatchOut(C.Structure):
+    _fields_ = [("cluster", C.c_void_p), ("box", C.c_void_p)]
+
+
 class MscJpegComp(C.Structure):
     _fields_ = [("h", C.c_int32), ("v", C.c_int32), ("blocks_x", C.c_int32), ("blocks_y", C.c_int32), ("ds_w", C.c_int32), ("ds_h", C.c_int32),
                 ("coef_off", C.c_int64), ("plane_off", C.c_int64), ("qt", C.c_uint16 * 64)]
@@ -113,6 +117,9 @@ _PROTOS = {
     "msc_lidar_batch_workspace_bytes": (C.c_size_t, [C.POINTER(MscParams), C.c_double, C.c_int32, C.c_uint32]),
     "msc_lidar_batch": (C.c_int, [C.POINTER(MscParams), C.c_double, C.c_int32, C.POINTER(MscBatchIn), C.POINTER(MscLidarBatchOut), C.c_void_p,
                                   C.c_size_t, C.c_void_p]),
+    "msc_cluster_match_batch_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_uint32]),
+    "msc_cluster_match_batch": (C.c_int, [C.POINTER(MscBatchIn), C.POINTER(MscLidarBatchOut), C.c_int32, C.POINTER(MscClusterMatchOut), C.c_void_p,
+                                          C.c_size_t, C.c_void_p]),
     "msc_jpeg_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc)]),
     "msc_jpeg_entropy_decode_host": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc), C.c_void_p]),
     "msc_jpeg_reconstruct": (C.c_int, [C.POINTER(MscJpegDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -213,6 +213,41 @@ class LidarBatchResult:
 
 
 @dataclass
+class ClusterMatchResult:
+    """Outputs of msc_cluster_match_batch (which annotated box each cluster of a run_lidar result lies in), still on the device."""
+    lidar: LidarBatchResult      # the run_lidar result the match was computed from (its status word and per-sample tables)
+    sample_box_off: np.ndarray
+    cluster: torch.Tensor        # i32 [cap, 3] match_box, match_points, in_any_box; cluster k of sample s at object_off[s] + k
+    box: torch.Tensor            # i32 [B, 5] rows, cluster_rows, clusters, best_cluster, best_points
+    workspace: torch.Tensor      # u8, msc_cluster_match_batch_workspace_bytes
+
+    def struct(self) -> _capi.MscClusterMatchOut:
+        return _capi.MscClusterMatchOut(self.cluster.data_ptr() or None, self.box.data_ptr() or None)
+
+    def to_host(self) -> List[Dict[str, np.ndarray]]:
+        """Per sample: "cluster_match" (K_s, 3) i32, row k = cluster k of the sample (match_box as a sample-local box index, -1 none;
+        match_points; in_any_box), "box_match" (B_s, 5) i32, row j = the sample's box j (rows, cluster_rows, clusters, best_cluster as a
+        sample-local label, -1 none; best_points), and "object_off" / "box_off", where the sample's clusters and boxes start in the
+        device tables.  This is the synchronisation point; a set msc_lidar_batch status word raises MscError (the rows were invalid)."""
+        lr = self.lidar
+        S = lr.n_samples
+        small = lr.small.cpu().numpy()
+        status = int(small[0]) if small.size else 0
+        if status:
+            raise _capi.MscError("msc_cluster_match_batch: the msc_lidar_batch status is 0x%x, its rows and the match must not be used" % status,
+                                 status)
+        tab = small[1:].reshape(7, S) if S else np.zeros((7, 0), np.int32)
+        counts, ooff, ncl = tab[0:3].reshape(S, 3).astype(np.int64), tab[4].astype(np.int64), tab[5].astype(np.int64)
+        M = int(counts[:, 2].sum())
+        cl, bx = self.cluster[:M].cpu().numpy(), self.box.cpu().numpy()
+        out = []
+        for s in range(S):
+            o0, b0, b1 = int(ooff[s]), int(self.sample_box_off[s]), int(self.sample_box_off[s + 1])
+            out.append({"cluster_match": cl[o0:o0 + int(ncl[s])], "box_match": bx[b0:b1], "object_off": o0, "box_off": b0})
+        return out
+
+
+@dataclass
 class LidarBevResult:
     """Finished BEVs of msc_keyframe_bev_batch for samples first .. first + n_samples - 1 of a LidarBatchResult, still on the device."""
     first: int
@@ -551,6 +586,34 @@ class GeometryEngine:
                                              need, C.c_void_p(stream)), "msc_lidar_batch")
         if hb.n_samples > 0:
             self.kernel_launches += 15  # 13 own kernels + the CUB sort and scan (each of those launches several kernels of its own)
+        return out
+
+    # ------------------------------------------------------------------ LiDAR clusters -> annotated boxes ([EXT])
+    def alloc_cluster_match(self, lr: LidarBatchResult, hb: HostBatch) -> ClusterMatchResult:
+        """Output buffers and workspace of run_cluster_match for the run_lidar result `lr` of the batch `hb`."""
+        need = int(self.lib.msc_cluster_match_batch_workspace_bytes(hb.n_samples, hb.n_boxes, lr.row_capacity))
+        if need == 0 and hb.n_samples > 0:
+            raise _capi.MscError("alloc_cluster_match: row_capacity %d is out of range" % lr.row_capacity, _capi.MSC_ERR_BAD_ARGUMENT)
+        d = self.device
+        return ClusterMatchResult(lr, hb.sample_box_off.copy(), torch.empty((lr.row_capacity, 3), dtype=torch.int32, device=d),
+                                  torch.empty((hb.n_boxes, 5), dtype=torch.int32, device=d), torch.empty(max(need, 256), dtype=torch.uint8, device=d))
+
+    def run_cluster_match(self, lr: LidarBatchResult, db: DeviceBatch, out: Optional[ClusterMatchResult] = None) -> ClusterMatchResult:
+        """Which annotated box each cluster of `lr` lies in, and which clusters each box holds, for every sample of the device-resident
+        batch `db` that `lr` was computed from (msc_cluster_match_batch), stream-ordered behind run_lidar.  With `out` given nothing is
+        allocated.  Nothing is synchronised; out.to_host() reads the results."""
+        hb = db.host
+        if out is None:
+            out = self.alloc_cluster_match(lr, hb)
+        if (lr.n_samples != hb.n_samples or out.lidar is not lr or tuple(out.cluster.shape) != (lr.row_capacity, 3)
+                or tuple(out.box.shape) != (hb.n_boxes, 5) or not np.array_equal(out.sample_box_off, hb.sample_box_off)):
+            raise _capi.MscError("run_cluster_match: the output buffers do not match the batch and its run_lidar result", _capi.MSC_ERR_BAD_ARGUMENT)
+        bi, rows, bo = db.struct(), lr.struct(), out.struct()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _capi.check(self.lib.msc_cluster_match_batch(C.byref(bi), C.byref(rows), hb.n_samples, C.byref(bo), out.workspace.data_ptr(),
+                                                     out.workspace.numel(), C.c_void_p(stream)), "msc_cluster_match_batch")
+        if hb.n_samples > 0:
+            self.kernel_launches += 3
         return out
 
     # ------------------------------------------------------------------ the LiDAR agent's images, batched

@@ -156,6 +156,27 @@ def set_order(cluster_first, noise_first: int) -> List[int]:
     return list(uniq)
 
 
+def annotation_match(order: List[int], clusters: np.ndarray, cluster_match: np.ndarray, box_match: np.ndarray,
+                     annotations: Optional[Sequence[dict]] = None) -> Dict[str, List[dict]]:
+    """The "annotation_match" of one sample (LiDARAgent.process_batch(match_annotations=True)) from its run_lidar cluster table
+    `clusters` (K, 11), its run_cluster_match tables cluster_match (K, 3) and box_match (B, 5) and the classifier's cluster order:
+      clusters:    per cluster of `order`, in that order: index (its position in `order`), num_points, annotation ("obj_<j>": the
+                   annotation j holding most of its rows; None: no row in any box), category (that annotation's category_name when the
+                   annotation dicts are given, else None) and points_in_annotation (its rows inside annotation j);
+      annotations: per annotation j: id "obj_<j>", rows (object rows inside, noise included), clusters (clusters with a row inside) and
+                   best_cluster (the index in `clusters` of the cluster with most rows inside; None when there is none or it is not in
+                   the classifier's order)."""
+    index_of = {int(l): i for i, l in enumerate(order)}
+    cl = []
+    for i, l in enumerate(order):
+        b, pts = int(cluster_match[l, 0]), int(cluster_match[l, 1])
+        cat = str(annotations[b].get("category_name", "unknown")) if annotations is not None and b >= 0 else None
+        cl.append({"index": i, "num_points": int(clusters[l, 10]), "annotation": f"obj_{b}" if b >= 0 else None, "category": cat,
+                   "points_in_annotation": pts})
+    anns = [{"id": f"obj_{j}", "rows": int(r[0]), "clusters": int(r[2]), "best_cluster": index_of.get(int(r[3]))} for j, r in enumerate(box_match)]
+    return {"clusters": cl, "annotations": anns}
+
+
 class LiDARAgent:
     def __init__(self, client, model: str, agent_name: str, engine: Optional[GeometryEngine] = None,
                  llm: Optional[Callable[..., str]] = None, cluster_classifier: Optional[Callable[..., List[dict]]] = None):
@@ -314,21 +335,29 @@ class LiDARAgent:
         return self._result(detected, ground, obj, bev, context)
 
     def process_batch(self, samples: Optional[Sequence[dict]] = None, device_batch: Optional[DeviceBatch] = None,
-                      contexts: Optional[Sequence[Optional[Dict]]] = None) -> List[Dict[str, Any]]:
+                      contexts: Optional[Sequence[Optional[Dict]]] = None, match_annotations: bool = False,
+                      annotations: Optional[Sequence[Sequence[dict]]] = None) -> List[Dict[str, Any]]:
         """[process(sample["point_cloud"], context) for each sample], with the filter, the ground split, DBSCAN and the cluster boxes of
         every sample's keyframe (sweep 0) in one device pass (GeometryEngine.run_lidar).  `device_batch` (e.g. engine.upload of
         io.stage_batch over lazy-loader samples, whose point_cloud is None) is used as it is; otherwise `samples` are packed and uploaded.
         The classifier sees the same images, mosaics and metadata in the same order as process's; the 800 x 800 BEV, which only the
         scene interpretation reads, is drawn only when an llm is injected (GeometryEngine.run_lidar_bev, enqueued behind run_lidar), and
-        cluster images only when a classifier is (GeometryEngine.run_cluster_views, CLUSTER_IMAGES_PER_CALL clusters at a time)."""
+        cluster images only when a classifier is (GeometryEngine.run_cluster_views, CLUSTER_IMAGES_PER_CALL clusters at a time).
+        match_annotations=True adds to each result the key "annotation_match" (lidar_agent.annotation_match): which annotated box each
+        cluster of the classifier's order lies in and which clusters each box holds (GeometryEngine.run_cluster_match, enqueued behind
+        run_lidar).  Categories come from the samples' annotation dicts, or from `annotations` (one list per sample) for a device_batch."""
         eng = self.engine
         if device_batch is None:
             if samples is None:
                 raise ValueError("process_batch needs samples or a device_batch")
             device_batch = eng.upload(pack_batch(list(samples), n_cams=eng.params.n_cams))
         res = eng.run_lidar(device_batch, params=self._params(), eps=self.dbscan_eps, min_samples=self.dbscan_min_samples)
+        match = eng.run_cluster_match(res, device_batch) if match_annotations else None
         bev = eng.run_lidar_bev(res, int(self.bev_resolution), float(self.bev_range)) if self.llm is not None else None
         per = res.to_host()
+        matches = match.to_host() if match is not None else None
+        if annotations is None and samples is not None:
+            annotations = [s.get("annotations", []) for s in samples]
         bevs = bev.to_host(("semantic",)) if bev is not None else [None] * len(per)
         orders = []
         for r in per:
@@ -345,6 +374,9 @@ class LiDARAgent:
                 detected = self._classified_objects(self._metadata_of(r["clusters"], order), images_of)
             base += len(order)
             out.append(self._result(detected, r["ground"], r["object"], bevs[s], contexts[s]))
+            if matches is not None:
+                out[-1]["annotation_match"] = annotation_match(order, r["clusters"], matches[s]["cluster_match"], matches[s]["box_match"],
+                                                               annotations[s] if annotations is not None else None)
         return out
 
     def _batch_cluster_images(self, res, per: List[Dict[str, Any]], orders: List[List[int]]) -> Callable[[int, int], List[np.ndarray]]:

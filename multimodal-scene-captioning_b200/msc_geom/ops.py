@@ -187,6 +187,21 @@ def camera_depth(eng: GeometryEngine, sample: dict, dp: Optional[DepthParams] = 
     return {"depth": out["depth"][0], "cam_points": out["cam_points"][0], "box_support": out["box_support"]}
 
 
+def cluster_match(eng: GeometryEngine, sample: dict, params: Optional[GeomParams] = None, eps: float = 0.5,
+                  min_samples: int = 10) -> Dict[str, np.ndarray]:
+    """[EXT] Which annotated box each LiDAR cluster of one loader sample's keyframe lies in: the batched calls (GeometryEngine.run_lidar,
+    then run_cluster_match) on a one-sample batch.  Returns that sample's dict of ClusterMatchResult.to_host() -- cluster_match (K, 3)
+    and box_match (B, 5) -- plus the run_lidar rows it was computed from (object, labels, clusters)."""
+    p = params or eng.params
+    db = eng.upload(pack_batch([sample], n_cams=p.n_cams))
+    lr = eng.run_lidar(db, params=p, eps=eps, min_samples=min_samples)
+    m = eng.run_cluster_match(lr, db)
+    rows = lr.to_host()[0]
+    out = m.to_host()[0]
+    out.update({k: rows[k] for k in ("object", "labels", "clusters")})
+    return out
+
+
 def aggregate_sweeps(eng: GeometryEngine, sweeps, remove_close_radius: float = 1.0):
     """[EXT] devkit LidarPointCloud.from_file_multisweep (App. A.1): sweeps = [(raw (n,5) f32, M 3x4 f64, time_lag)];
     returns (N,4) f32 rows x', y', z', intensity and (N,) f32 time lags, order-preserving."""

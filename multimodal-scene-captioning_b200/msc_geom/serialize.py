@@ -75,11 +75,12 @@ def jpeg_base64(img: np.ndarray) -> str:
 
 def ext_evidence(annotations: Sequence[Dict], box_count: np.ndarray, box_nearest: np.ndarray, box_centroid: np.ndarray,
                  proj_visible: np.ndarray, camera_names: Sequence[str], relations: Optional[Dict[str, Any]] = None,
-                 max_pairs: int = 20, camera_support: Optional[np.ndarray] = None) -> Dict[str, Any]:
+                 max_pairs: int = 20, camera_support: Optional[np.ndarray] = None, cluster_match: Optional[np.ndarray] = None) -> Dict[str, Any]:
     """[EXT] evidence of one sample (rows e3, e5, e6 of SURVEY.md section 8a) as a JSON-serialisable dict: the `context` a caller
     hands to CameraAgent.process / SceneGraphAgent.process.  Floats are rounded the way the reference rounds distances (1 decimal).
     camera_support: the sample's box_support [B, C, 4] of msc_camera_depth_batch (row e7); adds per object "lidar_in_camera" with the
-    block counts of every camera the box is visible in."""
+    block counts of every camera the box is visible in.  cluster_match: the sample's box table [B, 5] of msc_cluster_match_batch; adds per
+    object "lidar_cluster" with the object rows inside the box and the LiDAR clusters they belong to, for boxes that hold a cluster."""
     objs = []
     for i, a in enumerate(annotations):
         n = int(box_count[i])
@@ -91,6 +92,8 @@ def ext_evidence(annotations: Sequence[Dict], box_count: np.ndarray, box_nearest
             objs[-1]["lidar_in_camera"] = {camera_names[c]: {"blocks": int(camera_support[i, c, 0]), "blocks_with_returns": int(camera_support[i, c, 1]),
                                                              "on_object": int(camera_support[i, c, 3]), "occluded": int(camera_support[i, c, 2])}
                                            for c in range(len(camera_names)) if camera_support[i, c, 0]}
+        if cluster_match is not None and int(cluster_match[i, 2]) > 0:
+            objs[-1]["lidar_cluster"] = {"rows": int(cluster_match[i, 0]), "clusters": int(cluster_match[i, 2])}
     out: Dict[str, Any] = {"objects": objs}
     if relations is not None:
         labels = relations.get("labels", ("ahead", "left", "behind", "right"))
