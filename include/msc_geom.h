@@ -245,6 +245,51 @@ int msc_jpeg_entropy_decode_host(const uint8_t* jpeg_host, size_t nbytes, const 
 int msc_jpeg_reconstruct(const msc_jpeg_desc* desc_host, const int16_t* coef, uint8_t* planes, uint8_t* out, void* stream);
 
 /*
+ * Batched camera-frame decode with every stage on the device, the Huffman decode included (DESIGN.md section 4.9).
+ *
+ * msc_jpeg_decode_plan (host only) parses a file's headers with the same parser as msc_jpeg_info -- so it accepts and refuses exactly
+ * the same files with the same status -- and fills a fixed-size record: the descriptor, where the entropy-coded scan lies in the file
+ * (scan_off: the byte after the SOS header; scan_bytes: from there to the end of the file), the restart interval, the per-component
+ * Huffman table selectors and the decode tables of every table the file defines (Annex F.2.2.3, plus a 9-bit lookahead).
+ *
+ * msc_jpeg_decode_batch decodes n files in one stream-ordered call.  files: device bytes, file i at files[file_off_host[i]] (its
+ * plans_host[i] must come from those bytes).  Image i writes
+ *   coef[coef_off_host[i] .. + plans_host[i].desc.coef_elems): int16, equal to msc_jpeg_entropy_decode_host (per component
+ *          [blocks_y][blocks_x][64], natural order, DC predicted); `coef` must be 16-byte aligned and coef_off_host[i] a multiple of 8;
+ *   out[out_off_host[i] ..): the frame, equal to msc_jpeg_reconstruct -- [height][width][3] RGB u8, or [height][width] for one component;
+ *   status[i] (device i32): 0, or MSC_ERR_BAD_ARGUMENT where msc_jpeg_entropy_decode_host fails (a corrupt code, a DC size above 15,
+ *          an AC run past coefficient 63, a missing restart marker).  A failed image's coef and out regions hold unspecified values;
+ *          every other image of the call is decoded exactly, and nothing outside the n regions is written.
+ * The bit stream reads like the host decoder's: a stuffed FF 00 is one FF byte; at any other marker, and past the end of the file, it
+ * reads as zero bits; decoding stops at the MCU count.  With a restart interval, segment k starts after the k-th FF D0..D7 of the scan.
+ * Four launches whatever the data, no allocation, no host synchronisation; plans_host and the offsets are copied into the workspace
+ * (one cudaMemcpyAsync), so they may be reused when the call returns.  workspace >= msc_jpeg_decode_batch_workspace_bytes(n, plans_host)
+ * bytes, 256-byte aligned (0 = arguments out of range).  n < 0, a NULL pointer with n > 0, a plan that is not a supported sequential
+ * file, a scan of 2^28 bytes or more, a misaligned `coef` or coef offset, a workspace that is short or not 256-byte aligned:
+ * MSC_ERR_BAD_ARGUMENT before anything is launched.
+ * n = 0 is a successful no-op.
+ */
+typedef struct {
+    uint16_t look[512];  /* 9-bit lookahead: (code length << 8) | symbol, 0 = the code is longer than 9 bits */
+    int32_t maxcode[18]; /* per code length the largest code, -1 when there is none                          */
+    int32_t valptr[17];  /* per code length: index in vals of its first symbol minus its first code          */
+    uint8_t vals[256];   /* symbols in code order                                                           */
+} msc_jpeg_huff;
+typedef struct {
+    msc_jpeg_desc desc;
+    int64_t scan_off, scan_bytes;
+    int32_t restart_interval; /* MCUs per restart segment, 0 = none */
+    int32_t td[3], ta[3];     /* DC / AC table of each component     */
+    int32_t reserved_;
+    msc_jpeg_huff dc[4], ac[4]; /* tables the file does not define are zero */
+} msc_jpeg_plan;
+int msc_jpeg_decode_plan(const uint8_t* jpeg_host, size_t nbytes, msc_jpeg_plan* plan_host);
+size_t msc_jpeg_decode_batch_workspace_bytes(int32_t n, const msc_jpeg_plan* plans_host);
+int msc_jpeg_decode_batch(int32_t n, const msc_jpeg_plan* plans_host, const uint8_t* files, const int64_t* file_off_host, int16_t* coef,
+                          const int64_t* coef_off_host, uint8_t* out, const int64_t* out_off_host, int32_t* status, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
+/*
  * Camera-frame encode (CameraAgent._encode_image, camera_agent.py:128-137): image i of the batch becomes, byte for byte, the file
  * `PIL.Image.fromarray(rgb[i]).save(buf, "JPEG", quality=quality)` writes -- libjpeg-turbo's default compression: JFIF 1.01, 4:2:0, the
  * Annex K tables (quantisation scaled by jpeg_set_quality, standard Huffman tables), slow-integer FDCT, no restart markers.

@@ -302,14 +302,6 @@ static int entropy_decode(ParsedJpeg& J, int16_t* coef) {
 }
 
 // ------------------------------------------------------------------------------------------------ device: IDCT, upsampling, colour
-// jidctint.c (jpeg_idct_islow): CONST_BITS 13, PASS1_BITS 2, the thirteen FIX() constants
-__device__ __forceinline__ int jd_descale(int x, int n) { return (x + (1 << (n - 1))) >> n; }
-// IDCT_range_limit(cinfo)[x & RANGE_MASK] with the table of jdmaster.c:prepare_range_limit_table (centre 128, 10-bit wrap)
-__device__ __forceinline__ uint8_t jd_idct_limit(int x) {
-    const int v = x & 1023;
-    return (uint8_t)(v < 128 ? 128 + v : v < 512 ? 255 : v < 896 ? 0 : v - 896);
-}
-
 struct IdctParams {
     const int16_t* coef;
     uint8_t* plane;
@@ -323,44 +315,18 @@ __global__ void __launch_bounds__(256) jpeg_idct_kernel(const IdctParams P) {
     const int lb = threadIdx.x >> 3, j = threadIdx.x & 7;
     const int b = blockIdx.x * 32 + lb;
     const bool live = b < P.n_blocks;
-    constexpr int C298 = 2446, C390 = 3196, C541 = 4433, C765 = 6270, C899 = 7373, C1175 = 9633, C1501 = 12299, C1847 = 15137, C1961 = 16069,
-                  C2053 = 16819, C2562 = 20995, C3072 = 25172;
-    auto butterfly = [&](int d0, int d1, int d2, int d3, int d4, int d5, int d6, int d7, int o[8], int shift) {
-        // even part
-        int z2 = d2, z3 = d6;
-        int z1 = (z2 + z3) * C541;
-        int tmp2 = z1 + z3 * (-C1847);
-        int tmp3 = z1 + z2 * C765;
-        z2 = d0; z3 = d4;
-        int tmp0 = (z2 + z3) << 13;
-        int tmp1 = (z2 - z3) << 13;
-        const int tmp10 = tmp0 + tmp3, tmp13 = tmp0 - tmp3, tmp11 = tmp1 + tmp2, tmp12 = tmp1 - tmp2;
-        // odd part
-        tmp0 = d7; tmp1 = d5; tmp2 = d3; tmp3 = d1;
-        z1 = tmp0 + tmp3; z2 = tmp1 + tmp2; z3 = tmp0 + tmp2;
-        int z4 = tmp1 + tmp3;
-        const int z5 = (z3 + z4) * C1175;
-        tmp0 *= C298; tmp1 *= C2053; tmp2 *= C3072; tmp3 *= C1501;
-        z1 *= -C899; z2 *= -C2562; z3 *= -C1961; z4 *= -C390;
-        z3 += z5; z4 += z5;
-        tmp0 += z1 + z3; tmp1 += z2 + z4; tmp2 += z2 + z3; tmp3 += z1 + z4;
-        o[0] = jd_descale(tmp10 + tmp3, shift); o[7] = jd_descale(tmp10 - tmp3, shift);
-        o[1] = jd_descale(tmp11 + tmp2, shift); o[6] = jd_descale(tmp11 - tmp2, shift);
-        o[2] = jd_descale(tmp12 + tmp1, shift); o[5] = jd_descale(tmp12 - tmp1, shift);
-        o[3] = jd_descale(tmp13 + tmp0, shift); o[4] = jd_descale(tmp13 - tmp0, shift);
-    };
     int o[8];
     if (live) {  // pass 1: columns, dequantised input, results scaled up by 2^PASS1_BITS
         const int16_t* c = P.coef + (size_t)b * 64 + j;
-        butterfly(c[0] * (int)P.qt[j], c[8] * (int)P.qt[8 + j], c[16] * (int)P.qt[16 + j], c[24] * (int)P.qt[24 + j], c[32] * (int)P.qt[32 + j],
-                  c[40] * (int)P.qt[40 + j], c[48] * (int)P.qt[48 + j], c[56] * (int)P.qt[56 + j], o, 13 - 2);
+        jd_butterfly(c[0] * (int)P.qt[j], c[8] * (int)P.qt[8 + j], c[16] * (int)P.qt[16 + j], c[24] * (int)P.qt[24 + j], c[32] * (int)P.qt[32 + j],
+                     c[40] * (int)P.qt[40 + j], c[48] * (int)P.qt[48 + j], c[56] * (int)P.qt[56 + j], o, 13 - 2);
 #pragma unroll
         for (int r = 0; r < 8; ++r) ws[lb][r * 8 + j] = o[r];
     }
     __syncthreads();
     if (live) {  // pass 2: rows, descale by CONST_BITS + PASS1_BITS + 3, level shift + range limit
         const int* w = &ws[lb][j * 8];
-        butterfly(w[0], w[1], w[2], w[3], w[4], w[5], w[6], w[7], o, 13 + 2 + 3);
+        jd_butterfly(w[0], w[1], w[2], w[3], w[4], w[5], w[6], w[7], o, 13 + 2 + 3);
         const int bx = b % P.blocks_x, by = b / P.blocks_x;
         uint8_t* dst = P.plane + ((size_t)(by * 8 + j) * P.blocks_x + bx) * 8;
         uint2 pk;
@@ -381,34 +347,6 @@ struct ColorParams {
     int hsub, vsub;          // 1 or 2
 };
 
-// one chroma sample at full resolution: jdsample.c fullsize / h2v1_fancy / h2v2_fancy (fancy only when downsampled_width > 2, else replication)
-__device__ __forceinline__ int jd_chroma(const uint8_t* __restrict__ pl, int stride, int cw, int ch, int hsub, int vsub, int x, int y) {
-    if (hsub == 1) return pl[(size_t)y * stride + x];
-    const int ix = x >> 1;
-    if (cw <= 2) return pl[(size_t)(vsub == 2 ? (y >> 1) : y) * stride + ix];  // h2v1_upsample / h2v2_upsample: plain replication
-    if (vsub == 1) {  // h2v1_fancy_upsample: 3/4 nearer + 1/4 further, rounding 1 on the left sample of a pair, 2 on the right one
-        const uint8_t* r = pl + (size_t)y * stride;
-        const int v = r[ix];
-        if ((x & 1) == 0) return ix == 0 ? v : (v * 3 + r[ix - 1] + 1) >> 2;
-        return ix == cw - 1 ? v : (v * 3 + r[ix + 1] + 2) >> 2;
-    }
-    // h2v2_fancy_upsample: column sums 3 * nearer row + further row, then the same filter horizontally with rounding 8 / 7 and >> 4
-    const int iy = y >> 1;
-    int ny = (y & 1) ? iy + 1 : iy - 1;  // further row: above for the upper output row of a pair, below for the lower one
-    ny = ny < 0 ? 0 : (ny > ch - 1 ? ch - 1 : ny);  // (context rows at the image edges duplicate the edge row, jdmainct.c)
-    const uint8_t* r0 = pl + (size_t)iy * stride;
-    const uint8_t* r1 = pl + (size_t)ny * stride;
-    const int cs = r0[ix] * 3 + r1[ix];
-    if ((x & 1) == 0) {
-        if (ix == 0) return (cs * 4 + 8) >> 4;
-        return (cs * 3 + (r0[ix - 1] * 3 + r1[ix - 1]) + 8) >> 4;
-    }
-    if (ix == cw - 1) return (cs * 4 + 7) >> 4;
-    return (cs * 3 + (r0[ix + 1] * 3 + r1[ix + 1]) + 7) >> 4;
-}
-
-__device__ __forceinline__ uint8_t jd_clamp(int v) { return (uint8_t)(v < 0 ? 0 : (v > 255 ? 255 : v)); }
-
 __global__ void __launch_bounds__(256) jpeg_color_kernel(const ColorParams P) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
     if (x >= P.width || y >= P.height) return;
@@ -419,13 +357,7 @@ __global__ void __launch_bounds__(256) jpeg_color_kernel(const ColorParams P) {
     }
     const int cb = jd_chroma(P.cb, P.c_stride, P.c_w, P.c_h, P.hsub, P.vsub, x, y) - 128;
     const int cr = jd_chroma(P.cr, P.c_stride, P.c_w, P.c_h, P.hsub, P.vsub, x, y) - 128;
-    // jdcolor.c build_ycc_rgb_table + ycc_rgb_convert: SCALEBITS 16, FIX(1.40200) = 91881, FIX(1.77200) = 116130, FIX(0.71414) = 46802,
-    // FIX(0.34414) = 22554, ONE_HALF = 32768
-    const int r = Y + ((91881 * cr + 32768) >> 16);
-    const int b = Y + ((116130 * cb + 32768) >> 16);
-    const int g = Y + (((-22554) * cb + 32768 + (-46802) * cr) >> 16);
-    uint8_t* o = P.out + ((size_t)y * P.width + x) * 3;
-    o[0] = jd_clamp(r); o[1] = jd_clamp(g); o[2] = jd_clamp(b);
+    jd_ycc_rgb(Y, cb, cr, P.out + ((size_t)y * P.width + x) * 3);
 }
 
 }  // namespace msc
@@ -450,6 +382,32 @@ int msc_jpeg_entropy_decode_host(const uint8_t* jpeg_host, size_t nbytes, const 
     if (rc != MSC_OK) return rc;
     MSC_REQUIRE(J.d.coef_elems == desc->coef_elems && J.d.width == desc->width && J.d.height == desc->height, "descriptor does not belong to this stream");
     return entropy_decode(J, coef_host);
+}
+
+int msc_jpeg_decode_plan(const uint8_t* jpeg_host, size_t nbytes, msc_jpeg_plan* plan) {
+    using namespace msc;
+    MSC_REQUIRE(jpeg_host && plan, "null argument");
+    ParsedJpeg J;
+    const int rc = parse_headers(jpeg_host, nbytes, &J);
+    if (rc != MSC_OK) return rc;
+    memset(plan, 0, sizeof(*plan));
+    plan->desc = J.d;
+    plan->scan_off = (int64_t)(J.scan - jpeg_host);
+    plan->scan_bytes = (int64_t)(J.end - J.scan);
+    plan->restart_interval = J.restart_interval;
+    for (int c = 0; c < 3; ++c) { plan->td[c] = J.td[c]; plan->ta[c] = J.ta[c]; }
+    for (int t = 0; t < 4; ++t) {
+        const HuffTable* src[2] = {&J.dc[t], &J.ac[t]};
+        msc_jpeg_huff* dst[2] = {&plan->dc[t], &plan->ac[t]};
+        for (int k = 0; k < 2; ++k) {
+            if (!src[k]->present) continue;
+            memcpy(dst[k]->look, src[k]->look, sizeof(dst[k]->look));
+            for (int l = 1; l <= 17; ++l) dst[k]->maxcode[l] = src[k]->maxcode[l];  // (entry 0 is unused; valptr is set for used lengths only)
+            for (int l = 1; l <= 16; ++l) dst[k]->valptr[l] = src[k]->bits[l] ? src[k]->valptr[l] : 0;
+            memcpy(dst[k]->vals, src[k]->vals, sizeof(dst[k]->vals));
+        }
+    }
+    return MSC_OK;
 }
 
 int msc_jpeg_reconstruct(const msc_jpeg_desc* desc, const int16_t* coef, uint8_t* planes, uint8_t* out, void* stream_v) {

@@ -78,6 +78,15 @@ class MscJpegDesc(C.Structure):
                 ("mcus_y", C.c_int32), ("reserved_", C.c_int32), ("coef_elems", C.c_int64), ("plane_bytes", C.c_int64), ("comp", MscJpegComp * 3)]
 
 
+class MscJpegHuff(C.Structure):
+    _fields_ = [("look", C.c_uint16 * 512), ("maxcode", C.c_int32 * 18), ("valptr", C.c_int32 * 17), ("vals", C.c_uint8 * 256)]
+
+
+class MscJpegPlan(C.Structure):
+    _fields_ = [("desc", MscJpegDesc), ("scan_off", C.c_int64), ("scan_bytes", C.c_int64), ("restart_interval", C.c_int32), ("td", C.c_int32 * 3),
+                ("ta", C.c_int32 * 3), ("reserved_", C.c_int32), ("dc", MscJpegHuff * 4), ("ac", MscJpegHuff * 4)]
+
+
 _lib = None
 
 _PROTOS = {
@@ -123,6 +132,10 @@ _PROTOS = {
     "msc_jpeg_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc)]),
     "msc_jpeg_entropy_decode_host": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(MscJpegDesc), C.c_void_p]),
     "msc_jpeg_reconstruct": (C.c_int, [C.POINTER(MscJpegDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "msc_jpeg_decode_plan": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p]),
+    "msc_jpeg_decode_batch_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_void_p]),
+    "msc_jpeg_decode_batch": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_size_t, C.c_void_p]),
     "msc_jpeg_encode_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_size_t]),
     "msc_jpeg_encode_batch": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -316,6 +316,62 @@ class JpegBatchResult:
         return [data[off[i]:off[i + 1]] for i in range(self.n_images)]
 
 
+# Workspace bytes of one msc_jpeg_decode_batch call (a 1600 x 900 4:2:0 frame needs about 2.5 MB).  It bounds the workspace only: the
+# coefficient (4.4 MB) and frame (4.3 MB) arenas of a 1600 x 900 frame are allocated for every staged file, so device memory grows with
+# the number of files staged at once (about 31 GB for 3,552 such frames); stage fewer samples per run_jpeg_decode to bound it.
+JPEG_DECODE_WORKSPACE_PER_CALL = 2 << 30
+
+
+def jpeg_decode_layout(staged):
+    """Frame shapes, coefficient offsets (elements) and frame offsets (bytes, one more than the files) of run_jpeg_decode's arenas for
+    the files of an io.StagedCameras."""
+    n = len(staged)
+    descs = [staged.plans[k].desc for k in range(n)]
+    shapes = [(d.height, d.width, 3) if d.n_comp == 3 else (d.height, d.width) for d in descs]
+    coef_off = np.zeros(n, np.int64)
+    out_off = np.zeros(n + 1, np.int64)
+    c = 0
+    for k, d in enumerate(descs):
+        coef_off[k] = c
+        c += int(d.coef_elems)
+        out_off[k + 1] = out_off[k] + int(np.prod(shapes[k]))
+    return shapes, coef_off, out_off
+
+
+@dataclass
+class JpegDecodeResult:
+    """Frames and coefficients of msc_jpeg_decode_batch for the files of an io.StagedCameras, still on the device: file k (staged.index[k])
+    is out[out_off[k]:] with shape shapes[k], its coefficients coef[coef_off[k]:] and its status status[k]."""
+    shapes: List[tuple]
+    coef: torch.Tensor      # i16, every file's coefficients
+    coef_off: np.ndarray    # i64 [n]
+    out: torch.Tensor       # u8, every file's frame
+    out_off: np.ndarray     # i64 [n + 1]
+    status: torch.Tensor    # i32 [n]
+    files: torch.Tensor     # u8, the device copy of the staged bytes
+    workspace: torch.Tensor
+    staged: object = None   # the io.StagedCameras of the last run (its host buffer must outlive the upload)
+
+    def frames(self) -> List[torch.Tensor]:
+        """Device views of the frames, (H, W, 3) or (H, W); nothing is synchronised."""
+        return [self.out[int(self.out_off[k]):int(self.out_off[k + 1])].view(shape) for k, shape in enumerate(self.shapes)]
+
+    def check(self) -> None:
+        """Synchronise on the status words; raise MscError naming the first file that failed and its status."""
+        st = self.status.cpu().numpy()
+        bad = np.flatnonzero(st)
+        if len(bad):
+            k = int(bad[0])
+            where = self.staged.index[k] if self.staged is not None else k
+            raise _capi.MscError("msc_jpeg_decode_batch: file %d (sample, camera %s) failed with status %d" % (k, where, int(st[k])), int(st[k]))
+
+    def to_host(self) -> List[np.ndarray]:
+        """The frames as host arrays.  This is the synchronisation point: one copy of the status words, then one of the frames."""
+        self.check()
+        host = self.out.cpu().numpy()
+        return [host[int(self.out_off[k]):int(self.out_off[k + 1])].reshape(shape) for k, shape in enumerate(self.shapes)]
+
+
 def _keyframe_row_counts(hb: HostBatch) -> np.ndarray:
     """Keyframe rows (sweep sample_sweep_off[s]) of every sample that has sweeps."""
     sso = hb.sample_sweep_off
@@ -748,6 +804,76 @@ class GeometryEngine:
                                                    C.c_void_p(stream)), "msc_jpeg_encode_batch")
         if n > 0:
             self.kernel_launches += 6
+        return out
+
+    # ------------------------------------------------------------------ camera files -> frames (NuScenesLoader._load_camera)
+    def _jpeg_decode_chunks(self, staged) -> List[tuple]:
+        """(first, count, workspace bytes) of every msc_jpeg_decode_batch call: consecutive files whose one-file workspaces sum to at most
+        JPEG_DECODE_WORKSPACE_PER_CALL (an upper bound of the call's need: the per-call records are shared)."""
+        base, size = C.addressof(staged.plans), C.sizeof(_capi.MscJpegPlan)
+        n = len(staged)
+        one = getattr(staged, "_ws_one", None)
+        if one is None:
+            one = staged._ws_one = [int(self.lib.msc_jpeg_decode_batch_workspace_bytes(1, base + k * size)) for k in range(n)]
+        if 0 in one:
+            raise _capi.MscError("run_jpeg_decode: file %d has no valid plan" % one.index(0), _capi.MSC_ERR_BAD_ARGUMENT)
+        chunks, a = [], 0
+        while a < n:
+            k, acc = 1, one[a]
+            while a + k < n and acc + one[a + k] <= JPEG_DECODE_WORKSPACE_PER_CALL:
+                acc += one[a + k]
+                k += 1
+            chunks.append((a, k, int(self.lib.msc_jpeg_decode_batch_workspace_bytes(k, base + a * size))))
+            a += k
+        return chunks
+
+    def alloc_jpeg_decode(self, staged) -> JpegDecodeResult:
+        """Buffers of run_jpeg_decode for the files of an io.StagedCameras: coefficient and frame arenas, status words, the device copy
+        of the staged bytes and the workspace of the largest call."""
+        n = len(staged)
+        shapes, coef_off, out_off = jpeg_decode_layout(staged)
+        c = int(sum(int(staged.plans[k].desc.coef_elems) for k in range(n)))
+        ws = max([need for _, _, need in self._jpeg_decode_chunks(staged)], default=256)
+        dv = self.device
+        return JpegDecodeResult(shapes, torch.empty(max(c, 8), dtype=torch.int16, device=dv), coef_off,
+                                torch.empty(max(int(out_off[-1]), 1), dtype=torch.uint8, device=dv), out_off,
+                                torch.zeros(max(n, 1), dtype=torch.int32, device=dv), torch.empty(max(staged.nbytes, 1), dtype=torch.uint8, device=dv),
+                                torch.empty(ws, dtype=torch.uint8, device=dv))
+
+    def run_jpeg_decode(self, staged, out: Optional[JpegDecodeResult] = None) -> JpegDecodeResult:
+        """Decode the files of an io.StagedCameras on the device, bit-identical to np.array(Image.open(path)): one copy of the used part
+        of the staged buffer, then one msc_jpeg_decode_batch call per JPEG_DECODE_WORKSPACE_PER_CALL bytes of workspace (unstuffing,
+        Huffman decode, DC prediction, IDCT, upsampling and colour conversion all run there).  Nothing is synchronised; out.to_host() or
+        out.check() reads the status words.  A given `out` must have been allocated for files of the same geometry (alloc_jpeg_decode on
+        the same plans); any other raises MscError before anything is copied or launched."""
+        if out is None:
+            out = self.alloc_jpeg_decode(staged)
+        n = len(staged)
+        # the regions of `out` must be the ones these plans need: a buffer allocated for other files would be written out of bounds
+        shapes, coef_off, out_off = jpeg_decode_layout(staged)
+        coef_end = int(coef_off[-1]) + int(staged.plans[n - 1].desc.coef_elems) if n else 0
+        if (list(out.shapes) != shapes or out.coef.dtype != torch.int16 or out.out.dtype != torch.uint8 or out.status.dtype != torch.int32
+                or not np.array_equal(out.coef_off, coef_off) or not np.array_equal(out.out_off, out_off)
+                or out.coef.numel() < coef_end or out.out.numel() < int(out_off[-1]) or out.status.numel() < n
+                or out.files.numel() < staged.nbytes):
+            raise _capi.MscError("run_jpeg_decode: the output buffers do not match the staged files", _capi.MSC_ERR_BAD_ARGUMENT)
+        out.staged = staged
+        if n == 0:
+            return out
+        chunks = self._jpeg_decode_chunks(staged)
+        if max(need for _, _, need in chunks) > out.workspace.numel():
+            raise _capi.MscError("run_jpeg_decode: the workspace is too small for these files", _capi.MSC_ERR_BAD_ARGUMENT)
+        src = torch.from_numpy(staged.data[:staged.nbytes]) if staged._holder is None else staged._holder.view(torch.uint8).reshape(-1)[:staged.nbytes]
+        out.files[:staged.nbytes].copy_(src, non_blocking=True)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        base, size = C.addressof(staged.plans), C.sizeof(_capi.MscJpegPlan)
+        file_off = np.ascontiguousarray(staged.file_off, np.int64)
+        for a, k, _ in chunks:
+            _capi.check(self.lib.msc_jpeg_decode_batch(k, base + a * size, out.files.data_ptr(), file_off[a:a + k].ctypes.data, out.coef.data_ptr(),
+                                                       out.coef_off[a:a + k].ctypes.data, out.out.data_ptr(), out.out_off[a:a + k].ctypes.data,
+                                                       out.status[a].data_ptr(), out.workspace.data_ptr(), out.workspace.numel(), stream),
+                        "msc_jpeg_decode_batch")
+            self.kernel_launches += 4
         return out
 
     # ------------------------------------------------------------------ batched pairwise relation tables ([EXT] e6)

@@ -111,6 +111,77 @@ def stage_batch(samples: Sequence[dict], n_cams: int = N_CAMS_DEFAULT, threads: 
     return hb
 
 
+class StagedCameras:
+    """The camera files of a batch in one host byte buffer (see stage_camera_files).  File k is data[file_off[k]:file_off[k] + size[k]],
+    plans[k] its msc_jpeg_plan and index[k] its (sample, camera) position; `unsupported` lists the (sample, camera, path) the planner
+    refused as MSC_ERR_UNSUPPORTED (progressive, 12-bit, CMYK ...), which are not in the buffer."""
+
+    def __init__(self, data, holder, file_off, size, plans, index, unsupported, n_cams):
+        self.data, self._holder, self.file_off, self.size = data, holder, file_off, size
+        self.plans, self.index, self.unsupported, self.n_cams = plans, index, unsupported, n_cams
+        self.nbytes = int(file_off[-1] + size[-1]) if len(size) else 0
+
+    def __len__(self):
+        return len(self.index)
+
+
+def stage_camera_files(samples: Sequence[dict], threads: int = 8, pool: Optional["PinnedPool"] = None, pinned: Optional[bool] = None) -> StagedCameras:
+    """Read every camera file of a batch (the `path` of each entry of a sample's `cameras`, as NuScenesLoader(lazy_sweeps=True) records
+    it) with `readinto` into one byte buffer -- pinned when CUDA is available unless `pinned=False`, taken from `pool` when one is given --
+    and plan each file's decode (msc_jpeg_decode_plan).  Files start at 256-byte offsets.  A file the planner refuses as
+    MSC_ERR_UNSUPPORTED is listed in `unsupported`; any other planner error raises MscError."""
+    import ctypes as C
+    from . import _capi
+    lib = _capi.load()
+    files = [(i, c, cam["path"]) for i, s in enumerate(samples) for c, cam in enumerate(s.get("cameras", []))]
+    sizes = np.array([os.path.getsize(p) for _, _, p in files], np.int64)
+    offs = np.zeros(len(files), np.int64)
+    cursor = 0
+    for k, n in enumerate(sizes):
+        offs[k] = cursor
+        cursor += (int(n) + 255) & ~255
+    total = max(cursor, 256)
+    if pinned is None:
+        try:
+            import torch
+            pinned = torch.cuda.is_available()
+        except Exception:
+            pinned = False
+    if pool is not None:
+        holder = pool.take((total + 19) // 20)
+        data = holder.numpy().view(np.uint8).reshape(-1)[:total]
+    elif pinned:
+        import torch
+        holder = torch.empty(total, dtype=torch.uint8).pin_memory()
+        data = holder.numpy()
+    else:
+        holder = None
+        data = np.empty(total, np.uint8)
+    plans = (_capi.MscJpegPlan * max(len(files), 1))()
+    rcs = [0] * len(files)
+
+    def load(k):
+        dst = data[int(offs[k]): int(offs[k]) + int(sizes[k])]
+        read_pcd_bin_into(files[k][2], dst)
+        rcs[k] = lib.msc_jpeg_decode_plan(dst.ctypes.data, int(sizes[k]), C.byref(plans[k]))
+
+    with ThreadPoolExecutor(max(1, threads)) as ex:
+        list(ex.map(load, range(len(files))))
+    keep, unsupported = [], []
+    for k, rc in enumerate(rcs):
+        if rc == _capi.MSC_ERR_UNSUPPORTED:
+            unsupported.append(files[k])
+        elif rc != 0:
+            raise _capi.MscError(f"{files[k][2]}: msc_jpeg_decode_plan failed with status {rc}", rc)
+        else:
+            keep.append(k)
+    kept_plans = (_capi.MscJpegPlan * max(len(keep), 1))()
+    for j, k in enumerate(keep):
+        kept_plans[j] = plans[k]
+    return StagedCameras(data, holder, offs[keep], sizes[keep], kept_plans, [files[k][:2] for k in keep], unsupported,
+                         [len(s.get("cameras", [])) for s in samples])
+
+
 def write_pcd_bin(path: str, rows: np.ndarray) -> None:
     """Write (n,5) float32 rows in the nuScenes .pcd.bin layout (used by tests and synthetic datasets)."""
     np.ascontiguousarray(rows, np.float32).tofile(path)

@@ -85,7 +85,8 @@ class NuScenesLoader:
 
     def __init__(self, dataroot: str, version: str = "v1.0-mini", n_sweeps: int = 10, lazy_sweeps: bool = False, engine=None):
         """lazy_sweeps: sweeps carry the .pcd.bin `path` instead of `points_raw` (and `point_cloud` / `images` are left out), so
-        msc_geom.io.stage_batch reads the files straight into one pinned batch buffer -- the on-disk step of the batched path.
+        msc_geom.io.stage_batch reads the files straight into one pinned batch buffer -- the on-disk step of the batched path; each
+        entry of `cameras` then carries its JPEG's `path` for msc_geom.io.stage_camera_files / msc_geom.ops.camera_frames.
         engine: a GeometryEngine; the six camera frames of a sample are then decoded by msc_geom.ops.decode_jpeg_batch (host Huffman
         decode in parallel, IDCT / upsampling / colour conversion on the device) -- the same bytes as the reference's
         np.array(Image.open(...)) (nuscenes_loader.py:136-144); files the decoder refuses (progressive, CMYK, PNG ...) go through PIL."""
@@ -116,6 +117,8 @@ class NuScenesLoader:
                 cs = nusc.get("calibrated_sensor", sd["calibrated_sensor_token"])
                 cameras.append({"channel": ch, "ego_pose": self._pose7(nusc.get("ego_pose", sd["ego_pose_token"])), "calib": self._pose7(cs),
                                 "intrinsic": np.asarray(cs["camera_intrinsic"], np.float64)})
+                if self.lazy_sweeps:  # the frame itself is read by msc_geom.io.stage_camera_files
+                    cameras[-1]["path"] = str(self.dataroot / sd["filename"])
         if image_paths:
             images = self._load_cameras(image_paths)
         ref_sd = nusc.get("sample_data", sample["data"]["LIDAR_TOP"])

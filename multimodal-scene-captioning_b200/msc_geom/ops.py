@@ -400,3 +400,25 @@ def encode_jpeg_batch(eng: GeometryEngine, images, quality: int = 85) -> List[by
             for k, f in zip(idx, files):
                 out[k] = f
     return out
+
+
+def camera_frames(eng: GeometryEngine, samples, to_host: bool = False, threads: int = 8, pool=None):
+    """Per sample, its camera frames in the order of its `cameras` entries (each with the JPEG's `path`, as NuScenesLoader(lazy_sweeps=True)
+    records it) -- the same arrays as np.array(Image.open(path)).  The files are staged in one buffer (io.stage_camera_files) and decoded
+    on the device in one call per GeometryEngine.run_jpeg_decode chunk, so a frame crosses PCIe only as compressed bytes.  Files the
+    decoder declares unsupported (progressive, 12-bit, CMYK ...) go through PIL, like NuScenesLoader._load_cameras, and are uploaded.
+    Returns device tensors, (H, W, 3) or (H, W), or host arrays with to_host=True.  A corrupt file raises MscError."""
+    from PIL import Image
+    from . import io as mio
+    staged = mio.stage_camera_files(samples, threads=threads, pool=pool)
+    res = eng.run_jpeg_decode(staged)
+    frames = res.to_host() if to_host else res.frames()
+    if not to_host:
+        res.check()
+    out = [[None] * n for n in staged.n_cams]
+    for (i, c), f in zip(staged.index, frames):
+        out[i][c] = f
+    for i, c, path in staged.unsupported:
+        a = np.array(Image.open(path))
+        out[i][c] = a if to_host else torch.from_numpy(a).to(eng.device)
+    return out
