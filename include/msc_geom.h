@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define MSC_ABI_VERSION 2
+#define MSC_ABI_VERSION 3
 #define MSC_MAX_CAMS 8
 #define MSC_MAX_BOXES_FUSED 255 /* per sample, fused kernel (cull cells hold u8 box ids; 0xff = empty) */
 #define MSC_STATS_STRIDE 16
@@ -473,6 +473,47 @@ size_t msc_cluster_views_batch_workspace_bytes(int32_t n_views, int32_t max_view
 int msc_cluster_views_batch(const float* rows, const int32_t* labels, const int32_t* views, int32_t n_views, int32_t max_view_points,
                             const uint32_t* stamp, int32_t stamp_len, uint8_t* out_bgr, uint32_t* status, void* workspace,
                             size_t workspace_bytes, void* stream);
+
+/*
+ * PNG files of n 8-bit images (h x w x c; c = 3: RGB, colour type 2; c = 1: grey, colour type 0) in one stream-ordered call.  Each file
+ * is the signature, IHDR (width, height, depth 8, colour type, 0, 0, 0: Pillow's), one IDAT and IEND, every CRC-32 correct.  The IDAT
+ * data is one zlib stream (header 78 9C, Adler-32) that inflates to exactly the payload of Pillow's Image.fromarray(img).save(buf, "PNG"):
+ * per row (the row above row 0 is zeros) a filter byte and the filtered row, the filter chosen as ZipEncode.c does -- None, Up, Sub,
+ * Paeth tried in that order, cost sum(v < 128 ? v : 256 - v) over the filtered bytes, a candidate taken only when strictly cheaper,
+ * Average never.  The deflate data is one dynamic-Huffman block or stored blocks of up to 65,535 bytes, whichever is smaller, so a file
+ * is never larger than 57 + 6 + raw + 5 ceil(raw / 65535) bytes (raw = h (1 + w c)).  swap_rb reads BGR pixels as RGB.  A file depends
+ * only on its image: not on the other images of the call, nor on the launch shape.
+ * Images may differ in shape; rows are row_pitch bytes apart on the device.  The descriptors are copied into the workspace.  The files
+ * are back to back in `out`: file i is out[out_off[i] .. out_off[i + 1]) (out_off: device i64 [n + 1]).  *status (device i32) is 1 when
+ * they need more than out_bytes; then nothing is written to `out`, but out_off is exact.  No host synchronisation, no allocation:
+ * workspace >= msc_png_encode_workspace_bytes(n, images) (the filtered streams, their tokens and their worst-case deflate data; it does
+ * not depend on out_bytes), 256-byte aligned.  Channels other than 1 or 3, swap_rb with one channel, h or w outside 1..65535, raw >= 2^31
+ * or a stored zlib stream beyond the 2^31 - 1 bytes of one PNG chunk, a pitch below w c, NULL pointers or a short workspace:
+ * MSC_ERR_BAD_ARGUMENT before anything is launched (the workspace size is then 0).  n = 0 is a successful no-op.
+ */
+typedef struct {
+    const uint8_t* pixels;
+    int64_t row_pitch;
+    int32_t height, width, channels, swap_rb;
+} msc_png_image;
+size_t msc_png_encode_workspace_bytes(int32_t n, const msc_png_image* images_host);
+int msc_png_encode_batch(int32_t n, const msc_png_image* images_host, uint8_t* out, size_t out_bytes, int64_t* out_off, int32_t* status,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * The classifier mosaics of LiDARAgent._classify_batch_with_llm (lidar_agent.cluster_mosaic) for n groups of 512 x 512 BGR cluster views
+ * already on the device, in one stream-ordered call.  groups: HOST i32 [n, 2] = (first, count), count in 1..10, first + count <= n_views;
+ * mosaic j is cluster_mosaic(views[first_j .. first_j + count_j)): the view itself for a count of 1, else a sheet of min(3, count)
+ * columns and ceil(count / 3) rows of views with the '#idx' labels and white empty cells.  The labels and the white come from
+ * stamps u32 [*, 2] (pixel y * W + x, B | G << 8 | R << 16) of lidar_agent.mosaic_stamp, written over the copied views: the stamp of a
+ * count k >= 2 is stamps[stamp_off[k] .. stamp_off[k + 1]) (stamp_off: HOST i32 [12]).  The mosaics are back to back in out_bgr, each
+ * (512 rows) x (512 cols) x 3.  No host synchronisation, no allocation: workspace >= msc_cluster_mosaics_workspace_bytes(n),
+ * 256-byte aligned; views and out_bgr 16-byte aligned.  A group out of range, NULL buffers, a misaligned buffer or a short workspace:
+ * MSC_ERR_BAD_ARGUMENT.  n = 0 is a successful no-op.
+ */
+size_t msc_cluster_mosaics_workspace_bytes(int32_t n);
+int msc_cluster_mosaics(const uint8_t* views, int32_t n_views, const int32_t* groups, int32_t n, const uint32_t* stamps, const int32_t* stamp_off,
+                        uint8_t* out_bgr, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

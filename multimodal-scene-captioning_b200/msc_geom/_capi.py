@@ -9,7 +9,7 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file_
 MSC_MAX_CAMS = 8
 MSC_MAX_BOXES_FUSED = 255
 MSC_STATS_STRIDE = 16
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class MscError(RuntimeError):
@@ -87,6 +87,11 @@ class MscJpegPlan(C.Structure):
                 ("ta", C.c_int32 * 3), ("reserved_", C.c_int32), ("dc", MscJpegHuff * 4), ("ac", MscJpegHuff * 4)]
 
 
+class MscPngImage(C.Structure):
+    _fields_ = [("pixels", C.c_void_p), ("row_pitch", C.c_int64), ("height", C.c_int32), ("width", C.c_int32), ("channels", C.c_int32),
+                ("swap_rb", C.c_int32)]
+
+
 _lib = None
 
 _PROTOS = {
@@ -146,6 +151,11 @@ _PROTOS = {
     "msc_cluster_views_batch_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "msc_cluster_views_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_size_t, C.c_void_p]),
+    "msc_png_encode_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_void_p]),
+    "msc_png_encode_batch": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "msc_cluster_mosaics_workspace_bytes": (C.c_size_t, [C.c_int32]),
+    "msc_cluster_mosaics": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                      C.c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_PROTOS)

@@ -261,10 +261,14 @@ class LidarBevResult:
     def to_host(self, layers: Sequence[str] = ("semantic", "height", "density")) -> List[Dict[str, np.ndarray]]:
         """Per sample, the layers asked for (finish_bev_layers' dict); only those are copied.  This is the synchronisation point; a set
         status word (a cell count beyond the density table) raises MscError."""
-        if int(self.status.cpu()[0]):
-            raise _capi.MscError("msc_keyframe_bev_batch: a cell count has no entry in the density table", 1)
+        self.check()
         host = {k: getattr(self, k).cpu().numpy() for k in layers}
         return [{k: host[k][i] for k in layers} for i in range(self.n_samples)]
+
+    def check(self) -> None:
+        """Reads the status word (a synchronisation point): a cell count beyond the density table raises MscError."""
+        if int(self.status.cpu()[0]):
+            raise _capi.MscError("msc_keyframe_bev_batch: a cell count has no entry in the density table", 1)
 
 
 @dataclass
@@ -276,9 +280,56 @@ class ClusterViewsResult:
 
     def to_host(self) -> np.ndarray:
         """u8 [n, 512, 512, 3].  This is the synchronisation point; a view above the maximum view size raises MscError."""
+        self.check()
+        return self.images.cpu().numpy()
+
+    def check(self) -> None:
+        """Reads the status word (a synchronisation point): a view above the maximum view size raises MscError."""
         if int(self.status.cpu()[0]):
             raise _capi.MscError("msc_cluster_views_batch: a view holds more points than max_view_points", 1)
-        return self.images.cpu().numpy()
+
+
+@dataclass
+class MosaicsResult:
+    """Classifier mosaics of msc_cluster_mosaics, still on the device: mosaic j is images[j], a view into one arena."""
+    groups: np.ndarray          # i32 [n, 2]: (first view, count)
+    images: List[torch.Tensor]  # u8 (512 rows, 512 cols, 3) each
+    arena: torch.Tensor
+
+
+def mosaic_shape(count: int) -> tuple:
+    """(H, W, 3) of lidar_agent.cluster_mosaic over `count` 512 x 512 views: min(3, count) columns, ceil(count / 3) rows."""
+    return (512 * ((count + 2) // 3), 512 * min(3, count), 3)
+
+
+PNG_FRAMING_BYTES = 63  # signature, IHDR, IDAT framing, IEND (57) and the zlib header and Adler-32 (6) of every msc_png_encode_batch file
+
+
+@dataclass
+class PngBatchResult:
+    """Files of msc_png_encode_batch, still on the device: image i is arena[out_off[i] : out_off[i + 1]].  `small` holds the status
+    word and out_off in one buffer, so reading them is one copy."""
+    n_images: int
+    shapes: List[tuple]       # (H, W, C) per image
+    small: torch.Tensor       # i64 [n + 2]: status (low 32 bits of word 0), out_off [n + 1]
+    arena: torch.Tensor       # u8 [out_bytes]
+    workspace: torch.Tensor   # u8, msc_png_encode_workspace_bytes
+    needed: Optional[int] = None  # arena bytes the last call needed, known after to_host()
+
+    @property
+    def out_off(self) -> torch.Tensor:
+        return self.small[1:]
+
+    def to_host(self) -> List[bytes]:
+        """The files as bytes.  This is the synchronisation point: one copy of status and offsets, then one copy of the used prefix of
+        the arena.  A set status word (the files need more than the arena) raises MscError with status 1 and the size they need."""
+        small = self.small.cpu().numpy()
+        off = small[1:].astype(np.int64)
+        self.needed = int(off[-1])
+        if int(small[0]) & 0xffffffff:
+            raise _capi.MscError("msc_png_encode_batch: the files need %d bytes, the arena holds %d" % (self.needed, self.arena.numel()), 1)
+        data = self.arena[:self.needed].cpu().numpy().tobytes()
+        return [data[off[i]:off[i + 1]] for i in range(self.n_images)]
 
 
 BEV_WORKSPACE_PER_CALL = 2 << 30            # workspace bytes of one msc_keyframe_bev_batch call (8 res^2 bytes per sample)
@@ -771,6 +822,95 @@ class GeometryEngine:
             _capi.check(self.lib.msc_cluster_views_batch(rows.data_ptr(), labels.data_ptr(), v32[a:a + k].ctypes.data, k, int(max_view_points),
                                                          stamp.data_ptr(), stamp.shape[0], out.images[a].data_ptr(), out.status.data_ptr(),
                                                          ws.data_ptr(), need, stream), "msc_cluster_views_batch")
+            self.kernel_launches += 6
+        return out
+
+    def run_cluster_mosaics(self, views: ClusterViewsResult, groups) -> MosaicsResult:
+        """The classifier mosaics lidar_agent.cluster_mosaic makes of views[first : first + count] for every (first, count) of `groups`
+        (count 1..10), drawn from a run_cluster_views result on the device in one stream-ordered call (msc_cluster_mosaics): the views
+        are copied into their cells, then each count's lidar_agent.mosaic_stamp ('#idx' labels, white empty cells) is written over them.
+        Nothing is synchronised."""
+        g = np.ascontiguousarray(np.asarray(groups, dtype=np.int64).reshape(-1, 2)).astype(np.int32)
+        n = g.shape[0]
+        if n and (g[:, 1].min() < 1 or g[:, 1].max() > 10 or g[:, 0].min() < 0 or (g[:, 0] + g[:, 1]).max() > views.n_views):
+            raise _capi.MscError("run_cluster_mosaics: a group is outside 1..10 of the %d views" % views.n_views, _capi.MSC_ERR_BAD_ARGUMENT)
+        shapes = [mosaic_shape(int(c)) for c in g[:, 1]]
+        sizes = [int(np.prod(sh)) for sh in shapes]
+        arena = torch.empty(max(sum(sizes), 16), dtype=torch.uint8, device=self.device)
+        images, o = [], 0
+        for sh, b in zip(shapes, sizes):
+            images.append(arena[o:o + b].view(sh))
+            o += b
+        if n == 0:
+            return MosaicsResult(g, images, arena)
+        if "mosaic" not in self._stamps:
+            from .lidar_agent import mosaic_stamp
+            st = [mosaic_stamp(k) if k >= 2 else np.zeros((0, 2), np.uint32) for k in range(11)]
+            self._mosaic_off = np.concatenate([[0, 0], np.cumsum([len(a) for a in st[1:]])]).astype(np.int32)
+        stamps = self._stamp("mosaic", lambda: np.concatenate(st))
+        need = int(self.lib.msc_cluster_mosaics_workspace_bytes(n))
+        ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        _capi.check(self.lib.msc_cluster_mosaics(views.images.data_ptr(), views.n_views, g.ctypes.data, n, stamps.data_ptr(),
+                                                 self._mosaic_off.ctypes.data, arena.data_ptr(), ws.data_ptr(), need, stream), "msc_cluster_mosaics")
+        self.kernel_launches += 2
+        return MosaicsResult(g, images, arena)
+
+    # ------------------------------------------------------------------ images -> PNG files (serialize.image_to_base64)
+    def _png_descs(self, images, swap_rb):
+        """msc_png_image descriptors of CUDA u8 images (H, W, 3) or (H, W) whose pixels are contiguous within a row (rows may be
+        strided); swap_rb: one flag for all, or one per image."""
+        n = len(images)
+        swaps = [bool(swap_rb)] * n if isinstance(swap_rb, (bool, int, np.bool_)) else [bool(v) for v in swap_rb]
+        if len(swaps) != n:
+            raise _capi.MscError("run_png_encode: %d swap_rb flags for %d images" % (len(swaps), n), _capi.MSC_ERR_BAD_ARGUMENT)
+        descs = (_capi.MscPngImage * max(n, 1))()
+        shapes = []
+        for i, im in enumerate(images):
+            ok = isinstance(im, torch.Tensor) and im.is_cuda and im.dtype == torch.uint8 and im.device == self.device and im.dim() in (2, 3)
+            if ok:
+                c = 1 if im.dim() == 2 else int(im.shape[2])
+                ok = c in (1, 3) and im.shape[0] > 0 and im.shape[1] > 0 and (im.dim() == 2 or im.stride(2) == 1) and im.stride(1) == c
+            if not ok:
+                raise _capi.MscError("run_png_encode: image %d must be a uint8 CUDA tensor (H, W, 3) or (H, W) on %s with contiguous rows"
+                                     % (i, self.device), _capi.MSC_ERR_BAD_ARGUMENT)
+            h, w = int(im.shape[0]), int(im.shape[1])
+            descs[i] = _capi.MscPngImage(im.data_ptr(), im.stride(0) if h > 1 else w * c, h, w, c, int(swaps[i]))
+            shapes.append((h, w, c))
+        return descs, shapes
+
+    def alloc_png(self, images, swap_rb=False, out_bytes: Optional[int] = None) -> PngBatchResult:
+        """Buffers of run_png_encode for these images: the file arena (default: a quarter of the raw payload plus the framing of every
+        file), offsets and status, and the workspace."""
+        descs, shapes = self._png_descs(images, swap_rb)
+        n = len(shapes)
+        if out_bytes is None:
+            out_bytes = sum(h * (1 + w * c) // 4 + PNG_FRAMING_BYTES for h, w, c in shapes)
+        need = int(self.lib.msc_png_encode_workspace_bytes(n, descs))
+        if need == 0 and n:
+            raise _capi.MscError("alloc_png: these images cannot be encoded in one call", _capi.MSC_ERR_BAD_ARGUMENT)
+        d = self.device
+        return PngBatchResult(n, shapes, torch.zeros(n + 2, dtype=torch.int64, device=d), torch.empty(max(out_bytes, 1), dtype=torch.uint8, device=d),
+                              torch.empty(max(need, 256), dtype=torch.uint8, device=d))
+
+    def run_png_encode(self, images, swap_rb=False, out: Optional[PngBatchResult] = None) -> PngBatchResult:
+        """PNG files of device images (a sequence of uint8 CUDA tensors (H, W, 3) RGB or (H, W) grey, shapes free, rows may be strided)
+        in one stream-ordered call (msc_png_encode_batch): Pillow's IHDR, and an IDAT that inflates to the payload of Pillow's
+        Image.fromarray(img).save(buf, "PNG").  swap_rb reads BGR images as RGB.  With `out` given nothing is allocated for the files;
+        out.to_host() reads them."""
+        if isinstance(images, torch.Tensor):
+            images = list(images) if images.dim() == 4 else [images]
+        descs, shapes = self._png_descs(images, swap_rb)
+        n = len(shapes)
+        if out is None:
+            out = self.alloc_png(images, swap_rb)
+        need = int(self.lib.msc_png_encode_workspace_bytes(n, descs))
+        if out.shapes != shapes or out.workspace.numel() < need:
+            raise _capi.MscError("run_png_encode: the output buffers do not match the images", _capi.MSC_ERR_BAD_ARGUMENT)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _capi.check(self.lib.msc_png_encode_batch(n, descs, out.arena.data_ptr(), out.arena.numel(), out.out_off.data_ptr(), out.small.data_ptr(),
+                                                  out.workspace.data_ptr(), out.workspace.numel(), C.c_void_p(stream)), "msc_png_encode_batch")
+        if n > 0:
             self.kernel_launches += 6
         return out
 

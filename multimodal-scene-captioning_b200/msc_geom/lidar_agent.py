@@ -15,6 +15,7 @@ What stays on the host, and why:
 """
 from __future__ import annotations
 
+import base64
 import json
 from dataclasses import dataclass
 from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
@@ -140,6 +141,16 @@ def cluster_mosaic(images: List[np.ndarray]) -> np.ndarray:
     return sheet
 
 
+def mosaic_stamp(count: int) -> np.ndarray:
+    """The '#idx' labels and the white empty cells cluster_mosaic draws on a mosaic of `count` (2..10) views, as an overlay_stamp: what
+    cluster_mosaic of the canvas's own 512 x 512 cells changes.  Written over the views copied into their cells, it gives the mosaic."""
+    rows, cols = (count + 2) // 3, min(3, count)
+
+    def draw(canvas):
+        return cluster_mosaic([canvas[r * 512:(r + 1) * 512, c * 512:(c + 1) * 512] for r, c in (divmod(i, cols) for i in range(count))])
+    return overlay_stamp(draw, rows * 512, cols * 512)
+
+
 def set_order(cluster_first, noise_first: int) -> List[int]:
     """The cluster labels (noise excluded) in the order `s = set(labels); s.discard(-1)` iterates them (lidar_agent.py:154-159), from
     each label's first row alone: cluster_first[k] is the smallest index of a row labelled k (a sequence over k = 0..K-1, or a dict
@@ -255,12 +266,15 @@ class LiDARAgent:
         images = self._cluster_visualizations(object_points, labels, order)
         return self._classified_objects(meta, lambda a, b: images[a:b])
 
-    def _classified_objects(self, meta: List[dict], images_of: Callable[[int, int], List[np.ndarray]]) -> List[DetectedObject]:
-        """The classifier loop of lidar_agent.py:189-239; images_of(a, b) gives the images of clusters a..b-1 of `meta`."""
+    def _classified_objects(self, meta: List[dict], images_of: Callable[[int, int], Any],
+                            classify: Optional[Callable[[Any, List[dict]], List[dict]]] = None) -> List[DetectedObject]:
+        """The classifier loop of lidar_agent.py:189-239; images_of(a, b) gives the images of clusters a..b-1 of `meta`, which
+        classify(images, metadata) (default: _classify_batch_with_llm) classifies."""
+        classify = classify or self._classify_batch_with_llm
         out: List[DetectedObject] = []
         for start in range(0, len(meta), 10):  # the reference classifies in batches of 10 (:189)
             batch = meta[start:start + 10]
-            cls = self._classify_batch_with_llm(images_of(start, start + len(batch)), batch)
+            cls = classify(images_of(start, start + len(batch)), batch)
             for m, c in zip(batch, cls):
                 if c["category"] != "unknown" and c["confidence"] > 0.3:
                     out.append(DetectedObject(c["category"], m["center"], m["dimensions"], m["num_points"], m["distance"], m["direction"],
@@ -336,7 +350,7 @@ class LiDARAgent:
 
     def process_batch(self, samples: Optional[Sequence[dict]] = None, device_batch: Optional[DeviceBatch] = None,
                       contexts: Optional[Sequence[Optional[Dict]]] = None, match_annotations: bool = False,
-                      annotations: Optional[Sequence[Sequence[dict]]] = None) -> List[Dict[str, Any]]:
+                      annotations: Optional[Sequence[Sequence[dict]]] = None, png: bool = False) -> List[Dict[str, Any]]:
         """[process(sample["point_cloud"], context) for each sample], with the filter, the ground split, DBSCAN and the cluster boxes of
         every sample's keyframe (sweep 0) in one device pass (GeometryEngine.run_lidar).  `device_batch` (e.g. engine.upload of
         io.stage_batch over lazy-loader samples, whose point_cloud is None) is used as it is; otherwise `samples` are packed and uploaded.
@@ -345,7 +359,10 @@ class LiDARAgent:
         cluster images only when a classifier is (GeometryEngine.run_cluster_views, CLUSTER_IMAGES_PER_CALL clusters at a time).
         match_annotations=True adds to each result the key "annotation_match" (lidar_agent.annotation_match): which annotated box each
         cluster of the classifier's order lies in and which clusters each box holds (GeometryEngine.run_cluster_match, enqueued behind
-        run_lidar).  Categories come from the samples' annotation dicts, or from `annotations` (one list per sample) for a device_batch."""
+        run_lidar).  Categories come from the samples' annotation dicts, or from `annotations` (one list per sample) for a device_batch.
+        png=True hands each callable what goes on the wire, encoded on the device (ops.encode_png_batch) so that only PNG bytes cross PCIe:
+        the llm gets bev_png=<base64 of the BEV's PNG> instead of bev_semantic=<array>, and the classifier is called
+        cluster_classifier(None, <base64 of the mosaic's PNG>, metadata) (GeometryEngine.run_cluster_mosaics on whole groups of ten)."""
         eng = self.engine
         if device_batch is None:
             if samples is None:
@@ -358,20 +375,30 @@ class LiDARAgent:
         matches = match.to_host() if match is not None else None
         if annotations is None and samples is not None:
             annotations = [s.get("annotations", []) for s in samples]
-        bevs = bev.to_host(("semantic",)) if bev is not None else [None] * len(per)
+        if bev is None:
+            bevs = [None] * len(per)
+        elif png:
+            bev.check()
+            bevs = [{"png": base64.b64encode(f).decode("ascii")} for f in ops.encode_png_batch(eng, list(bev.semantic), swap_rb=True)]
+        else:
+            bevs = bev.to_host(("semantic",))
         orders = []
         for r in per:
             table = r["clusters"]
             orders.append([l for l in set_order(r["cluster_first"], r["noise_first"]) if int(table[l, 10]) >= 5]
                           if len(r["object"]) >= self.dbscan_min_samples else [])  # the guard of _detect_objects_3d
-        images = self._batch_cluster_images(res, per, orders) if self.cluster_classifier is not None else None
+        images = None
+        if self.cluster_classifier is not None:
+            images = self._batch_cluster_mosaics(res, per, orders) if png else self._batch_cluster_images(res, per, orders)
+        # without a classifier every path takes _classify_batch_with_llm's default
+        classify = (lambda mosaic, meta: self.cluster_classifier(None, mosaic, meta)) if png and images is not None else None
         contexts = list(contexts) if contexts is not None else [None] * len(per)
         out, base = [], 0
         for s, (r, order) in enumerate(zip(per, orders)):
             detected: List[DetectedObject] = []
             if order:
                 images_of = (lambda a, b, o=base: images(o + a, o + b)) if images is not None else (lambda a, b: [])
-                detected = self._classified_objects(self._metadata_of(r["clusters"], order), images_of)
+                detected = self._classified_objects(self._metadata_of(r["clusters"], order), images_of, classify)
             base += len(order)
             out.append(self._result(detected, r["ground"], r["object"], bevs[s], contexts[s]))
             if matches is not None:
@@ -399,6 +426,41 @@ class LiDARAgent:
             return got
         return images
 
+    def _batch_cluster_mosaics(self, res, per: List[Dict[str, Any]], orders: List[List[int]]) -> Callable[[int, int], Optional[str]]:
+        """mosaic(a, b): the base64 PNG of the classifier mosaic of clusters a..b-1 of all samples' orders laid end to end (a group of
+        at most ten of one sample), drawn and encoded on the device for whole groups, at most CLUSTER_IMAGES_PER_CALL views at a time, as
+        they are asked for (in increasing order).  Only the PNG files are copied to the host."""
+        views = np.array([(r["object_off"], r["object_off"] + len(r["object"]), l) for r, order in zip(per, orders) for l in order],
+                         np.int64).reshape(-1, 3)
+        sizes = np.array([int(r["clusters"][l, 10]) for r, order in zip(per, orders) for l in order], np.int64)
+        groups, base = [], 0
+        for order in orders:
+            groups += [(base + a, min(10, len(order) - a)) for a in range(0, len(order), 10)]
+            base += len(order)
+        chunks, g0 = [], 0  # whole groups, at most CLUSTER_IMAGES_PER_CALL views (at least one group) per chunk
+        while g0 < len(groups):
+            g1 = g0 + 1
+            while g1 < len(groups) and groups[g1][0] + groups[g1][1] - groups[g0][0] <= CLUSTER_IMAGES_PER_CALL:
+                g1 += 1
+            chunks.append((g0, g1))
+            g0 = g1
+        chunk_of = {groups[g][0]: c for c, (a, b) in enumerate(chunks) for g in range(a, b)}
+        held: Dict[int, Dict[int, str]] = {}
+
+        def mosaic(a: int, b: int) -> Optional[str]:
+            c = chunk_of[a]
+            if c not in held:
+                held.clear()
+                g0, g1 = chunks[c]
+                v0, v1 = groups[g0][0], groups[g1 - 1][0] + groups[g1 - 1][1]
+                vr = self.engine.run_cluster_views(res.object, res.labels, views[v0:v1], max_view_points=int(sizes[v0:v1].max()))
+                mos = self.engine.run_cluster_mosaics(vr, [(f - v0, n) for f, n in groups[g0:g1]])
+                vr.check()
+                files = ops.encode_png_batch(self.engine, mos.images, swap_rb=True)
+                held[c] = {groups[g][0]: base64.b64encode(f).decode("ascii") for g, f in zip(range(g0, g1), files)}
+            return held[c][a]
+        return mosaic
+
     def _result(self, detected: List[DetectedObject], ground: np.ndarray, obj: np.ndarray, bev: Optional[Dict[str, np.ndarray]],
                 context: Optional[Dict]) -> Dict[str, Any]:
         features = self._extract_semantic_features(detected, ground, obj)
@@ -414,6 +476,8 @@ class LiDARAgent:
         prompt = "Analyze this driving scene from LiDAR data:\n\n" + report
         if context:
             prompt += "\n\nAdditional context from other sensors:\n" + json.dumps(context, indent=2)
+        if "png" in bev:
+            return self.call_llm([{"role": "user", "content": prompt}], temperature=0.4, bev_png=bev["png"])
         return self.call_llm([{"role": "user", "content": prompt}], temperature=0.4, bev_semantic=bev["semantic"])
 
 

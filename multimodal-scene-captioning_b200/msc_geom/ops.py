@@ -422,3 +422,36 @@ def camera_frames(eng: GeometryEngine, samples, to_host: bool = False, threads: 
         a = np.array(Image.open(path))
         out[i][c] = a if to_host else torch.from_numpy(a).to(eng.device)
     return out
+
+
+PNG_WORKSPACE_PER_CALL = 4 << 30  # workspace bytes one device call of encode_png_batch may use (an 800 x 800 RGB image reserves 11.5 MB)
+
+
+def encode_png_batch(eng: GeometryEngine, images, swap_rb=False) -> List[bytes]:
+    """PNG files of uint8 images, (H, W, 3) RGB or (H, W) grey, host arrays or CUDA tensors, encoded on the device: each has Pillow's
+    IHDR and an IDAT that inflates to the payload of `Image.fromarray(img).save(buf, "PNG")`, so it decodes to the same pixels.
+    swap_rb reads BGR images as RGB (serialize.image_to_base64's [:, :, ::-1]).  Consecutive images are encoded in one device call per
+    PNG_WORKSPACE_PER_CALL bytes of workspace; a call whose files outgrow the default arena is encoded once more into an arena of the
+    exact size."""
+    frames = [img if isinstance(img, torch.Tensor) and img.is_cuda else torch.from_numpy(np.ascontiguousarray(img)).to(eng.device) for img in images]
+    swaps = [bool(swap_rb)] * len(frames) if isinstance(swap_rb, (bool, int, np.bool_)) else [bool(v) for v in swap_rb]
+    descs, _ = eng._png_descs(frames, swaps)
+    size = C.sizeof(_capi.MscPngImage)
+    per = [int(eng.lib.msc_png_encode_workspace_bytes(1, C.addressof(descs) + k * size)) for k in range(len(frames))]
+    out: List[bytes] = []
+    a = 0
+    while a < len(frames):
+        b, acc = a + 1, per[a]
+        while b < len(frames) and acc + per[b] <= PNG_WORKSPACE_PER_CALL:
+            acc += per[b]
+            b += 1
+        res = eng.run_png_encode(frames[a:b], swaps[a:b])
+        try:
+            files = res.to_host()
+        except _capi.MscError as e:
+            if e.status != 1:
+                raise
+            files = eng.run_png_encode(frames[a:b], swaps[a:b], out=eng.alloc_png(frames[a:b], swaps[a:b], out_bytes=res.needed)).to_host()
+        out += files
+        a = b
+    return out
