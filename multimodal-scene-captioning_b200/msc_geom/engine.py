@@ -787,8 +787,10 @@ class GeometryEngine:
         """The finished 4-view image of LiDARAgent._generate_cluster_visualization (discs, axes, titles) of every view, in one
         stream-ordered call per CLUSTER_VIEWS_WORKSPACE_PER_CALL bytes of workspace (msc_cluster_views_batch).  rows: f32 [*, 4] and
         labels: i32 [*] CUDA tensors (e.g. a LidarBatchResult's object and labels); views: (row_begin, row_end, label) triples, the
-        points of a view being the rows of its range with its label, in row order.  max_view_points bounds the points of one view
-        (default: the longest range); a larger view raises in to_host().  Nothing is synchronised."""
+        points of a view being the rows of its range with its label, in row order.  The points of every view must be finite, as a
+        LidarBatchResult's object rows are (the keyframe gate drops non-finite rows): the reference draws no point of a cluster whose
+        mean is not finite, and nothing here checks for one (ops.cluster_views refuses such a cluster on the host).  max_view_points
+        bounds the points of one view (default: the longest range); a larger view raises in to_host().  Nothing is synchronised."""
         v = np.ascontiguousarray(np.asarray(views, dtype=np.int64).reshape(-1, 3))
         n = v.shape[0]
         if not (isinstance(rows, torch.Tensor) and rows.is_cuda and rows.dtype == torch.float32 and rows.dim() == 2 and rows.shape[1] == 4

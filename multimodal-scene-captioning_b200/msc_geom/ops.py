@@ -237,7 +237,9 @@ def cluster_views(eng: GeometryEngine, points: np.ndarray, clusters) -> np.ndarr
     """Point discs of LiDARAgent._generate_cluster_visualization (lidar_agent.py:241-351) for a list of clusters of one cloud.
     points: (N,4) f32; clusters: list of index arrays into points (original order inside a cluster).  Returns u8
     [K,512,512,3] without axes / titles (see lidar_agent.finish_cluster_view).  The cluster mean and pixel scale are
-    evaluated on the host with NumPy exactly as the reference does (:255-264) -- a few hundred floats per cluster."""
+    evaluated on the host with NumPy exactly as the reference does (:255-264) -- a few hundred floats per cluster.  A cluster whose
+    mean is not finite (a NaN or infinite coordinate) raises ValueError: the reference's astype(int) puts every point of it outside
+    every view, while the device's float-to-int conversion would turn NaN into a pixel."""
     K = len(clusters)
     if K == 0:
         return np.zeros((0, 512, 512, 3), np.uint8)
@@ -248,6 +250,8 @@ def cluster_views(eng: GeometryEngine, points: np.ndarray, clusters) -> np.ndarr
     for k, idx in enumerate(clusters):
         cp = pts[idx, :3]
         center = cp.mean(axis=0)
+        if not np.isfinite(center).all():
+            raise ValueError("cluster %d: its mean is not finite (a NaN or infinite coordinate); the reference draws none of its points" % k)
         centered = cp - center
         max_range = max(centered[:, 0].max() - centered[:, 0].min(), centered[:, 1].max() - centered[:, 1].min(),
                         centered[:, 2].max() - centered[:, 2].min())
